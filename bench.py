@@ -20,6 +20,9 @@ Workload (BASELINE.json configs[1]): a batch of 4096 x 8 s synthetic 16 kHz utte
   cpu_baseline : the oracle (CPU restatement of the reference path) on a bounded sample, rank 0, N=1.
 `--impl reference` times the reference's CPU implementation of the path (the oracle port) instead, on the same
 `config.workload` (a bounded sample of its rows per step).
+`--dump-outputs DIR` writes what the last timed step of the device-resident arm returned (rank 0's probabilities, decisions and
+per-row segment counts, and the gathered segment list) as DIR/<name>.npy, so that two builds can be compared output for output:
+the inputs and weights are seeded, identical from run to run.
 Multi-GPU: `torchrun --nproc-per-node N bench.py --gpus N ...`; utterances are sharded across ranks (no data-path
 collective); segment lists are gathered with NCCL on a side stream, one step behind the compute (b200vad.SegmentGatherer),
 and drained inside the timed region; scaling = weak.
@@ -86,6 +89,30 @@ def load_peaks():
             d = json.load(f)
         return {"hbm_gbs": d["hbm_gbs"], "tf_burst": d["bf16_tflops"], "tf_sustained": d["bf16_tflops_sustained"], "src": "measured"}
     return {"hbm_gbs": 6650.0, "tf_burst": 1590.0, "tf_sustained": 1400.0, "src": "fallback"}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each array as DIR/<name>.npy: integers wider than 16 bits as float64, everything else as float32 (both exact
+    for the outputs of the path).  Each array gets an equal share of DUMP_BYTES; one larger than that is replaced by a fixed,
+    seeded sample of its rows, sorted, whose row indices are written as DIR/<name>_rows.npy."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 1024          # room for the .npy headers
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float64 if a.dtype.kind in "iu" and a.dtype.itemsize > 2 else np.float32)
+        rows_path = os.path.join(dirname, f"{name}_rows.npy")
+        if a.nbytes > share:
+            per_row = a.nbytes // a.shape[0] + 8
+            idx = np.sort(np.random.default_rng(0).choice(a.shape[0], share // per_row, replace=False))
+            a = a[idx]
+            np.save(rows_path, idx.astype(np.float64))
+        elif os.path.exists(rows_path):
+            os.remove(rows_path)
+        np.save(os.path.join(dirname, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -287,7 +314,13 @@ def main():
     ap.add_argument("--rows", type=int, default=ROWS, help="utterances per GPU per step (default = the named workload)")
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-modes", action="store_true", help="skip the PyanNet arm and the configs 1 / 3 / 4 / 5 timings")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (at most 64 MB; b200 path only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     if args.impl == "reference":
         return run_reference(args, jout)
 
@@ -309,7 +342,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     warmup = max(args.warmup, 3)
-    steps = max(args.steps, 1)
+    steps = args.steps
     rows = args.rows
     L = _lib.lib()
 
@@ -336,6 +369,7 @@ def main():
     def device_step():
         prob, dec, seg, counts, seg_off = torch.ops.b200vad.vad_pipeline_padded(wav_dev, None, blob, 4, 0.5, 49)
         gatherer.push(seg, seg_off, row_base=lo)
+        return prob, dec, counts
 
     def barrier():
         if world > 1:
@@ -355,8 +389,10 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record()
-    for _ in range(steps):
+    # only the last step's outputs are kept: each earlier step's are released at once, so every step reuses the same buffers
+    for _ in range(steps - 1):
         device_step()
+    last = device_step()
     gathered = gatherer.drain()                 # completes the pending gathers; the compute stream waits for the side stream
     e1.record()
     barrier()
@@ -369,6 +405,10 @@ def main():
         _lib.check(L.b200vad_profile_collect(kind, C.byref(tot_ms), C.byref(nl)), "profile_collect")
         prof[kind] = (tot_ms.value, nl.value)
     L.b200vad_profile_enable(0)
+    if args.dump_outputs and rank == 0:
+        prob, dec, counts = last
+        dump_outputs(args.dump_outputs, {"prob": prob, "dec": dec, "counts": counts, "segments": gathered[-1]})
+    del last
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
