@@ -83,8 +83,9 @@ B200VAD_API int b200vad_lstm_fused_clusters(void);
  * layer-output store, 4 no cell arithmetic, 8 no recurrent MMAs, 16 no input-projection MMAs; lag >= 0 sets how many part
  * slots the input MMAs of a part trail its recurrent MMAs (default 3).  flags = 0 restores the product path. */
 B200VAD_API int b200vad_set_lstm_fused_debug(int flags, int lag);
-/* with flag 32 set, the last fused launch leaves per (CTA, warp, wait site) cycle totals / counts of its mbarrier waits in a
- * device table; this copies the first n int64 values [cta 148][warp 18][site 8][cycles, count] to host (synchronises) */
+/* with flag 32 set, the last fused launch leaves per (CTA, warp, wait site) cycle totals / counts of its waits in a device
+ * table; this copies the first n int64 values to host (synchronises).  Mode 1: [cta 148][warp 25][site 8][cycles, waits,
+ * mbarrier polls], site 0 = [kernel cycles, steps run, -]; mode 2: the CTA-pair kernel's table (tools/pair_waits.py) */
 B200VAD_API int b200vad_lstm_fused_read_debug(long long* host, int n);
 /* the fused kernel's waits are bounded (a protocol bug traps instead of hanging the GPU); the first wait that timed out leaves
  * {1, block, thread, wait site, barrier address, parity, grid size} in page-locked host memory, readable after the fault */

@@ -47,24 +47,40 @@ def main():
         print(f"{label:58s} layer kernel {out[0][0]:8.3f} ms x{out[0][1]:3d}   projection {out[1][0]:7.3f} ms x{out[1][1]}", flush=True)
 
     def waits(flags, label):
-        """per-role wait-time table of cluster 0 (flag 32): cycles per step spent in each wait site"""
+        """per-role wait-time table (flag 32): share of the kernel each warp spends in each wait site (non-immediate waits; a
+        named barrier counts every passage), and the mbarrier polls (try_wait / test_wait instructions) per step and CTA"""
         lib.b200vad_set_lstm_fused(1)
         lib.b200vad_set_lstm_fused_debug(flags | 32, 3)
         torch.ops.b200vad.lstm_head(x, blob, 4)
         torch.cuda.synchronize()
-        n = 148 * 26 * 16
+        W, TAGS, F = 25, 8, 3                                   # warps per CTA, wait tags, fields (cycles, waits, polls): lstm_fused.cu
+        n = 148 * W * TAGS * F
         buf = (C.c_longlong * n)()
         lib.b200vad_lstm_fused_read_debug(buf, n)
-        roles = {"prod": {1: "x_empty"}, "pw": {6: "acc_ready"}, "mmah": {2: "x_done", 4: "h_ready"},
-                 "mmax": {2: "acc_free", 3: "x_full", 5: "drain"}, "pub": {1: "slice"}, "load": {1: "y_done", 7: "h_free"}}
-        print(f"--- wait sites, {label} (last layer launch; cycles per kernel, non-immediate waits)")
+        roles = {"prod": {1: "x_empty"}, "pw": {6: "acc_ready", 5: "acc_ready bar", 4: "slice bar"}, "mmah": {2: "x_done", 4: "h_ready"},
+                 "mmax": {2: "acc_free", 3: "x_full", 5: "drain"}, "send": {1: "slice", 7: "h_free"}}
+        role_of = lambda w: "pw" if w < 16 else "prod" if w == 16 else "mmah" if w < 19 else "mmax" if w < 21 else "send"
+        at = lambda cta, warp, tag, f: buf[((cta * W + warp) * TAGS + tag) * F + f]
+        print(f"--- wait sites, {label} (last layer launch; share of the kernel in non-immediate waits)")
         for cta in (0, 1, 5):
-            for warp, role in ((0, "pw"), (5, "pw"), (10, "pw"), (15, "pw"), (16, "prod"), (17, "mmah"), (18, "mmah"), (19, "mmax"), (20, "mmax"), (21, "pub"), (24, "pub"), (25, "load")):
-                base = (cta * 26 + warp) * 16
-                tot = buf[base]
-                names = roles[role]
-                parts = [f"{names.get(t, t)} {buf[base + 2 * t] / max(tot, 1) * 100:5.1f}% (n={buf[base + 2 * t + 1]})" for t in range(1, 8) if buf[base + 2 * t + 1]]
+            for warp in (0, 1, 5, 10, 15, 16, 17, 18, 19, 20, 21, 24):
+                role = role_of(warp)
+                tot = at(cta, warp, 0, 0)
+                parts = [f"{roles[role].get(t, t)} {at(cta, warp, t, 0) / max(tot, 1) * 100:5.1f}% (n={at(cta, warp, t, 1)})"
+                         for t in range(1, TAGS) if at(cta, warp, t, 1)]
                 print(f"cta {cta} warp {warp:2d} {role:5s}: total {tot / 1e6:8.3f} Mcyc  " + "  ".join(parts), flush=True)
+        print(f"--- mbarrier polls per step and CTA, {label} (all 25 warps; lane 0 counts the warp's poll instructions)")
+        for cta in (0, 1, 5):
+            steps = max(at(cta, 16, 0, 1), 1)
+            site = {}
+            for warp in range(W):
+                role = role_of(warp)
+                for t in range(1, TAGS):
+                    if at(cta, warp, t, 2):
+                        k = f"{role}:{roles[role].get(t, t)}"
+                        site[k] = site.get(k, 0) + at(cta, warp, t, 2)
+            print(f"cta {cta} ({steps} steps): total {sum(site.values()) / steps:7.1f}   " +
+                  "  ".join(f"{k} {v / steps:6.1f}" for k, v in sorted(site.items())), flush=True)
         lib.b200vad_set_lstm_fused_debug(0, 3)
 
     def timeline(flags, label):

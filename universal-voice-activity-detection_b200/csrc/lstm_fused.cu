@@ -24,7 +24,9 @@
 //   * 16 pointwise warps: warp (pg, g) serves parts pg and pg + 4 alternately (while one part's h travels, the other is
 //     computed) and owns TMEM lane quarter g.  Lane 32 g + l of the accumulator is gate (l & 3) of unit 8 g + (l >> 2):
 //     the four gates of a cell sit in four adjacent lanes of ONE warp, so the (gate x sequence) transposition runs through a
-//     warp-private 2 KB scratch with __syncwarp only -- no cross-warp barrier anywhere in the per-step chain;
+//     warp-private 2 KB scratch with __syncwarp only.  One warp of the group polls acc_ready and releases the other three
+//     through a named barrier, and the staged h slice goes to the sender through another (F_BAR_ACC, F_BAR_SLICE): blocked
+//     warps issue nothing, where polling ones took issue slots from the pointwise pass;
 //   * 4 exchange-sender warps (h exchange over distributed shared memory): the pointwise warps write h_s (fp16 planes,
 //     operand layout) into the CTA's own 2 KB staging slice of the part; a sender warp copies it with 16-byte st.async stores
 //     into k-block `rank` of the part's operand tile in all four CTAs (the destination mbarriers count the bytes).  The MMA K
@@ -35,7 +37,9 @@
 // chain latency (recurrent MMAs -> accumulator read -> cell arithmetic -> h exchange -> next MMAs, ~2 900 cycles) plus a per-part
 // cost of ~475 cycles: a part needs 384 tensor-pipe cycles (16 recurrent MMAs x 8 + 16 input MMAs x 16), 6 KB out + 6 KB in over
 // the SM-to-SM port (~17 B/clk: 360-720 cycles) and ~320 issue slots per SM sub-partition.  n = 8 is all the accumulator columns
-// TMEM has left, so half of the step is unhidden latency.  Exchange mechanisms tried: cp.async.bulk by a sender thread (~3000 cycles per
+// TMEM has left, so half of the step is unhidden latency.  Replacing 12 of the 16 acc_ready pollers and the 4 slice pollers by named
+// barriers (~160 -> ~86 polls per step and CTA) cut the one-part step to 1.18 us and the layer by 3.4 %, but not the per-part slope
+// (profiles/r03_lstm_fused_handoffs.md): the issue slots taken by polls are not what sets the per-part cost.  Exchange mechanisms tried: cp.async.bulk by a sender thread (~3000 cycles per
 // copy through the TMA unit), st.async from the pointwise warps (they stall on the port), and an exchange through the output
 // planes in L2 (TMA store + multicast TMA load: two ~1-2 us TMA round trips on the per-step chain; that variant showed
 // intermittent launch failures -- in hindsight probably the x_full race described at bar_x_full, which any delay of the x tiles
@@ -103,9 +107,10 @@ struct FusedParams {
     int flags;               // timing probes (wrong results): 2 no y store, 4 no cell math, 8 no recurrent MMAs, 16 no input MMAs, 32 wait-time table, 64 timeline
 };
 
-// wait-time probe (flags & 32, tools/fused_ablate.py): per (CTA, warp, wait tag) cycles spent in non-immediate waits and their count
-constexpr int F_DBG_TAGS = 8, F_DBG_WARPS = 25, F_DBG_MAX_CTAS = 148;
-__device__ long long g_fused_dbg[F_DBG_MAX_CTAS * F_DBG_WARPS * F_DBG_TAGS * 2];
+// wait-time probe (flags & 32, tools/fused_ablate.py): per (CTA, warp, wait tag) cycles spent in non-immediate waits, their count,
+// and the mbarrier polls of the site (try_wait / test_wait instructions, immediate ones included); tag 0 = kernel cycles, steps run
+constexpr int F_DBG_TAGS = 8, F_DBG_FIELDS = 3, F_DBG_WARPS = 25, F_DBG_MAX_CTAS = 148;
+__device__ long long g_fused_dbg[F_DBG_MAX_CTAS * F_DBG_WARPS * F_DBG_TAGS * F_DBG_FIELDS];
 
 // timeline probe (flags & 64): clock64 stamps of one part (part 0 of CTA 0's first item) over F_TRACE_STEPS steps
 constexpr int F_TRACE_S0 = 100, F_TRACE_STEPS = 8;
@@ -124,7 +129,10 @@ __device__ volatile int* g_fused_err_host = nullptr;
 template <bool CLUSTER_ACQUIRE>
 __device__ __forceinline__ void mbar_wait_tag(uint32_t bar, uint32_t parity, int tag, long long* wacc) {
     if (!wacc && (CLUSTER_ACQUIRE ? mbar_try_wait_cluster(bar, parity) : mbar_try_wait(bar, parity))) return;
-    if (wacc && !CLUSTER_ACQUIRE && mbar_test_wait(bar, parity)) return;   // probe mode: count every wait that is not already satisfied
+    if (wacc && !CLUSTER_ACQUIRE) {                                     // probe mode: count every wait that is not already satisfied
+        wacc[F_DBG_FIELDS * tag + 2] += 1;
+        if (mbar_test_wait(bar, parity)) return;
+    }
     const long long t0 = wacc ? clock64() : 0;
     // suspended in hardware for up to 20 us per try (the default limit is ~80 cycles: see mbar_try_wait_hint); the time
     // bound (~2 s) is checked once per 64 tries
@@ -145,7 +153,29 @@ __device__ __forceinline__ void mbar_wait_tag(uint32_t bar, uint32_t parity, int
             __trap();
         }
     }
-    if (wacc) { wacc[2 * tag] += clock64() - t0; wacc[2 * tag + 1] += 1; }
+    if (wacc) { wacc[F_DBG_FIELDS * tag] += clock64() - t0; wacc[F_DBG_FIELDS * tag + 1] += 1; wacc[F_DBG_FIELDS * tag + 2] += tries + 1; }
+}
+
+// Named barriers of the per-step chain (IDs 0 = __syncthreads and 9-15 are free).  A warp blocked in bar.sync issues nothing,
+// where an mbarrier wait keeps polling (the suspend-time hint is capped by the hardware): polls were ~30 % of the kernel's
+// issued instructions, on the same four schedulers that run the pointwise pass.
+//   * F_BAR_ACC + pg (1-4), 128 threads: the 4 pointwise warps of part group pg, once per (step, part q in {pg, pg + 4} with
+//     q < nparts), after the group's poller (warp 5 pg, lane quarter g == pg: one poller per SM sub-partition) has seen
+//     acc_ready(q).  The poller's mbarrier wait keeps the bounded wait and its time-out record.
+//   * F_BAR_SLICE + pg (5-8), 160 threads: the same 4 warps and sender warp pg, once per (step s with s + 1 < T, part q in
+//     {pg, pg + 4} with q < nparts), when the part's h_s slice is staged.  Replaces an mbarrier arrive + sender poll; holding
+//     the pointwise warps until the sender arrives costs the chain nothing, because what they wait for next, acc_ready of the
+//     group's other part, needs the sender's previous send (h of that part) to have landed anyway.
+// Both sides of a barrier run the same (s, q) sequence from the same conditions (q < nparts per item, s + 1 < T for the
+// exchange), and bar.sync blocks every participant until all have arrived: no participant can arrive at generation n + 1
+// before generation n completed, so generations cannot mix.  A participation mismatch would hang instead of trapping.
+constexpr uint32_t F_BAR_ACC = 1, F_BAR_SLICE = 5;
+__device__ __forceinline__ void fused_bar(uint32_t id, uint32_t threads, int tag, long long* wacc) {
+    const long long t0 = wacc ? clock64() : 0;
+    named_bar_sync(id, threads);
+    // every passage, no polls.  The counts are exact; the times measured so far read implausibly low (0.2-0.6 % of the kernel for
+    // warps that wait on the poller), so they are not used (profiles/r03_lstm_fused_handoffs.md)
+    if (wacc) { wacc[F_DBG_FIELDS * tag] += clock64() - t0; wacc[F_DBG_FIELDS * tag + 1] += 1; }
 }
 
 // The MMA-issuing threads are serial resources (one tcgen05.mma of N = 16 occupies the tensor pipe for 8 cycles):
@@ -188,7 +218,6 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
     auto bar_h_ready = [&](int q) { return bar_base + 384 + 8 * q; };
     auto bar_h_free = [&](int q) { return bar_base + 448 + 8 * q; };
     const uint32_t tmem_slot = bar_base + 512;
-    auto bar_slice = [&](int q) { return bar_base + 528 + 8 * q; };
     auto bar_x_done = [&](int pp) { return bar_base + 592 + 8 * pp; };   // per pair of parts
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -207,7 +236,6 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
             mbar_init(bar_acc_free(q), 4);
             mbar_init(bar_h_ready(q), FUSED_EXCH_PLAIN ? FC : 1);
             mbar_init(bar_h_free(q), FC);
-            mbar_init(bar_slice(q), 4);
             mbar_init(bar_x_done(q), 1);
         }
         mbar_fence_init();
@@ -221,9 +249,9 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
 
     // wait-time probe: lane 0 of every warp accumulates straight into its row of the global table (probe mode only)
     long long* const wacc = (PROBE && (p.flags & 32) && lane == 0 && blockIdx.x < F_DBG_MAX_CTAS)
-                                ? &g_fused_dbg[((size_t)blockIdx.x * F_DBG_WARPS + warp) * (2 * F_DBG_TAGS)] : nullptr;
+                                ? &g_fused_dbg[((size_t)blockIdx.x * F_DBG_WARPS + warp) * (F_DBG_FIELDS * F_DBG_TAGS)] : nullptr;
     if (wacc) {
-        for (int i = 0; i < 2 * F_DBG_TAGS; ++i) wacc[i] = 0;
+        for (int i = 0; i < F_DBG_FIELDS * F_DBG_TAGS; ++i) wacc[i] = 0;
         wacc[0] = -clock64();
     }
     long long* const trace = (PROBE && (p.flags & 64) && blockIdx.x == 0 && lane == 0) ? g_fused_trace : nullptr;
@@ -241,6 +269,7 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
         const int seq0 = part0 * FPN;
         if (nparts == 0) continue;                            // (uniform over the cluster)
         const bool tr_item = trace && item == cluster_id;
+        if (wacc) wacc[1] += T;                               // steps this CTA runs (the per-step normaliser of the table)
 
         // ---------------- weights of this direction -> tensor memory (pointwise warps; only when the direction changes)
         if (warp < F_PW_WARPS && loaded_dir != dir) {
@@ -477,17 +506,16 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
             uint32_t cta_delta[FC];                                            // [d]: address offset of CTA (rank + d) & 3 (static indices only)
 #pragma unroll
             for (uint32_t d = 0; d < FC; ++d) cta_delta[d] = mapa_shared(smem_base, (rank + d) & (FC - 1)) - smem_base;
-            // ph_a: slice phase bits, ph_b: h_free phase bits
+            // ph_b: h_free phase bits
             for (int s = 0; s + 1 < T; ++s) {
                 for (int q = warp - F_W_SEND; q < nparts; q += 4) {
                     const bool trl = tr_item && q == 0 && s >= F_TRACE_S0 && s < F_TRACE_S0 + F_TRACE_STEPS;
+                    fused_bar(F_BAR_SLICE + (q & 3), 160, 1, wacc);               // the part's four pointwise warps have written h_s
                     if (lane == 0) {
-                        FUSED_WAIT(bar_slice(q), (ph_a >> q) & 1u, 1);            // the part's four pointwise warps have written h_s
                         if (trl) trace[(s - F_TRACE_S0) * 16 + 7] = clock64();
                         // every CTA's recurrent MMAs of step s have finished reading the part's tile (it still holds h_{s-1})
                         FUSED_WAIT(bar_h_free(q), (ph_b >> q) & 1u, 7);
                     }
-                    ph_a ^= 1u << q;
                     ph_b ^= 1u << q;
                     __syncwarp();
                     const uint32_t src = smem_base + g_off + ((s & 1) * FMAXP + q) * F_BOX + lane * 16;
@@ -549,7 +577,8 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
             // after the staging pass: lane = (sequence row lane & 15, plane lane >> 4), the 16-byte chunk of this warp's 8 units
             const int yrow = lane & 15;
             __half* const yplane = (lane >> 4) ? p.y_b : p.y_a;
-            // ph_a: acc_ready phase bits (bit pi)
+            // ph_a: acc_ready phase bits (bit pi; used by the group's poller only)
+            const bool poller = g == pg;
             for (int s = 0; s < T; ++s) {
                 const int t = dir == 0 ? s : T - 1 - s;
                 const bool exchange = s + 1 < T;
@@ -557,9 +586,10 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
                 for (int pi = 0; pi < 2; ++pi) {
                     const int q = pg + 4 * pi;
                     if (q >= nparts) break;
-                    FUSED_WAIT(bar_acc_ready(q), (ph_a >> pi) & 1u, 6);
+                    if (poller) FUSED_WAIT(bar_acc_ready(q), (ph_a >> pi) & 1u, 6);
                     ph_a ^= 1u << pi;
-                    tc_fence_after();
+                    fused_bar(F_BAR_ACC + pg, 128, 5, wacc);                       // the poller saw acc_ready(q)
+                    tc_fence_after();                                              // (commit -> mbarrier -> poller -> bar.sync -> tcgen05.ld)
                     const bool tr_on = tr_item && warp == 0 && pi == 0 && s >= F_TRACE_S0 && s < F_TRACE_S0 + F_TRACE_STEPS;
                     if (tr_on) trace[(s - F_TRACE_S0) * 16 + 2] = clock64();
                     float z[16];
@@ -616,7 +646,7 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
                         *reinterpret_cast<__half*>(rp + (((4 + g) ^ (row & 7)) << 4)) = a2;
                     }
                     __syncwarp();
-                    if (exchange && lane == 0) mbar_arrive(bar_slice(q));          // (release: the sender warp reads the slice with plain loads)
+                    if (exchange) fused_bar(F_BAR_SLICE + pg, 160, 4, wacc);       // hand the slice to sender warp pg (it reads it with plain loads)
                     // layer output planes (B, T, 256) = the same chunks: lane = (row, plane), this warp's 16 bytes (8 units)
                     const uint4 v = *reinterpret_cast<const uint4*>(stg + yrow * 128 + ((((lane >> 4) * 4 + g) ^ (yrow & 7)) << 4));
                     const int b = seq0 + q * FPN + yrow;
@@ -655,7 +685,7 @@ int lstm_fused_read_debug(long long* host, int n) {
         B200VAD_CUDA(cudaMemcpyFromSymbol(host, g_fused_trace, sizeof(long long) * std::min(-n, F_TRACE_STEPS * 16 + 128)));
         return B200VAD_OK;
     }
-    const size_t bytes = sizeof(long long) * (size_t)std::min<long long>(n, (long long)F_DBG_MAX_CTAS * F_DBG_WARPS * F_DBG_TAGS * 2);
+    const size_t bytes = sizeof(long long) * (size_t)std::min<long long>(n, (long long)F_DBG_MAX_CTAS * F_DBG_WARPS * F_DBG_TAGS * F_DBG_FIELDS);
     B200VAD_CUDA(cudaMemcpyFromSymbol(host, g_fused_dbg, bytes));
     return B200VAD_OK;
 }
