@@ -204,6 +204,26 @@ B200VAD_API int b200vad_pipeline_fbank_i16(const void* packed, int num_layers, c
                                int64_t N, int64_t wav_stride, float thr, int kernel, float* prob, uint8_t* dec, int32_t* counts,
                                int64_t* seg_off, int32_t* seg, int64_t cap, void* workspace, size_t ws_bytes, void* stream);
 
+/* ---- whole path of the reference's SincNet flow (feature_extractor="sincnet", config/config.py) on device buffers:
+ * SincNet -> PyanNet's LSTM stack + head (src/models/segmentation/PyanNet.py:164-197) -> threshold / median filter
+ * (src/engines/vad_engine.py:204-211: kernel 49 = window 0.01 since encoding_dim != 768) -> run-length segments that keep
+ * single-frame runs (src/scripts/predict_sincnet.py:348-370, min_run = 1).  The front end hands the LSTM its layer-0 operand
+ * as fp16 planes directly (no fp32 (B, Ts, 60) round trip): prob / dec equal b200vad_sincnet_forward_f32 followed by
+ * b200vad_model_forward_f32 and b200vad_threshold_median bit for bit.
+ * packed_model: b200vad_model_pack_* blob with D = 60; packed_sincnet: b200vad_sincnet_pack blob.  Ts =
+ * b200vad_sincnet_num_frames(N) frames per row; N >= 991 (one SincNet frame).  There is no lens argument: the reference pads
+ * SincNet windows with zero audio, which its InstanceNorm sees.  cap: B * ceil(Ts / 2) holds every possible segment. */
+B200VAD_API size_t b200vad_pipeline_sincnet_workspace_bytes(int B, int64_t N);
+B200VAD_API int b200vad_pipeline_sincnet_f32(const void* packed_model, const void* packed_sincnet, int num_layers, const float* wav,
+                                 int B, int64_t N, int64_t wav_stride, float thr, int kernel, float* prob /* (B,Ts) */,
+                                 uint8_t* dec /* (B,Ts) */, int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap,
+                                 void* workspace, size_t ws_bytes, void* stream);
+/* 16-bit PCM rows (int16 / 32768, exact): identical results to the f32 form on the converted waveform, half the bytes */
+B200VAD_API int b200vad_pipeline_sincnet_i16(const void* packed_model, const void* packed_sincnet, int num_layers, const int16_t* wav,
+                                 int B, int64_t N, int64_t wav_stride, float thr, int kernel, float* prob, uint8_t* dec,
+                                 int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, void* workspace, size_t ws_bytes,
+                                 void* stream);
+
 /* ---- host-buffer session: the same path with HOST waveforms and HOST results -- what a caller holding
  * lhotse/DataLoader batches in host memory uses (src/engines/vad_engine.py:204-211 fed by
  * src/datasets/data_module.py:194-206).  The session owns device buffers for two batches in flight and three
@@ -217,6 +237,11 @@ B200VAD_API int b200vad_pipeline_fbank_i16(const void* packed, int num_layers, c
 typedef struct b200vad_session b200vad_session;
 B200VAD_API int b200vad_session_create(int device, const void* packed_device, int num_layers, int max_chunk_rows, int64_t N,
                            b200vad_session** out);
+/* the same session on the SincNet path (b200vad_pipeline_sincnet_*; the reference feeds it from
+ * src/scripts/predict_sincnet.py's DataLoader): T = b200vad_sincnet_num_frames(N), up to ceil(T / 2) segments per row.
+ * It is driven by the calls below, unchanged. */
+B200VAD_API int b200vad_session_create_sincnet(int device, const void* packed_model, const void* packed_sincnet, int num_layers,
+                                   int max_chunk_rows, int64_t N, b200vad_session** out);
 /* wav_host: (B, N) f32; outputs on host: dec (B,T) u8 (optional), prob (B,T) f32 (optional),
  * seg (cap,3) i32, *nseg total segments.  Blocks until results are on the host. */
 B200VAD_API int b200vad_session_run_host(b200vad_session* s, const float* wav_host, int B, float thr, int kernel, uint8_t* dec_host,
@@ -241,6 +266,11 @@ B200VAD_API void b200vad_session_destroy(b200vad_session* s);
 typedef struct b200vad_stream b200vad_stream;
 B200VAD_API int b200vad_stream_create(int device, const void* packed_device, int num_layers, int num_streams, int64_t window_samples,
                           int hop_samples, int use_graph, b200vad_stream** out);
+/* the same on the SincNet path: SincNet -> PyanNet -> threshold / median on every buffered window (the graph covers the
+ * front end too).  hop_samples must be a multiple of 270 (the SincNet frame step), window_samples >= 991; a push returns
+ * the newest hop_samples / 270 frames, the last ones of the b200vad_sincnet_num_frames(window_samples) frames of the window. */
+B200VAD_API int b200vad_stream_create_sincnet(int device, const void* packed_model, const void* packed_sincnet, int num_layers,
+                                  int num_streams, int64_t window_samples, int hop_samples, int use_graph, b200vad_stream** out);
 B200VAD_API int b200vad_stream_push(b200vad_stream* s, const float* chunk, int chunk_on_host, float thr, int kernel, float* prob_new_host,
                         uint8_t* dec_new_host, float* device_ms);
 /* parity / debugging: current windows (S, window) f32 and all frame outputs (S, T) of the last push, to host buffers */

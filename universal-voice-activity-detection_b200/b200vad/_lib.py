@@ -72,6 +72,13 @@ PROTOTYPES = {
                                            c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
     "b200vad_pipeline_fbank_i16": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int, c_int64, c_int64, c_float, c_int,
                                            c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
+    "b200vad_pipeline_sincnet_workspace_bytes": (c_size_t, [c_int, c_int64]),
+    "b200vad_pipeline_sincnet_f32": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int64, c_int64, c_float, c_int,
+                                             c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
+    "b200vad_pipeline_sincnet_i16": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int64, c_int64, c_float, c_int,
+                                             c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
+    "b200vad_session_create_sincnet": (c_int, [c_int, c_void_p, c_void_p, c_int, c_int, c_int64, C.POINTER(c_void_p)]),
+    "b200vad_stream_create_sincnet": (c_int, [c_int, c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_int, C.POINTER(c_void_p)]),
     "b200vad_session_submit_host_i16": (c_int, [c_void_p, c_int, c_void_p, c_int, c_float, c_int, c_void_p, c_void_p]),
     "b200vad_session_create": (c_int, [c_int, c_void_p, c_int, c_int, c_int64, C.POINTER(c_void_p)]),
     "b200vad_session_run_host": (c_int, [c_void_p, c_void_p, c_int, c_float, c_int, c_void_p, c_void_p, c_void_p, c_int64,

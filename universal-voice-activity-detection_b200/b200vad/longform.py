@@ -9,6 +9,12 @@ run-length encoded (predict.py:472-490).
 Extension (hop < window): overlapping windows; probabilities are stitched by taking every frame from the window
 whose centre is nearest (``b200vad_stitch_center``), then threshold + median + segments run once over the stitched
 stream.  Windows are rows of an ``as_strided`` view of the waveform: nothing is copied.
+
+SincNet -> PyanNet (``sincnet_packed``), as predict_sincnet.get_new_cuts does it: the same 5 s windows, but the tail window
+is zero padded in AUDIO (the SincNet InstanceNorm sees the zeros; no lens), per-window median filter, concatenation, a slice
+of ``ceil(get_num_frames(16000 d)) + 1`` frames per recording (predict_sincnet.py:330-337), run-length encoding that keeps
+single-frame runs and whole-second timestamps (predict_sincnet.py:348-370, 492-504).  Overlapped windows need a hop of whole
+SincNet frame steps (270 samples) so that every window's frames fall on one global grid.
 """
 
 from __future__ import annotations
@@ -17,15 +23,24 @@ from typing import Optional
 
 import torch
 
-from .host import cut_into_windows, merge_intervals_with_buffer, recording_offsets, segments_to_intervals
+from .host import (cut_into_windows, fbank_num_frames, get_num_frames, merge_intervals_with_buffer, recording_offsets,
+                   segments_to_intervals)
+
+SINC_STEP = 270       # samples between SincNet frames
 
 
 class LongFormVad:
     def __init__(self, packed: torch.Tensor, num_layers: int = 4, window: int = 80000, hop: Optional[int] = None,
-                 thr: float = 0.5, kernel: int = 49, max_rows: int = 4096, frame_shift: float = 0.01):
-        self.packed, self.L = packed, num_layers
+                 thr: float = 0.5, kernel: int = 49, max_rows: int = 4096, frame_shift: float = 0.01,
+                 sincnet_packed: Optional[torch.Tensor] = None):
+        self.packed, self.L, self.sinc = packed, num_layers, sincnet_packed
         self.window, self.hop = int(window), int(hop if hop is not None else window)
-        if self.window % 160 or self.hop % 160 or not (0 < self.hop <= self.window):
+        if self.sinc is not None:
+            if self.window < 991 or not (0 < self.hop <= self.window):
+                raise ValueError("need window >= 991 samples (one SincNet frame) and 0 < hop <= window")
+            if self.hop != self.window and self.hop % SINC_STEP:
+                raise ValueError("overlapped SincNet windows need a hop that is a multiple of 270 samples (the SincNet frame step)")
+        elif self.window % 160 or self.hop % 160 or not (0 < self.hop <= self.window):
             raise ValueError("window and hop must be multiples of 160 samples with 0 < hop <= window")
         self.thr, self.kernel, self.max_rows, self.fs = thr, kernel, max_rows, frame_shift
 
@@ -66,26 +81,33 @@ class LongFormVad:
         duration = N / 16000.0 if duration is None else duration
         wins = self.windows(N)
         rows, tail, lens = self._rows(wav, wins)
-        Tw = (self.window + 80) // 160
+        sinc = self.sinc is not None
+        Tw = get_num_frames(self.window) if sinc else fbank_num_frames(self.window)
+
+        def run(r, lens):
+            if sinc:            # the tail row is zero padded audio: no lens
+                return torch.ops.b200vad.vad_pipeline_sincnet(r, self.packed, self.sinc, self.L, self.thr, self.kernel)
+            return torch.ops.b200vad.vad_pipeline(r, lens, self.packed, self.L, self.thr, self.kernel)
+
         probs, decs = [], []
         for b0 in range(0, rows.shape[0], self.max_rows):
-            r = rows[b0:b0 + self.max_rows]
-            p, d, _, _ = torch.ops.b200vad.vad_pipeline(r, None, self.packed, self.L, self.thr, self.kernel)
+            p, d, _, _ = run(rows[b0:b0 + self.max_rows], None)
             probs.append(p); decs.append(d)
         if tail is not None:
-            p, d, _, _ = torch.ops.b200vad.vad_pipeline(tail, lens[-1:], self.packed, self.L, self.thr, self.kernel)
+            p, d, _, _ = run(tail, lens[-1:])
             probs.append(p); decs.append(d)
         prob = torch.cat(probs) if probs else wav.new_empty((0, Tw))
+        min_run = 1 if sinc else 2      # the SincNet RLE keeps single-frame runs (predict_sincnet.py:348-370)
         if self.hop == self.window:
             # reference semantics: per-window median filter, concatenation, per-recording slice, RLE
             dec = torch.cat(decs).reshape(-1) if decs else torch.empty(0, dtype=torch.uint8, device=wav.device)
-            offs = recording_offsets([duration], dec.numel(), self.fs)
-            seg, _ = torch.ops.b200vad.segments(dec, torch.tensor(offs, dtype=torch.int64, device=wav.device), 2)
+            offs = recording_offsets([duration], dec.numel(), self.fs, sincnet=sinc)
+            seg, _ = torch.ops.b200vad.segments(dec, torch.tensor(offs, dtype=torch.int64, device=wav.device), min_run)
             stream = dec[: offs[1]]
         else:
-            L = (N + 80) // 160                            # frames of the whole recording
-            sp = torch.ops.b200vad.stitch_center(prob, self.hop // 160, L)
+            L = get_num_frames(N) if sinc else fbank_num_frames(N)       # frames of the whole recording
+            sp = torch.ops.b200vad.stitch_center(prob, self.hop // (SINC_STEP if sinc else 160), L)
             stream = torch.ops.b200vad.threshold_median(sp.view(1, -1), self.thr, self.kernel, False).view(-1)
-            seg, _ = torch.ops.b200vad.segments(stream.view(1, -1), None, 2)
-        ivs = segments_to_intervals(seg.tolist(), 1, self.fs)[0]
+            seg, _ = torch.ops.b200vad.segments(stream.view(1, -1), None, min_run)
+        ivs = segments_to_intervals(seg.tolist(), 1, self.fs, sincnet_durations=[duration] if sinc else None)[0]
         return {"prob": prob, "stream_dec": stream, "intervals": merge_intervals_with_buffer(ivs, duration, 0), "windows": wins}

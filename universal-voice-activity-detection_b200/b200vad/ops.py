@@ -6,6 +6,7 @@
   b200vad::threshold_median(prob, thr, kernel, i64) -> (B, T) u8 | i64     [a6/a7]
   b200vad::segments(dec, offsets?, min_run)         -> (S, 3) i32, (R) i32 [a8/a9]
   b200vad::vad_pipeline(wav, lens?, packed, L, thr, kernel) -> prob, dec, seg, counts
+  b200vad::vad_pipeline_sincnet(wav, packed_model, packed_sincnet, L, thr, kernel) -> prob, dec, seg, counts
 
 Each op enqueues on ``torch.cuda.current_stream()`` and never synchronises, except
 ``segments`` / ``vad_pipeline`` which read one int64 (the segment total) to size their output.
@@ -217,17 +218,28 @@ def _(dec, offsets=None, min_run=2):
 
 
 # ------------------------------------------------------------------ whole path
-def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel):
+def _seg_per_row(T: int, sincnet: bool) -> int:
+    """Most segments a row of T frames can hold: runs of >= 2 frames (fbank path) or of >= 1 frame (the SincNet RLE,
+    predict_sincnet.py:348-370)."""
+    return (T + 1) // 2 if sincnet else (T + 2) // 3
+
+
+def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc=None):
     """Enqueues the whole path on the current stream; returns device buffers only (nothing synchronises):
     prob (B, T) f32, dec (B, T) u8, seg (cap, 3) i32 of which the first seg_off[B] rows are valid, counts (B,) i32,
-    seg_off (B + 1,) i64."""
+    seg_off (B + 1,) i64.  ``sinc``: packed SincNet blob -> the SincNet -> PyanNet path (then ``lens`` must be None)."""
     wav = _prep_rows(wav, "wav")
     if wav.dim() != 2:
         raise _lib.B200VadError("wav must be (B, N)")
     B, N = wav.shape
     L = _lib.lib()
     dev = wav.device
-    T = L.b200vad_fbank_num_frames(N)
+    if sinc is None:
+        T = L.b200vad_fbank_num_frames(N)
+    else:
+        T = L.b200vad_sincnet_num_frames(N)
+        if T < 1:
+            raise _lib.B200VadError("waveform shorter than the SincNet receptive field (991 samples)")
     prob = torch.empty((B, T), dtype=torch.float32, device=dev)
     dec = torch.empty((B, T), dtype=torch.uint8, device=dev)
     counts = torch.zeros(B, dtype=torch.int32, device=dev)
@@ -236,8 +248,7 @@ def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel):
         return prob, dec, torch.empty((0, 3), dtype=torch.int32, device=dev), counts, seg_off
     if B > _MAX_PIPELINE_ROWS:
         raise _lib.B200VadError(f"one pipeline launch handles at most {_MAX_PIPELINE_ROWS} rows (vad_pipeline splits larger batches)")
-    per_row = (T + 2) // 3
-    cap = B * per_row
+    cap = B * _seg_per_row(T, sinc is not None)
     seg = torch.empty((cap, 3), dtype=torch.int32, device=dev)
     with torch.cuda.device(dev):
         _ensure(dev)
@@ -245,15 +256,27 @@ def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel):
         if lens is not None:
             lens = _prep(lens.to(torch.int32), torch.int32, "lens")
             lens_ptr = lens.data_ptr()
-        need = L.b200vad_pipeline_workspace_bytes(B, N)
-        minimum = L.b200vad_pipeline_workspace_bytes(B, N) - L.b200vad_model_workspace_bytes(B, T) + \
-            L.b200vad_model_workspace_bytes(1, T)
-        ws = _ws(min(need, max(_MAX_WS_BYTES, minimum)), dev)
-        fn = L.b200vad_pipeline_fbank_i16 if wav.dtype == torch.int16 else L.b200vad_pipeline_fbank_f32
-        _lib.check(fn(packed.data_ptr(), num_layers, wav.data_ptr(), lens_ptr, B, N, wav.stride(0),
-                      float(thr), int(kernel), prob.data_ptr(), dec.data_ptr(), counts.data_ptr(),
-                      seg_off.data_ptr(), seg.data_ptr(), cap, ws.data_ptr(), ws.numel(),
-                      _stream_ptr(dev)), "b200vad_pipeline_fbank_f32")
+        if sinc is None:
+            need = L.b200vad_pipeline_workspace_bytes(B, N)
+            minimum = L.b200vad_pipeline_workspace_bytes(B, N) - L.b200vad_model_workspace_bytes(B, T) + \
+                L.b200vad_model_workspace_bytes(1, T)
+            ws = _ws(min(need, max(_MAX_WS_BYTES, minimum)), dev)
+            fn = L.b200vad_pipeline_fbank_i16 if wav.dtype == torch.int16 else L.b200vad_pipeline_fbank_f32
+            _lib.check(fn(packed.data_ptr(), num_layers, wav.data_ptr(), lens_ptr, B, N, wav.stride(0),
+                          float(thr), int(kernel), prob.data_ptr(), dec.data_ptr(), counts.data_ptr(),
+                          seg_off.data_ptr(), seg.data_ptr(), cap, ws.data_ptr(), ws.numel(),
+                          _stream_ptr(dev)), "b200vad_pipeline_fbank_f32")
+        else:
+            if lens is not None:
+                raise _lib.B200VadError("the SincNet path takes no lens: pad rows with zero audio, as the reference does")
+            need = L.b200vad_pipeline_sincnet_workspace_bytes(B, N)
+            minimum = 256 * B * T + L.b200vad_pipeline_sincnet_workspace_bytes(1, N)    # + the whole batch's layer-0 planes
+            ws = _ws(min(need, max(_MAX_WS_BYTES, minimum)), dev)
+            fn = L.b200vad_pipeline_sincnet_i16 if wav.dtype == torch.int16 else L.b200vad_pipeline_sincnet_f32
+            _lib.check(fn(packed.data_ptr(), sinc.data_ptr(), num_layers, wav.data_ptr(), B, N, wav.stride(0),
+                          float(thr), int(kernel), prob.data_ptr(), dec.data_ptr(), counts.data_ptr(),
+                          seg_off.data_ptr(), seg.data_ptr(), cap, ws.data_ptr(), ws.numel(),
+                          _stream_ptr(dev)), "b200vad_pipeline_sincnet_f32")
     return prob, dec, seg, counts, seg_off
 
 
@@ -283,15 +306,19 @@ def vad_pipeline(wav: torch.Tensor, lens: Optional[torch.Tensor], packed: torch.
                  kernel: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
     """prob, dec, seg (S, 3), counts.  The exact-size segment list needs S on the host: ONE blocking read of the total per
     call, after everything is enqueued (use vad_pipeline_padded to avoid it).  Batches of more than 65 535 rows are split."""
+    return _pipeline_exact(wav, lens, packed, num_layers, thr, kernel)
+
+
+def _pipeline_exact(wav, lens, packed, num_layers, thr, kernel, sinc=None):
     B = wav.shape[0]
     if B <= _MAX_PIPELINE_ROWS:
-        prob, dec, seg, counts, seg_off = _pipeline_launch(wav, lens, packed, num_layers, thr, kernel)
+        prob, dec, seg, counts, seg_off = _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc)
         total = int(seg_off[B].item()) if B > 0 else 0
         return prob, dec, seg[:total].clone(), counts
     outs = []
     for b0 in range(0, B, _MAX_PIPELINE_ROWS):
         sl = slice(b0, min(B, b0 + _MAX_PIPELINE_ROWS))
-        outs.append((b0,) + _pipeline_launch(wav[sl], None if lens is None else lens[sl], packed, num_layers, thr, kernel))
+        outs.append((b0,) + _pipeline_launch(wav[sl], None if lens is None else lens[sl], packed, num_layers, thr, kernel, sinc))
     segs = []
     for b0, _, _, seg, _, seg_off in outs:
         s = seg[: int(seg_off[-1].item())].clone()
@@ -306,6 +333,47 @@ def _(wav, lens, packed, num_layers, thr, kernel):
     n = ctx.new_dynamic_size()
     B, N = wav.shape
     T = (N + 80) // 160
+    return (wav.new_empty((B, T), dtype=torch.float32), wav.new_empty((B, T), dtype=torch.uint8), wav.new_empty((n, 3), dtype=torch.int32),
+            wav.new_empty((B,), dtype=torch.int32))
+
+
+def _sincnet_frames(N: int) -> int:
+    from .host import get_num_frames
+    return get_num_frames(N)
+
+
+@torch.library.custom_op("b200vad::vad_pipeline_sincnet_padded", mutates_args=(), device_types="cuda")
+def vad_pipeline_sincnet_padded(wav: torch.Tensor, packed_model: torch.Tensor, packed_sincnet: torch.Tensor, num_layers: int,
+                                thr: float, kernel: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """vad_pipeline_padded on the SincNet -> PyanNet path (the reference's feature_extractor="sincnet" flow): prob / dec
+    (B, Ts), Ts = get_num_frames(N); segments keep single-frame runs (predict_sincnet.py:348-370), so the fixed capacity is
+    B * ceil(Ts / 2) rows.  wav: (B, N) float32 or int16 PCM rows, N >= 991; pad short audio with zeros (no lens)."""
+    return _pipeline_launch(wav, None, packed_model, num_layers, thr, kernel, packed_sincnet)
+
+
+@vad_pipeline_sincnet_padded.register_fake
+def _(wav, packed_model, packed_sincnet, num_layers, thr, kernel):
+    B, N = wav.shape
+    T = _sincnet_frames(N)
+    return (wav.new_empty((B, T), dtype=torch.float32), wav.new_empty((B, T), dtype=torch.uint8),
+            wav.new_empty((B * _seg_per_row(T, True), 3), dtype=torch.int32), wav.new_empty((B,), dtype=torch.int32),
+            wav.new_empty((B + 1,), dtype=torch.int64))
+
+
+@torch.library.custom_op("b200vad::vad_pipeline_sincnet", mutates_args=(), device_types="cuda")
+def vad_pipeline_sincnet(wav: torch.Tensor, packed_model: torch.Tensor, packed_sincnet: torch.Tensor, num_layers: int, thr: float,
+                         kernel: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """vad_pipeline on the SincNet -> PyanNet path: prob (B, Ts), dec (B, Ts), seg (S, 3) with single-frame runs kept (min_run
+    1), counts.  One blocking read of the segment total per call; batches of more than 65 535 rows are split."""
+    return _pipeline_exact(wav, None, packed_model, num_layers, thr, kernel, packed_sincnet)
+
+
+@vad_pipeline_sincnet.register_fake
+def _(wav, packed_model, packed_sincnet, num_layers, thr, kernel):
+    ctx = torch.library.get_ctx()
+    n = ctx.new_dynamic_size()
+    B, N = wav.shape
+    T = _sincnet_frames(N)
     return (wav.new_empty((B, T), dtype=torch.float32), wav.new_empty((B, T), dtype=torch.uint8), wav.new_empty((n, 3), dtype=torch.int32),
             wav.new_empty((B,), dtype=torch.int32))
 

@@ -75,20 +75,31 @@ class HostSession:
     three CUDA streams (H2D / compute / D2H).  ``run`` is the blocking form (rows are cut into
     chunks of ``chunk_rows`` and pipelined internally); ``submit`` / ``wait`` is the asynchronous
     form for a caller that streams batches.  Pass pinned tensors (``tensor.pin_memory()``).
+
+    ``sincnet_packed`` (a ``pack_sincnet`` blob; ``packed`` then holds the D = 60 LSTM stack + head) selects the SincNet ->
+    PyanNet path: ``T`` = get_num_frames(num_samples) frames per row, segments keep single-frame runs.
     """
 
     def __init__(self, packed: torch.Tensor, num_layers: int, num_samples: int, chunk_rows: int = 1024,
-                 device: Optional[int] = None):
-        if not packed.is_cuda:
+                 device: Optional[int] = None, sincnet_packed: Optional[torch.Tensor] = None):
+        from .host import fbank_num_frames, get_num_frames
+        from .ops import _seg_per_row
+        if not packed.is_cuda or (sincnet_packed is not None and not sincnet_packed.is_cuda):
             raise _lib.B200VadError("packed weights must live on the GPU")
         self.device = packed.device.index if device is None else device
-        self.packed = packed
+        self.packed, self.sincnet_packed = packed, sincnet_packed
         self.N = int(num_samples)
-        self.T = (self.N + 80) // 160
+        sinc = sincnet_packed is not None
+        self.T = get_num_frames(self.N) if sinc else fbank_num_frames(self.N)
+        self._seg_per_row = _seg_per_row(self.T, sinc)
         self.chunk_rows = int(chunk_rows)
         h = C.c_void_p()
-        _lib.check(_lib.lib().b200vad_session_create(self.device, packed.data_ptr(), num_layers, self.chunk_rows, self.N,
-                                                     C.byref(h)), "b200vad_session_create")
+        if sinc:
+            _lib.check(_lib.lib().b200vad_session_create_sincnet(self.device, packed.data_ptr(), sincnet_packed.data_ptr(), num_layers,
+                                                                 self.chunk_rows, self.N, C.byref(h)), "b200vad_session_create_sincnet")
+        else:
+            _lib.check(_lib.lib().b200vad_session_create(self.device, packed.data_ptr(), num_layers, self.chunk_rows, self.N,
+                                                         C.byref(h)), "b200vad_session_create")
         self._h = h
 
     def run(self, wav: torch.Tensor, thr: float = 0.5, kernel: int = 49, want_dec: bool = True, want_prob: bool = False,
@@ -102,7 +113,7 @@ class HostSession:
             out["dec"] = torch.empty((B, self.T), dtype=torch.uint8).pin_memory()
         if want_prob and ("prob" not in out or out["prob"].shape[0] < B):
             out["prob"] = torch.empty((B, self.T), dtype=torch.float32).pin_memory()
-        cap = B * ((self.T + 2) // 3)
+        cap = B * self._seg_per_row
         if "seg_buf" not in out or out["seg_buf"].shape[0] < cap:
             out["seg_buf"] = torch.empty((max(cap, 1), 3), dtype=torch.int32).pin_memory()
         nseg = C.c_int64(0)
@@ -127,7 +138,7 @@ class HostSession:
             out["dec"] = torch.empty((B, self.T), dtype=torch.uint8).pin_memory()
         if want_prob and ("prob" not in out or out["prob"].shape[0] != B):
             out["prob"] = torch.empty((B, self.T), dtype=torch.float32).pin_memory()
-        cap = B * ((self.T + 2) // 3)
+        cap = B * self._seg_per_row
         if "seg_buf" not in out or out["seg_buf"].shape[0] < cap:
             out["seg_buf"] = torch.empty((max(cap, 1), 3), dtype=torch.int32).pin_memory()
         out["_wav"] = wav          # keep the source alive until wait()

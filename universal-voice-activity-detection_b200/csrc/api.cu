@@ -156,10 +156,11 @@ static int head_forward(const ModelLayout& m, const char* pk, const float* y, in
     return classifier_launch(z2, rows, reinterpret_cast<const float*>(pk + m.wc), reinterpret_cast<const float*>(pk + m.bc), prob, st);
 }
 
-// x: (B, T, D) fp32, or null with the layer-0 input already split into fp16 planes xp_hi / xp_lo (B, T, D), D % 8 == 0
+// x: (B, T, D) fp32, or null with the layer-0 input already split into fp16 planes xp_hi / xp_lo (B, T, round8(D)) whose
+// padding channels are zero (the fused fbank: D = 80; the SincNet front end: D = 60, pitch 64)
 static int model_forward(const void* packed, int D, int L, const float* x, const __half* xp_hi, const __half* xp_lo, int B,
                          int64_t T, float* prob, void* ws, size_t ws_bytes, cudaStream_t st) {
-    B200VAD_CHECK_ARG(packed && (x || (xp_hi && xp_lo && D % 8 == 0 && g_impl == 2)) && prob && ws, "null pointer");
+    B200VAD_CHECK_ARG(packed && (x || (xp_hi && xp_lo && g_impl == 2)) && prob && ws, "null pointer");
     B200VAD_CHECK_ARG(D > 0 && L > 0 && B >= 0 && T >= 0, "bad shape");
     B200VAD_CHECK_ARG((reinterpret_cast<uintptr_t>(ws) & 255) == 0, "workspace must be 256-byte aligned");
     if (B == 0 || T == 0) return B200VAD_OK;
@@ -212,7 +213,7 @@ static int model_forward(const void* packed, int D, int L, const float* x, const
         const __half* a_hi = x_hi;
         const __half* a_lo = x_lo;
         if (!xin) {
-            a_hi = xp_hi + b0 * T * D; a_lo = xp_lo + b0 * T * D;                  // planes straight from the fused fbank
+            a_hi = xp_hi + b0 * T * D8; a_lo = xp_lo + b0 * T * D8;                // planes straight from the front end
         } else {
             if (D % 8 == 0) rc = split_planes_launch(xin, rows * D, x_hi, x_lo, st);
             else rc = split_planes_pad_launch(xin, rows, D, D8, x_hi, x_lo, st);   // e.g. the 60 SincNet channels -> pitch 64
@@ -301,6 +302,7 @@ struct SincLayout {
 };
 // tcgen05 path: weights zero padded to 128 output rows; conv2's 60 input channels are padded to 64 (16-byte rows)
 constexpr int kSincTLd = 256, kC1TLd = 448, kC2Cp = 64, kC2TLd = 5 * kC2Cp;
+constexpr int kSincStep = 270;   // samples between SincNet frames: 10 x 3 x 3 x 3 (receptive_field.py)
 constexpr int kSincK = 251, kSincKp = 256, kC1K = 400, kC1Kp = 416, kC2K = 300, kC2Kp = 320;
 static SincLayout sinc_layout() {
     SincLayout s;
@@ -349,6 +351,10 @@ static bool sinc_fused() {
     return fused != 0;
 }
 static inline int64_t sinc_np(int64_t N) { return (N + 16 + 7) / 8 * 8; }     // padded length of a shifted waveform copy
+// rows per front-end launch: the warp-MMA GEMM grid limit (65000 x 128 conv rows) and the per-row kernels' grid.y
+static int64_t sinc_chunk_rows(int64_t N) {
+    return std::min<int64_t>(60000, std::max<int64_t>(1, 65000LL * 128 / std::max<int64_t>(sinc_dims(N).L1, 1)));
+}
 static size_t sinc_ws_per_row(int64_t N) {
     SincDims d = sinc_dims(N);
     // normalised wave (fp32, or 4 shifted fp16 hi/lo copies) + conv1 out + pooled1 (+ planes) + conv2 out + pooled2 (+ planes)
@@ -635,21 +641,29 @@ size_t b200vad_sincnet_workspace_bytes(int B, int64_t N) {
     return (size_t)B * sinc_ws_per_row(N) + 4096;
 }
 
-int b200vad_sincnet_forward_f32(const void* packed, const float* wav, int B, int64_t N, int64_t wav_stride, float* out,
-                                void* workspace, size_t ws_bytes, void* stream) {
-    B200VAD_CHECK_ARG(packed && wav && out && workspace, "null pointer");
-    B200VAD_CHECK_ARG(B >= 0 && N >= 0 && wav_stride >= N, "bad shape");
+// SincNet front end on (B, N) rows `wav_stride` samples apart (f32, or int16 PCM with wav_i16), in chunks of rows that fit
+// the workspace.  Output: `out` (B, Ts, 60) f32, or -- tcgen05 path, o_hi / o_lo given -- the LSTM's layer-0 operand as fp16
+// (hi, lo) planes (B, Ts, 64) with channels 60..63 zero: the unscaled split of split_planes_pad_kernel, so model_forward sees
+// the same bits either way, without the fp32 round trip through HBM and the split pass.  Every chunk writes its own rows of
+// the whole-batch output.
+static int sincnet_forward(const void* packed, const void* wav, int wav_i16, int B, int64_t N, int64_t wav_stride, float* out,
+                           __half* o_hi, __half* o_lo, void* workspace, size_t ws_bytes, cudaStream_t st) {
+    const bool planes = o_hi != nullptr;
+    B200VAD_CHECK_ARG(packed && wav && (out || (o_hi && o_lo)) && workspace, "null pointer");
+    B200VAD_CHECK_ARG(B >= 0 && N >= 0 && wav_stride >= 1, "bad shape");
     B200VAD_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "workspace must be 256-byte aligned");
     const SincDims d = sinc_dims(N);
     B200VAD_CHECK_ARG(d.P3 >= 1, "waveform shorter than the SincNet receptive field (991 samples)");
+    if ((planes || wav_i16) && g_impl != 2) {
+        set_error("sincnet: int16 input and plane output need the tcgen05 path (b200vad_set_impl(2))");
+        return B200VAD_ESTATE;
+    }
     if (B == 0) return B200VAD_OK;
-    cudaStream_t st = (cudaStream_t)stream;
     const SincLayout s = sinc_layout();
     const char* pk = reinterpret_cast<const char*>(packed);
     const size_t per_row = sinc_ws_per_row(N);
     int64_t Bc = std::min<int64_t>((int64_t)(ws_bytes / per_row), B);
-    Bc = std::min<int64_t>(Bc, 60000);
-    Bc = std::min<int64_t>(Bc, std::max<int64_t>(1, 65000LL * 128 / std::max<int64_t>(d.L1, 1)));
+    Bc = std::min<int64_t>(Bc, sinc_chunk_rows(N));
     if (Bc < 1) {
         set_error("sincnet_forward: workspace too small (%zu bytes; need >= %zu per row)", ws_bytes, per_row);
         return B200VAD_ENOMEM;
@@ -672,13 +686,16 @@ int b200vad_sincnet_forward_f32(const void* packed, const float* wav, int B, int
         __half* p2_lo = p2_hi + d.P2 * kC2Cp * bc;
         float* c3 = fused_convs ? nullptr : reinterpret_cast<float*>(take(sizeof(float) * d.L3 * 60 * bc));
         double* stats = reinterpret_cast<double*>(take(sizeof(double) * 2 * 80 * bc));
+        __half* const o3_hi = planes ? o_hi + b0 * d.P3 * kC2Cp : nullptr;
+        __half* const o3_lo = planes ? o_lo + b0 * d.P3 * kC2Cp : nullptr;
         int rc;
         if (g_impl == 2) {
             // ---- tcgen05 path: every convolution is an overlapping-row GEMM on gemm_ts (weights resident in TMEM)
             const int sms = num_sms_cached();
             __half* wn_hi = reinterpret_cast<__half*>(wn_raw);
             __half* wn_lo = wn_hi + 4 * (int64_t)bc * Np;
-            if ((rc = wave_norm_planes_launch(wav + b0 * wav_stride, bc, N, wav_stride, Np, reinterpret_cast<const float*>(pk + s.wn_w),
+            const void* wrow = reinterpret_cast<const char*>(wav) + (wav_i16 ? sizeof(int16_t) : sizeof(float)) * b0 * wav_stride;
+            if ((rc = wave_norm_planes_launch(wrow, wav_i16, bc, N, wav_stride, Np, reinterpret_cast<const float*>(pk + s.wn_w),
                                               reinterpret_cast<const float*>(pk + s.wn_b), stats, wn_hi, wn_lo, st, 0))) return rc;
             if (sinc_fused()) {
                 // (three fp16 products per k-step: the 2-product scheme of the LSTM projections costs 3e-3 on the normalised SincNet
@@ -718,12 +735,12 @@ int b200vad_sincnet_forward_f32(const void* packed, const float* wav, int B, int
                                                 sms, st))) return rc;
                 if ((rc = norm_lrelu_launch(p2, bc, d.P2, 60, stats, reinterpret_cast<const float*>(pk + s.n1_w),
                                             reinterpret_cast<const float*>(pk + s.n1_b), st, p2_hi, p2_lo, kC2Cp, 0))) return rc;
-                float* o3 = out + b0 * d.P3 * 60;
+                float* o3 = planes ? p2 : out + b0 * d.P3 * 60;     // plane output: the dead pooled2 buffer takes the fp32 values
                 if ((rc = zero_f64_launch(stats, (int64_t)2 * bc * 60, st))) return rc;
                 if ((rc = conv_pool_gemm_launch(p2_hi, p2_lo, kC2Cp, d.P2 * kC2Cp, bc, d.L3, kC2TLd, w2h, w2l, kC2TLd, kC2TLd, 60, b2, 3, o3, 60,
                                                 stats, sms, st))) return rc;
                 if ((rc = norm_lrelu_launch(o3, bc, d.P3, 60, stats, reinterpret_cast<const float*>(pk + s.n2_w),
-                                            reinterpret_cast<const float*>(pk + s.n2_b), st))) return rc;
+                                            reinterpret_cast<const float*>(pk + s.n2_b), st, o3_hi, o3_lo, kC2Cp, 0))) return rc;
                 continue;
             }
             // Conv1d(80, 60, 5): row t = p1[b, t : t + 5, :] = 400 contiguous values, K split 256 + 144
@@ -738,12 +755,13 @@ int b200vad_sincnet_forward_f32(const void* packed, const float* wav, int B, int
                                           60, d.L3, 1, 0, sms, st))) return rc;
             if ((rc = gemm_ts_rows_launch(p2_hi + 256, p2_lo + 256, kC2Cp, d.P2 * kC2Cp, bc, (int)d.L3, 64, w2h + 256, w2l + 256, 64,
                                           kC2TLd, 60, nullptr, 1, 0, c3, 60, d.L3, 1, 0, sms, st))) return rc;
-            if ((rc = pool_norm_lrelu_launch(c3, bc, d.L3, 60, out + b0 * d.P3 * 60, stats, reinterpret_cast<const float*>(pk + s.n2_w),
-                                             reinterpret_cast<const float*>(pk + s.n2_b), st))) return rc;
+            if ((rc = pool_norm_lrelu_launch(c3, bc, d.L3, 60, planes ? p2 : out + b0 * d.P3 * 60, stats,
+                                             reinterpret_cast<const float*>(pk + s.n2_w), reinterpret_cast<const float*>(pk + s.n2_b), st,
+                                             o3_hi, o3_lo, kC2Cp))) return rc;
             continue;
         }
         // ---- warp-MMA validation path
-        rc = wave_instnorm_launch(wav + b0 * wav_stride, bc, N, wav_stride, reinterpret_cast<const float*>(pk + s.wn_w),
+        rc = wave_instnorm_launch(reinterpret_cast<const float*>(wav) + b0 * wav_stride, bc, N, wav_stride, reinterpret_cast<const float*>(pk + s.wn_w),
                                   reinterpret_cast<const float*>(pk + s.wn_b), stats, wn, st);
         if (rc) return rc;
         GemmArgs g;
@@ -778,6 +796,12 @@ int b200vad_sincnet_forward_f32(const void* packed, const float* wav, int B, int
         if (rc) return rc;
     }
     return B200VAD_OK;
+}
+
+int b200vad_sincnet_forward_f32(const void* packed, const float* wav, int B, int64_t N, int64_t wav_stride, float* out,
+                                void* workspace, size_t ws_bytes, void* stream) {
+    B200VAD_CHECK_ARG(wav_stride >= N, "bad shape");
+    return sincnet_forward(packed, wav, 0, B, N, wav_stride, out, nullptr, nullptr, workspace, ws_bytes, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------- post-processing
@@ -844,61 +868,110 @@ int b200vad_stitch_center(const float* prob, int num_windows, int frames_per_win
 }
 
 // ---------------------------------------------------------------- fused device pipeline
-static size_t pipeline_ws_bytes(int B, int64_t N) {
-    int64_t T = b200vad_fbank_num_frames(N);
-    return align_up(sizeof(float) * (size_t)B * T * kNumMel) + align_up(sizeof(double) * B) +
-           b200vad_model_workspace_bytes(B, T) + 4096;
+// Front end of the whole path: the fused fbank (sinc == nullptr: a1 -> PyanNet2) or SincNet with its packed blob (a3/a4 ->
+// PyanNet).  Both hand the LSTM its layer-0 operand as fp16 (hi, lo) planes with row pitch round8(D).
+static inline int64_t fe_frames(bool sinc, int64_t N) { return sinc ? sinc_dims(N).P3 : b200vad_fbank_num_frames(N); }
+static inline int fe_dim(bool sinc) { return sinc ? 60 : kNumMel; }
+// segments per row at most: runs of >= 2 frames (fbank) are ceil(T / 3) apart, the SincNet RLE keeps single-frame runs
+// (predict_sincnet.py:348-370): ceil(T / 2)
+static inline int64_t fe_max_seg_per_row(bool sinc, int64_t T) { return sinc ? (T + 1) / 2 : (T + 2) / 3; }
+// layout: layer-0 input (fp32 features or planes, the same bytes) | fbank row sums | model workspace; the SincNet front end's
+// workspace shares the model's region (it is dead before the model runs on the same stream)
+static size_t fe_feat_bytes(bool sinc, int B, int64_t T) { return align_up(sizeof(float) * (size_t)B * T * round8(fe_dim(sinc))); }
+static size_t fe_sums_bytes(bool sinc, int B) { return sinc ? 0 : align_up(sizeof(double) * B); }
+static size_t pipeline_ws_bytes(int B, int64_t N, bool sinc = false) {
+    const int64_t T = fe_frames(sinc, N);
+    size_t rest = b200vad_model_workspace_bytes(B, T);
+    if (sinc) rest = std::max(rest, (size_t)std::min<int64_t>(B, sinc_chunk_rows(N)) * sinc_ws_per_row(N) + 4096);
+    return fe_feat_bytes(sinc, B, T) + fe_sums_bytes(sinc, B) + rest + 4096;
 }
 size_t b200vad_pipeline_workspace_bytes(int B, int64_t N) {
     if (B <= 0 || N <= 0) return 0;
     return pipeline_ws_bytes(B, N);
 }
+size_t b200vad_pipeline_sincnet_workspace_bytes(int B, int64_t N) {
+    if (B <= 0 || N < 991) return 0;
+    return pipeline_ws_bytes(B, N, true);
+}
 
-static int pipeline_run(const void* packed, int L, const void* wav, int wav_i16, const int32_t* lens, int B, int64_t N, int64_t stride,
-                        float thr, int kernel, int row_base, float* prob, uint8_t* dec, int32_t* counts, int64_t* seg_off,
-                        int32_t* seg, int64_t cap, void* ws, size_t ws_bytes, cudaStream_t st) {
+static int pipeline_run(const void* packed, const void* sinc, int L, const void* wav, int wav_i16, const int32_t* lens, int B,
+                        int64_t N, int64_t stride, float thr, int kernel, int row_base, float* prob, uint8_t* dec, int32_t* counts,
+                        int64_t* seg_off, int32_t* seg, int64_t cap, void* ws, size_t ws_bytes, cudaStream_t st) {
     B200VAD_CHECK_ARG(packed && wav && prob && dec && counts && seg_off && ws, "null pointer");
     B200VAD_CHECK_ARG((reinterpret_cast<uintptr_t>(ws) & 255) == 0, "workspace must be 256-byte aligned");
-    const int64_t T = b200vad_fbank_num_frames(N);
+    const int64_t T = fe_frames(sinc != nullptr, N);
+    const int D = fe_dim(sinc != nullptr);
     if (B == 0 || T == 0) return B200VAD_OK;
     char* w = reinterpret_cast<char*>(ws);
-    float* feats = reinterpret_cast<float*>(w); w += align_up(sizeof(float) * (size_t)B * T * kNumMel);
-    double* sums = reinterpret_cast<double*>(w); w += align_up(sizeof(double) * B);
+    float* feats = reinterpret_cast<float*>(w); w += fe_feat_bytes(sinc != nullptr, B, T);
+    double* sums = reinterpret_cast<double*>(w); w += fe_sums_bytes(sinc != nullptr, B);
     size_t used = (size_t)(w - reinterpret_cast<char*>(ws));
-    if (ws_bytes < used + b200vad_model_workspace_bytes(1, T)) {
+    const size_t rest_min = sinc ? std::max(b200vad_model_workspace_bytes(1, T), sinc_ws_per_row(N)) : b200vad_model_workspace_bytes(1, T);
+    if (ws_bytes < used + rest_min) {
         set_error("pipeline: workspace too small (%zu bytes)", ws_bytes);
         return B200VAD_ENOMEM;
     }
-    int dev = 0;
-    B200VAD_CUDA(cudaGetDevice(&dev));
-    // the tcgen05 path takes the features as fp16 (hi, lo) planes straight from the fbank kernel (same bytes as fp32)
+    // the tcgen05 path takes the layer-0 input as fp16 (hi, lo) planes straight from the front end (same bytes as fp32)
     __half* f_hi = reinterpret_cast<__half*>(feats);
-    __half* f_lo = f_hi + (size_t)B * T * kNumMel;
+    __half* f_lo = f_hi + (size_t)B * T * round8(D);
     const bool planes = g_impl == 2;
-    int rc = fbank_launch(wav, wav_i16, lens, B, N, stride, planes ? nullptr : feats, planes ? f_hi : nullptr, planes ? f_lo : nullptr, T,
+    int rc;
+    if (sinc) {
+        if (!planes) {
+            set_error("pipeline: the SincNet front end runs on the tcgen05 path only (b200vad_set_impl(2))");
+            return B200VAD_ESTATE;
+        }
+        rc = sincnet_forward(sinc, wav, wav_i16, B, N, stride, nullptr, f_hi, f_lo, w, ws_bytes - used, st);
+    } else {
+        int dev = 0;
+        B200VAD_CUDA(cudaGetDevice(&dev));
+        rc = fbank_launch(wav, wav_i16, lens, B, N, stride, planes ? nullptr : feats, planes ? f_hi : nullptr, planes ? f_lo : nullptr, T,
                           sums, dev, st);
+    }
     if (rc) return rc;
-    rc = model_forward(packed, kNumMel, L, planes ? nullptr : feats, f_hi, f_lo, B, T, prob, w, ws_bytes - used, st);
+    rc = model_forward(packed, D, L, planes ? nullptr : feats, f_hi, f_lo, B, T, prob, w, ws_bytes - used, st);
     if (rc) return rc;
     rc = threshold_median_launch(prob, B, T, thr, kernel, dec, 1, nullptr, 0.f, st);
     if (rc) return rc;
-    return segments_launch(dec, nullptr, T, B, 2, row_base, counts, seg_off, seg, cap, st);
+    return segments_launch(dec, nullptr, T, B, sinc ? 1 : 2, row_base, counts, seg_off, seg, cap, st);
 }
 
 int b200vad_pipeline_fbank_f32(const void* packed, int L, const float* wav, const int32_t* lens, int B, int64_t N,
                                int64_t stride, float thr, int kernel, float* prob, uint8_t* dec, int32_t* counts,
                                int64_t* seg_off, int32_t* seg, int64_t cap, void* ws, size_t ws_bytes, void* stream) {
     B200VAD_CHECK_ARG(B >= 0 && B <= 65535 && N >= 1 && stride >= 1, "bad shape");
-    return pipeline_run(packed, L, wav, 0, lens, B, N, stride, thr, kernel, 0, prob, dec, counts, seg_off, seg, cap, ws, ws_bytes,
-                        (cudaStream_t)stream);
+    return pipeline_run(packed, nullptr, L, wav, 0, lens, B, N, stride, thr, kernel, 0, prob, dec, counts, seg_off, seg, cap, ws,
+                        ws_bytes, (cudaStream_t)stream);
 }
 
 int b200vad_pipeline_fbank_i16(const void* packed, int L, const int16_t* wav, const int32_t* lens, int B, int64_t N,
                                int64_t stride, float thr, int kernel, float* prob, uint8_t* dec, int32_t* counts,
                                int64_t* seg_off, int32_t* seg, int64_t cap, void* ws, size_t ws_bytes, void* stream) {
     B200VAD_CHECK_ARG(B >= 0 && B <= 65535 && N >= 1 && stride >= 1, "bad shape");
-    return pipeline_run(packed, L, wav, 1, lens, B, N, stride, thr, kernel, 0, prob, dec, counts, seg_off, seg, cap, ws, ws_bytes,
-                        (cudaStream_t)stream);
+    return pipeline_run(packed, nullptr, L, wav, 1, lens, B, N, stride, thr, kernel, 0, prob, dec, counts, seg_off, seg, cap, ws,
+                        ws_bytes, (cudaStream_t)stream);
+}
+
+static int pipeline_sincnet_entry(const void* packed, const void* sinc, int L, const void* wav, int wav_i16, int B, int64_t N,
+                                  int64_t stride, float thr, int kernel, float* prob, uint8_t* dec, int32_t* counts, int64_t* seg_off,
+                                  int32_t* seg, int64_t cap, void* ws, size_t ws_bytes, void* stream) {
+    B200VAD_CHECK_ARG(sinc, "null pointer");
+    B200VAD_CHECK_ARG(L > 0 && B >= 0 && B <= 65535 && stride >= 1 && cap >= 0, "bad shape");
+    B200VAD_CHECK_ARG(N >= 991, "waveform shorter than the SincNet receptive field (991 samples)");
+    return pipeline_run(packed, sinc, L, wav, wav_i16, nullptr, B, N, stride, thr, kernel, 0, prob, dec, counts, seg_off, seg, cap, ws,
+                        ws_bytes, (cudaStream_t)stream);
+}
+int b200vad_pipeline_sincnet_f32(const void* packed_model, const void* packed_sincnet, int num_layers, const float* wav, int B,
+                                 int64_t N, int64_t wav_stride, float thr, int kernel, float* prob, uint8_t* dec, int32_t* counts,
+                                 int64_t* seg_off, int32_t* seg, int64_t cap, void* ws, size_t ws_bytes, void* stream) {
+    return pipeline_sincnet_entry(packed_model, packed_sincnet, num_layers, wav, 0, B, N, wav_stride, thr, kernel, prob, dec, counts,
+                                  seg_off, seg, cap, ws, ws_bytes, stream);
+}
+int b200vad_pipeline_sincnet_i16(const void* packed_model, const void* packed_sincnet, int num_layers, const int16_t* wav, int B,
+                                 int64_t N, int64_t wav_stride, float thr, int kernel, float* prob, uint8_t* dec, int32_t* counts,
+                                 int64_t* seg_off, int32_t* seg, int64_t cap, void* ws, size_t ws_bytes, void* stream) {
+    return pipeline_sincnet_entry(packed_model, packed_sincnet, num_layers, wav, 1, B, N, wav_stride, thr, kernel, prob, dec, counts,
+                                  seg_off, seg, cap, ws, ws_bytes, stream);
 }
 
 // ---------------------------------------------------------------- host-buffer session
@@ -919,6 +992,7 @@ struct SessionSlot {
 struct b200vad_session {
     int device;
     const void* packed;
+    const void* sinc;       // packed SincNet blob (SincNet -> PyanNet path), or null (fbank -> PyanNet2)
     int L;
     int chunk;
     int64_t N, T, max_seg_per_row;
@@ -929,17 +1003,18 @@ struct b200vad_session {
     size_t ws_bytes;
 };
 
-int b200vad_session_create(int device, const void* packed_device, int num_layers, int max_chunk_rows, int64_t N,
-                           b200vad_session** out) {
+static int session_create(int device, const void* packed_device, const void* sinc, int num_layers, int max_chunk_rows, int64_t N,
+                          b200vad_session** out) {
     B200VAD_CHECK_ARG(out && packed_device, "null pointer");
     B200VAD_CHECK_ARG(num_layers > 0 && max_chunk_rows > 0 && max_chunk_rows <= 65535 && N >= 1, "bad shape");
+    B200VAD_CHECK_ARG(!sinc || N >= 991, "waveform shorter than the SincNet receptive field (991 samples)");
     int rc = b200vad_init(device);
     if (rc) return rc;
     b200vad_session* s = new b200vad_session();
     memset(s, 0, sizeof(*s));
-    s->device = device; s->packed = packed_device; s->L = num_layers; s->chunk = max_chunk_rows; s->N = N;
-    s->T = b200vad_fbank_num_frames(N);
-    s->max_seg_per_row = (s->T + 2) / 3;
+    s->device = device; s->packed = packed_device; s->sinc = sinc; s->L = num_layers; s->chunk = max_chunk_rows; s->N = N;
+    s->T = fe_frames(sinc != nullptr, N);
+    s->max_seg_per_row = fe_max_seg_per_row(sinc != nullptr, s->T);
     cudaError_t e = cudaSuccess;
     auto ok = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
     ok(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
@@ -961,7 +1036,7 @@ int b200vad_session_create(int device, const void* packed_device, int num_layers
         ok(cudaMalloc(&sl.seg_dev, sizeof(int32_t) * 3 * (size_t)s->chunk * s->max_seg_per_row));
         ok(cudaMallocHost(&sl.total_host, sizeof(int64_t)));
     }
-    s->ws_bytes = pipeline_ws_bytes(s->chunk, N);
+    s->ws_bytes = pipeline_ws_bytes(s->chunk, N, sinc != nullptr);
     ok(cudaMalloc(&s->ws, s->ws_bytes));
     ok(cudaEventCreate(&s->epoch));
     ok(cudaEventRecord(s->epoch, s->copy_stream));
@@ -972,6 +1047,15 @@ int b200vad_session_create(int device, const void* packed_device, int num_layers
     }
     *out = s;
     return B200VAD_OK;
+}
+int b200vad_session_create(int device, const void* packed_device, int num_layers, int max_chunk_rows, int64_t N,
+                           b200vad_session** out) {
+    return session_create(device, packed_device, nullptr, num_layers, max_chunk_rows, N, out);
+}
+int b200vad_session_create_sincnet(int device, const void* packed_model, const void* packed_sincnet, int num_layers,
+                                   int max_chunk_rows, int64_t N, b200vad_session** out) {
+    B200VAD_CHECK_ARG(packed_sincnet, "null pointer");
+    return session_create(device, packed_model, packed_sincnet, num_layers, max_chunk_rows, N, out);
 }
 
 static int session_submit(b200vad_session* s, int slot, const void* wav_host, int wav_i16, int B, int row_base, float thr, int kernel,
@@ -984,7 +1068,7 @@ static int session_submit(b200vad_session* s, int slot, const void* wav_host, in
     B200VAD_CUDA(cudaEventRecord(sl.copied, s->copy_stream));
     B200VAD_CUDA(cudaStreamWaitEvent(s->compute_stream, sl.copied, 0));
     B200VAD_CUDA(cudaEventRecord(sl.compute_begin, s->compute_stream));
-    int rc = pipeline_run(s->packed, s->L, sl.wav_dev, wav_i16, nullptr, B, N, N, thr, kernel, row_base, sl.prob_dev, sl.dec_dev,
+    int rc = pipeline_run(s->packed, s->sinc, s->L, sl.wav_dev, wav_i16, nullptr, B, N, N, thr, kernel, row_base, sl.prob_dev, sl.dec_dev,
                           sl.counts_dev, sl.seg_off_dev, sl.seg_dev, (int64_t)B * s->max_seg_per_row, s->ws, s->ws_bytes,
                           s->compute_stream);
     if (rc) return rc;
@@ -1131,6 +1215,7 @@ void b200vad_session_destroy(b200vad_session* s) {
 struct b200vad_stream {
     int device;
     const void* packed;
+    const void* sinc;       // packed SincNet blob, or null (fbank front end)
     int L, S, hop, nf, pos;
     int64_t W, T;
     float thr;
@@ -1148,11 +1233,13 @@ struct b200vad_stream {
 };
 
 static int stream_forward(b200vad_stream* s) {
+    const int D = fe_dim(s->sinc != nullptr);
     __half* f_hi = reinterpret_cast<__half*>(s->feats);
-    __half* f_lo = f_hi + (size_t)s->S * s->T * kNumMel;
-    int rc = fbank_launch(s->lin, 0, nullptr, s->S, s->W, s->W, nullptr, f_hi, f_lo, s->T, s->sums, s->device, s->st);
+    __half* f_lo = f_hi + (size_t)s->S * s->T * round8(D);
+    int rc = s->sinc ? sincnet_forward(s->sinc, s->lin, 0, s->S, s->W, s->W, nullptr, f_hi, f_lo, s->ws, s->ws_bytes, s->st)
+                     : fbank_launch(s->lin, 0, nullptr, s->S, s->W, s->W, nullptr, f_hi, f_lo, s->T, s->sums, s->device, s->st);
     if (rc) return rc;
-    rc = model_forward(s->packed, kNumMel, s->L, nullptr, f_hi, f_lo, s->S, s->T, s->prob, s->ws, s->ws_bytes, s->st);
+    rc = model_forward(s->packed, D, s->L, nullptr, f_hi, f_lo, s->S, s->T, s->prob, s->ws, s->ws_bytes, s->st);
     if (rc) return rc;
     rc = threshold_median_launch(s->prob, s->S, s->T, s->thr, s->kernel, s->dec, 1, nullptr, 0.f, s->st);
     if (rc) return rc;
@@ -1174,19 +1261,26 @@ static int stream_capture(b200vad_stream* s) {
     return B200VAD_OK;
 }
 
-int b200vad_stream_create(int device, const void* packed_device, int num_layers, int num_streams, int64_t window_samples,
-                          int hop_samples, int use_graph, b200vad_stream** out) {
+static int stream_create(int device, const void* packed_device, const void* sinc, int num_layers, int num_streams,
+                         int64_t window_samples, int hop_samples, int use_graph, b200vad_stream** out) {
     B200VAD_CHECK_ARG(out && packed_device, "null pointer");
     B200VAD_CHECK_ARG(num_layers > 0 && num_streams > 0 && num_streams <= 65535, "bad shape");
-    B200VAD_CHECK_ARG(hop_samples > 0 && hop_samples % kFrameShift == 0 && window_samples % kFrameShift == 0 &&
-                          window_samples >= hop_samples && window_samples <= (1 << 30),
-                      "window and hop must be multiples of 160 samples, hop <= window");
+    if (sinc) {
+        // frames of consecutive windows fall on one grid only when the hop is a whole number of SincNet frame steps
+        B200VAD_CHECK_ARG(hop_samples > 0 && hop_samples % kSincStep == 0 && window_samples >= 991 && window_samples >= hop_samples &&
+                              window_samples <= (1 << 30) && hop_samples / kSincStep <= sinc_dims(window_samples).P3,
+                          "SincNet streaming: hop must be a multiple of 270 samples, window >= 991 samples, hop <= window");
+    } else {
+        B200VAD_CHECK_ARG(hop_samples > 0 && hop_samples % kFrameShift == 0 && window_samples % kFrameShift == 0 &&
+                              window_samples >= hop_samples && window_samples <= (1 << 30),
+                          "window and hop must be multiples of 160 samples, hop <= window");
+    }
     int rc = b200vad_init(device);
     if (rc) return rc;
     b200vad_stream* s = new b200vad_stream();
     memset(s, 0, sizeof(*s));
-    s->device = device; s->packed = packed_device; s->L = num_layers; s->S = num_streams; s->hop = hop_samples;
-    s->W = window_samples; s->T = b200vad_fbank_num_frames(window_samples); s->nf = hop_samples / kFrameShift;
+    s->device = device; s->packed = packed_device; s->sinc = sinc; s->L = num_layers; s->S = num_streams; s->hop = hop_samples;
+    s->W = window_samples; s->T = fe_frames(sinc != nullptr, window_samples); s->nf = hop_samples / (sinc ? kSincStep : kFrameShift);
     s->thr = 0.5f; s->kernel = 49; s->use_graph = use_graph != 0;
     cudaError_t e = cudaSuccess;
     auto ok = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
@@ -1196,7 +1290,7 @@ int b200vad_stream_create(int device, const void* packed_device, int num_layers,
     ok(cudaMalloc(&s->ring, sizeof(float) * S * 2 * W));
     ok(cudaMalloc(&s->lin, sizeof(float) * S * W));
     ok(cudaMalloc(&s->chunk, sizeof(float) * S * s->hop));
-    ok(cudaMalloc(&s->feats, sizeof(float) * S * T * kNumMel));
+    ok(cudaMalloc(&s->feats, sizeof(float) * S * T * round8(fe_dim(sinc != nullptr))));
     ok(cudaMalloc(&s->sums, sizeof(double) * S));
     ok(cudaMalloc(&s->prob, sizeof(float) * S * T));
     ok(cudaMalloc(&s->dec, S * T));
@@ -1205,6 +1299,8 @@ int b200vad_stream_create(int device, const void* packed_device, int num_layers,
     ok(cudaMallocHost(&s->prob_new_host, sizeof(float) * S * s->nf));
     ok(cudaMallocHost(&s->dec_new_host, S * s->nf));
     s->ws_bytes = b200vad_model_workspace_bytes(s->S, s->T);
+    if (sinc)   // the front end's workspace is dead before the model runs on the same stream
+        s->ws_bytes = std::max(s->ws_bytes, (size_t)std::min<int64_t>(s->S, sinc_chunk_rows(s->W)) * sinc_ws_per_row(s->W) + 4096);
     ok(cudaMalloc(&s->ws, s->ws_bytes));
     if (e == cudaSuccess) ok(cudaMemsetAsync(s->ring, 0, sizeof(float) * S * 2 * W, s->st));
     if (e == cudaSuccess) ok(cudaMemsetAsync(s->lin, 0, sizeof(float) * S * W, s->st));
@@ -1216,6 +1312,15 @@ int b200vad_stream_create(int device, const void* packed_device, int num_layers,
     if (s->use_graph && (rc = stream_capture(s))) { b200vad_stream_destroy(s); return rc; }
     *out = s;
     return B200VAD_OK;
+}
+int b200vad_stream_create(int device, const void* packed_device, int num_layers, int num_streams, int64_t window_samples,
+                          int hop_samples, int use_graph, b200vad_stream** out) {
+    return stream_create(device, packed_device, nullptr, num_layers, num_streams, window_samples, hop_samples, use_graph, out);
+}
+int b200vad_stream_create_sincnet(int device, const void* packed_model, const void* packed_sincnet, int num_layers, int num_streams,
+                                  int64_t window_samples, int hop_samples, int use_graph, b200vad_stream** out) {
+    B200VAD_CHECK_ARG(packed_sincnet, "null pointer");
+    return stream_create(device, packed_model, packed_sincnet, num_layers, num_streams, window_samples, hop_samples, use_graph, out);
 }
 
 int b200vad_stream_push(b200vad_stream* s, const float* chunk, int chunk_on_host, float thr, int kernel, float* prob_new_host,

@@ -89,8 +89,9 @@ int norm_lrelu_launch(float* pooled, int B, int64_t P, int C, const double* stat
                       cudaStream_t s, __half* p_hi = nullptr, __half* p_lo = nullptr, int Cp = 0, int scaled_planes = 0);
 int pool_norm_lrelu_launch(const float* in, int B, int64_t L, int C, float* pooled, double* stats, const float* gamma,
                            const float* beta, cudaStream_t s, __half* p_hi = nullptr, __half* p_lo = nullptr, int Cp = 0, int scaled_planes = 0);
-int wave_norm_planes_launch(const float* wav, int B, int64_t N, int64_t stride, int64_t Np, const float* gamma, const float* beta,
-                            double* stats, __half* hi, __half* lo, cudaStream_t s, int scaled_planes = 0);
+// wav: (B, N) f32 rows, or int16 PCM rows (wav_i16 != 0; samples int16 / 32768), `stride` elements apart
+int wave_norm_planes_launch(const void* wav, int wav_i16, int B, int64_t N, int64_t stride, int64_t Np, const float* gamma,
+                            const float* beta, double* stats, __half* hi, __half* lo, cudaStream_t s, int scaled_planes = 0);
 int pad_rows_launch(const float* w, int Cout, int K, int ld, float* out, cudaStream_t s);
 int repack_conv_pad_launch(const float* w, int Cout, int Cin, int k, int Cp, int ld, float* out, cudaStream_t s);
 

@@ -209,9 +209,14 @@ stream_append_kernel(float* __restrict__ ring, const float* __restrict__ chunk, 
 __global__ void __launch_bounds__(256)
 stream_linearise_kernel(const float* __restrict__ ring, float* __restrict__ lin, int S, int Wn, int start) {
     const int s = blockIdx.y;
-    const float4* src = reinterpret_cast<const float4*>(ring + (int64_t)s * 2 * Wn + start);
-    float4* dst = reinterpret_cast<float4*>(lin + (int64_t)s * Wn);
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < Wn / 4; i += gridDim.x * blockDim.x) dst[i] = __ldg(src + i);
+    const float* src = ring + (int64_t)s * 2 * Wn + start;
+    float* dst = lin + (int64_t)s * Wn;
+    if (((Wn | start) & 3) == 0) {
+        for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < Wn / 4; i += gridDim.x * blockDim.x)
+            reinterpret_cast<float4*>(dst)[i] = __ldg(reinterpret_cast<const float4*>(src) + i);
+    } else {   // SincNet hops (multiples of 270 samples) leave the window start off 16-byte boundaries
+        for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < Wn; i += gridDim.x * blockDim.x) dst[i] = __ldg(src + i);
+    }
 }
 // newest `nf` frames of every stream: prob (S, T) / dec (S, T) -> (S, nf)
 __global__ void stream_newest_kernel(const float* __restrict__ prob, const uint8_t* __restrict__ dec, int S, int64_t T, int nf,

@@ -66,16 +66,22 @@ int repack_conv_launch(const float* w, int Cout, int Cin, int k, float* out, cud
 }
 
 // ---------------------------------------------------------------- waveform instance norm
+// Samples are fp32, or 16-bit PCM converted as an audio loader does (int16 / 32768, exact): every later operation sees the
+// same floats, so the output from int16 input equals the output from the converted fp32 waveform bit for bit.
+__device__ __forceinline__ float sample_f32(float v) { return v; }
+__device__ __forceinline__ float sample_f32(int16_t v) { return (float)v * (1.f / 32768.f); }
+
 // stats[b] = (sum, sumsq) in double
-__global__ void __launch_bounds__(256) wave_stats_kernel(const float* __restrict__ wav, int64_t N, int64_t stride,
+template <typename S>
+__global__ void __launch_bounds__(256) wave_stats_kernel(const S* __restrict__ wav, int64_t N, int64_t stride,
                                                          double* __restrict__ stats) {
     const int b = blockIdx.y;
-    const float* row = wav + (int64_t)b * stride;
+    const S* row = wav + (int64_t)b * stride;
     const int64_t chunk = 256 * 32;
     int64_t begin = (int64_t)blockIdx.x * chunk, end = min(begin + chunk, N);
     float s = 0.f, q = 0.f;
     for (int64_t i = begin + threadIdx.x; i < end; i += 256) {
-        float v = __ldg(row + i);
+        float v = sample_f32(__ldg(row + i));
         s += v;
         q = fmaf(v, v, q);
     }
@@ -112,7 +118,7 @@ int wave_instnorm_launch(const float* wav, int B, int64_t N, int64_t stride, con
                          double* stats, float* out, cudaStream_t s) {
     { int rc = zero_f64_launch(stats, (int64_t)2 * B, s); if (rc) return rc; }
     dim3 g1((unsigned)((N + 8191) / 8192), B);
-    wave_stats_kernel<<<g1, 256, 0, s>>>(wav, N, stride, stats);
+    wave_stats_kernel<float><<<g1, 256, 0, s>>>(wav, N, stride, stats);
     B200VAD_LAUNCH_CHECK();
     dim3 g2((unsigned)((N + 4095) / 4096), B);
     wave_norm_kernel<<<g2, 256, 0, s>>>(wav, N, stride, stats, gamma, beta, out);
@@ -125,7 +131,22 @@ int wave_instnorm_launch(const float* wav, int B, int64_t N, int64_t stride, con
 // stride; but rows t = 4 m + r of one residue class r start at 40 m + 10 r = (40 m + 8 floor(10 r / 8)) + (10 r mod 8),
 // i.e. at a 16-byte aligned offset of the copy shifted by 10 r mod 8 in {0, 2, 4, 6}, 80 bytes apart: four
 // overlapping-row tensor maps, one per residue class, feed the tcgen05 GEMM without an im2col pass.
-__global__ void __launch_bounds__(256) wave_norm_planes_kernel(const float* __restrict__ wav, int64_t N, int64_t stride, int64_t Np,
+// 8 samples row[i .. i + 7] as floats with 16-byte loads (vec_ok: 16-byte aligned rows)
+__device__ __forceinline__ void load8_f32(const float* row, float (&v)[8]) {
+    const float4 a0 = __ldg(reinterpret_cast<const float4*>(row)), a1 = __ldg(reinterpret_cast<const float4*>(row + 4));
+    v[0] = a0.x; v[1] = a0.y; v[2] = a0.z; v[3] = a0.w; v[4] = a1.x; v[5] = a1.y; v[6] = a1.z; v[7] = a1.w;
+}
+__device__ __forceinline__ void load8_f32(const int16_t* row, float (&v)[8]) {
+    const uint4 a = __ldg(reinterpret_cast<const uint4*>(row));
+    const uint32_t w[4] = {a.x, a.y, a.z, a.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        v[2 * j] = sample_f32((int16_t)(w[j] & 0xffffu));
+        v[2 * j + 1] = sample_f32((int16_t)(w[j] >> 16));
+    }
+}
+template <typename S>
+__global__ void __launch_bounds__(256) wave_norm_planes_kernel(const S* __restrict__ wav, int64_t N, int64_t stride, int64_t Np,
                                                                int B, const double* __restrict__ stats, const float* __restrict__ gamma,
                                                                const float* __restrict__ beta, __half* __restrict__ hi,
                                                                __half* __restrict__ lo, float s1) {
@@ -134,18 +155,17 @@ __global__ void __launch_bounds__(256) wave_norm_planes_kernel(const float* __re
     double var = stats[2 * b + 1] / (double)N - mean * mean;
     float rstd = (float)(1.0 / sqrt(fmax(var, 0.0) + 1e-5));
     float m = (float)mean, g = gamma[0], be = beta[0];
-    const float* row = wav + (int64_t)b * stride;
+    const S* row = wav + (int64_t)b * stride;
     // 8 consecutive samples per thread (Np and the copies' bases are multiples of 8 elements): copy e receives them at
     // element i - 2 e, i.e. at a 16 / 4 / 8 / 4-byte aligned address for e = 0 / 1 / 2 / 3
-    const bool vec_ok = (stride % 4 == 0) && ((reinterpret_cast<uintptr_t>(wav) & 15) == 0);
+    const bool vec_ok = ((stride * (int64_t)sizeof(S)) % 16 == 0) && ((reinterpret_cast<uintptr_t>(wav) & 15) == 0);
     for (int64_t i = ((int64_t)blockIdx.x * 256 + threadIdx.x) * 8; i < Np + 8; i += (int64_t)gridDim.x * 256 * 8) {
         float v[8];
         if (vec_ok && i + 8 <= N) {
-            const float4 a0 = __ldg(reinterpret_cast<const float4*>(row + i)), a1 = __ldg(reinterpret_cast<const float4*>(row + i + 4));
-            v[0] = a0.x; v[1] = a0.y; v[2] = a0.z; v[3] = a0.w; v[4] = a1.x; v[5] = a1.y; v[6] = a1.z; v[7] = a1.w;
+            load8_f32(row + i, v);
         } else {
 #pragma unroll
-            for (int j = 0; j < 8; ++j) v[j] = (i + j < N) ? row[i + j] : 0.f;
+            for (int j = 0; j < 8; ++j) v[j] = (i + j < N) ? sample_f32(row[i + j]) : 0.f;
         }
         __align__(16) __half h[8], l[8];
 #pragma unroll
@@ -182,16 +202,23 @@ __global__ void __launch_bounds__(256) wave_norm_planes_kernel(const float* __re
         }
     }
 }
-int wave_norm_planes_launch(const float* wav, int B, int64_t N, int64_t stride, int64_t Np, const float* gamma, const float* beta,
-                            double* stats, __half* hi, __half* lo, cudaStream_t s, int scaled_planes) {
+template <typename S>
+static int wave_norm_planes_run(const S* wav, int B, int64_t N, int64_t stride, int64_t Np, const float* gamma, const float* beta,
+                                double* stats, __half* hi, __half* lo, cudaStream_t s, int scaled_planes) {
     { int rc = zero_f64_launch(stats, (int64_t)2 * B, s); if (rc) return rc; }
     dim3 g1((unsigned)((N + 8191) / 8192), B);
-    wave_stats_kernel<<<g1, 256, 0, s>>>(wav, N, stride, stats);
+    wave_stats_kernel<S><<<g1, 256, 0, s>>>(wav, N, stride, stats);
     B200VAD_LAUNCH_CHECK();
     dim3 g2((unsigned)((Np + 8 + 2047) / 2048), B);
-    wave_norm_planes_kernel<<<g2, 256, 0, s>>>(wav, N, stride, Np, B, stats, gamma, beta, hi, lo, scaled_planes ? 1.f - kPlaneScale : 1.f);
+    wave_norm_planes_kernel<S><<<g2, 256, 0, s>>>(wav, N, stride, Np, B, stats, gamma, beta, hi, lo, scaled_planes ? 1.f - kPlaneScale : 1.f);
     B200VAD_LAUNCH_CHECK();
     return B200VAD_OK;
+}
+int wave_norm_planes_launch(const void* wav, int wav_i16, int B, int64_t N, int64_t stride, int64_t Np, const float* gamma,
+                            const float* beta, double* stats, __half* hi, __half* lo, cudaStream_t s, int scaled_planes) {
+    if (wav_i16)
+        return wave_norm_planes_run(reinterpret_cast<const int16_t*>(wav), B, N, stride, Np, gamma, beta, stats, hi, lo, s, scaled_planes);
+    return wave_norm_planes_run(reinterpret_cast<const float*>(wav), B, N, stride, Np, gamma, beta, stats, hi, lo, s, scaled_planes);
 }
 
 // GEMM weights for the tcgen05 path, zero padded to 128 output rows: (Cout, K) -> (128, ld)
