@@ -36,6 +36,7 @@ extern "C" {
 #define B200VAD_ABI_VERSION 1
 #define B200VAD_HIDDEN 128      /* LSTM hidden size (PyanNet2.py:60-66 LSTM_DEFAULTS) */
 #define B200VAD_NUM_MEL 80      /* FbankConfig.num_filters */
+#define B200VAD_MAX_INPUT_DIM 768   /* widest LSTM input D (768-dim SSL features): b200vad_model_workspace_bytes sizes for it */
 
 B200VAD_API int b200vad_abi_version(void);
 B200VAD_API const char* b200vad_last_error(void);
@@ -56,7 +57,9 @@ B200VAD_API int b200vad_set_projection_terms(int terms);
 /* Kernel of the input projections with K <= 256: 2 (default) = CTA pairs (tcgen05.mma.cta_group::2: two feature blocks
  * share an activation tile, each CTA loading half of it), both weight planes in tensor memory, 2 or 3 products per
  * k-step (see above); 1 = the same on single CTAs with an 8-warp epilogue; 0 = the general K-split kernel (always 3
- * products; validation, and the path of inputs wider than 256). */
+ * products; validation, and the path of inputs wider than 256).  In LSTM modes 1 and 2 (b200vad_set_lstm_fused) the fused
+ * layer kernels compute every projection with K <= 256 themselves, so there this choice reaches no kernel: layers >= 1
+ * use 2 or 3 products as b200vad_set_projection_terms says, whichever kernel is set. */
 B200VAD_API int b200vad_set_projection_kernel(int which);
 /* 1 (default): the head (two Linear + LeakyReLU, classifier, sigmoid -- PyanNet2.py:183-187) runs as one kernel whose hidden
  * activations stay in shared memory; 0: two GEMM launches with the hidden activations as fp16 planes in HBM (validation;
@@ -121,7 +124,8 @@ B200VAD_API int b200vad_fbank_i16(const int16_t* wav, const int32_t* lens, int B
 
 /* ---- a2: PyanNet2.forward (src/models/segmentation/PyanNet2.py:154-187): nn.LSTM stack
  * (4 x BiLSTM(128) by default) + Linear/LeakyReLU x2 + Linear(1) + Sigmoid.
- * Weights are packed once into an opaque device blob in kernel layout. */
+ * Weights are packed once into an opaque device blob in kernel layout.  Input widths 1 <= D <= B200VAD_MAX_INPUT_DIM:
+ * packed_bytes returns 0 for any other D, and the pack and forward calls refuse it with B200VAD_EINVAL. */
 B200VAD_API size_t b200vad_model_packed_bytes(int D, int num_layers);
 /* one call per (layer, direction); w_ih (512, D_l), w_hh (512, 128), b_ih/b_hh (512): f32 device */
 B200VAD_API int b200vad_model_pack_lstm(void* packed, int D, int num_layers, int layer, int direction, const float* w_ih,

@@ -2,9 +2,12 @@
 their acc_ready poller and the exchange senders meet on named barriers once per (step, part) with q < nparts and, for the
 exchange, s + 1 < T, so every parts count per work item (1..8), items of unequal parts counts, a partial last part and the
 shortest sequences (T = 1: no exchange at all) must give the same layer outputs as the CTA-pair kernel (mode 2), bit for bit.
-Run on the B200 box: pytest -m gpu."""
+D = 100 and 192 run the generic instantiation of both kernels (run-time k-step count) on 6- and 4-stage x rings, D = 80 and
+256 the nk = 5 and nk = 16 specialisations on 12- and 3-stage rings.  Run on the B200 box: pytest -m gpu."""
 import pytest
 import torch
+
+import util
 
 pytestmark = pytest.mark.gpu
 
@@ -27,7 +30,7 @@ def _batches(clusters):
     return sorted(set(bs))
 
 
-@pytest.mark.parametrize("D", [80, 256])
+@pytest.mark.parametrize("D", [80, 100, 192, 256])
 @pytest.mark.parametrize("T", [1, 2, 3, 50])
 def test_fused_layer_equals_pair_kernel_at_every_parts_count(dev, D, T):
     import b200vad
@@ -38,6 +41,11 @@ def test_fused_layer_equals_pair_kernel_at_every_parts_count(dev, D, T):
     m = oracle.VadModel("PyanNet2", {"encoding_dim": D, "lstm": {"hidden_size": 128, "num_layers": L, "bidirectional": True,
                                                                  "monolithic": True, "dropout": 0.0}}).eval()
     blob = b200vad.pack_model(m.model.state_dict(), dev, D, L)
+    # at one T, narrower inputs also run zero-padded to 256 (random weight columns): the nk = 16 kernel must give the same bits
+    padded = T == 3 and D < 256
+    if padded:
+        sdp, _ = util.pad_input_width(m.model.state_dict(), torch.zeros(1, 1, D), 256, seed=D)
+        blob_p = b200vad.pack_model(sdp, dev, 256, L)
     g = torch.Generator(device=dev).manual_seed(1000 * D + T)
     try:
         for B in _batches(lib.b200vad_lstm_fused_clusters()):
@@ -48,7 +56,11 @@ def test_fused_layer_equals_pair_kernel_at_every_parts_count(dev, D, T):
             for mode in (1, 2):
                 lib.b200vad_set_lstm_fused(mode)
                 out[mode] = torch.ops.b200vad.lstm_head(x, blob, L)
+            if padded:
+                out["pad"] = torch.ops.b200vad.lstm_head(torch.nn.functional.pad(x, (0, 256 - D)), blob_p, L)
             torch.cuda.synchronize()
             assert torch.equal(out[1], out[2]), f"B={B} T={T} D={D}: mode 1 != mode 2"
+            if padded:
+                assert torch.equal(out[2], out["pad"]), f"B={B} T={T} D={D}: != the same input zero-padded to 256"
     finally:
         lib.b200vad_set_lstm_fused(1)

@@ -214,7 +214,10 @@ def test_reference_golden_trained_spreads(dev, golden_dir):
         assert near[b, max(0, t - 24): t + 25].any(), (b, t)
 
 
-@pytest.mark.parametrize("shape", [(16, 8, 80, 1), (3, 100, 80, 2), (130, 40, 60, 4), (300, 30, 256, 2), (1000, 64, 80, 4)])
+@pytest.mark.parametrize("shape", [(16, 8, 80, 1), (3, 100, 80, 2), (130, 40, 60, 4), (300, 30, 256, 2), (1000, 64, 80, 4),
+                                   # depths: L = 1 hands layer 0's planes straight to the head (at D = 300 from the K-split
+                                   # layer 0 with hi / lo output planes); odd depths alternate the layer buffers unevenly
+                                   (37, 33, 80, 3), (37, 33, 80, 5), (37, 33, 80, 6), (37, 33, 300, 1), (37, 33, 300, 3)])
 def test_lstm_layer_modes_agree(dev, shape):
     """The three LSTM layer paths (b200vad_set_lstm_fused): 2 = fused layer on CTA pairs (cta_group::2 MMAs, csrc/lstm_pair.cu) must be
     BIT-identical to 1 = fused layer (csrc/lstm_fused.cu) -- same products in the same order, only the operand tiles are split

@@ -46,3 +46,16 @@ def make_oracle(model_name="PyanNet2", model_dict=None, seed=42, spread=False, f
 def synth_wave(B, N, seed=0):
     import b200vad
     return b200vad.synth.meeting_batch(B, N, seed=seed)
+
+
+def pad_input_width(sd, x, Dp, seed=0):
+    """The same model and input at layer-0 width Dp >= D: x gets Dp - D zero channels and weight_ih_l0[_reverse] gets
+    Dp - D extra columns of RANDOM values.  Every extra product is exactly zero, so a kernel that adds them in the same order
+    as the products of the first D channels must return the unpadded result bit for bit."""
+    g = torch.Generator().manual_seed(seed)
+    D = x.shape[-1]
+    out = dict(sd)
+    for k in ("lstm.weight_ih_l0", "lstm.weight_ih_l0_reverse"):
+        w = sd[k]
+        out[k] = torch.cat([w, torch.randn(w.shape[0], Dp - D, generator=g).to(w)], dim=1)
+    return out, torch.nn.functional.pad(x, (0, Dp - D))

@@ -19,6 +19,8 @@ _lib = None
 
 c_void_p, c_int, c_int64, c_size_t, c_float, c_double = C.c_void_p, C.c_int, C.c_int64, C.c_size_t, C.c_float, C.c_double
 
+MAX_INPUT_DIM = 768     # B200VAD_MAX_INPUT_DIM: the widest LSTM input the model entry points accept
+
 # name -> (restype, argtypes); mirrors include/b200vad.h one to one
 PROTOTYPES = {
     "b200vad_abi_version": (c_int, []),

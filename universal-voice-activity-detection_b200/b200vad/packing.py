@@ -66,16 +66,19 @@ def pack_model(sd: dict, device, encoding_dim: int, num_layers: int = 4, monolit
     return blob
 
 
+# SincNet parameters in the argument order of b200vad_sincnet_pack
+SINCNET_KEYS = ("wav_norm1d.weight", "wav_norm1d.bias", "conv1d.0.filterbank.low_hz_", "conv1d.0.filterbank.band_hz_",
+                "conv1d.0.filterbank.window_", "conv1d.0.filterbank.n_", "conv1d.1.weight", "conv1d.1.bias",
+                "conv1d.2.weight", "conv1d.2.bias", "norm1d.0.weight", "norm1d.0.bias", "norm1d.1.weight", "norm1d.1.bias",
+                "norm1d.2.weight", "norm1d.2.bias")
+
+
 def pack_sincnet(sd: dict, device, prefix: str = "sincnet.") -> torch.Tensor:
     device = torch.device(device)
     if device.type != "cuda":
         raise _lib.B200VadError("packing needs a CUDA device (no CPU path)")
     L = _lib.lib()
-    keys = ["wav_norm1d.weight", "wav_norm1d.bias", "conv1d.0.filterbank.low_hz_", "conv1d.0.filterbank.band_hz_",
-            "conv1d.0.filterbank.window_", "conv1d.0.filterbank.n_", "conv1d.1.weight", "conv1d.1.bias",
-            "conv1d.2.weight", "conv1d.2.bias", "norm1d.0.weight", "norm1d.0.bias", "norm1d.1.weight", "norm1d.1.bias",
-            "norm1d.2.weight", "norm1d.2.bias"]
-    ts = [_f32(sd[prefix + k], device) for k in keys]
+    ts = [_f32(sd[prefix + k], device) for k in SINCNET_KEYS]
     if tuple(ts[6].shape) != (60, 80, 5) or tuple(ts[8].shape) != (60, 60, 5) or ts[2].numel() != 40 or ts[4].numel() != 125:
         raise _lib.B200VadError("unsupported SincNet shape (expected the reference's 80x251 sinc + 60x80x5 + 60x60x5)")
     blob = torch.zeros(L.b200vad_sincnet_packed_bytes(), dtype=torch.uint8, device=device)

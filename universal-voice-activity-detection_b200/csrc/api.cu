@@ -162,6 +162,7 @@ static int model_forward(const void* packed, int D, int L, const float* x, const
                          int64_t T, float* prob, void* ws, size_t ws_bytes, cudaStream_t st) {
     B200VAD_CHECK_ARG(packed && (x || (xp_hi && xp_lo && g_impl == 2)) && prob && ws, "null pointer");
     B200VAD_CHECK_ARG(D > 0 && L > 0 && B >= 0 && T >= 0, "bad shape");
+    B200VAD_CHECK_ARG(D <= B200VAD_MAX_INPUT_DIM, "input width D > 768 (the widest supported input, B200VAD_MAX_INPUT_DIM)");
     B200VAD_CHECK_ARG((reinterpret_cast<uintptr_t>(ws) & 255) == 0, "workspace must be 256-byte aligned");
     if (B == 0 || T == 0) return B200VAD_OK;
     B200VAD_CHECK_ARG(T < (1 << 24), "T too large");
@@ -265,8 +266,9 @@ static int model_forward(const void* packed, int D, int L, const float* x, const
             __half* yh = reinterpret_cast<__half*>(outbuf);
             __half* yl = yh + rows * 2 * kHidden;
             // the output planes of a layer that feeds a 2-MMA projection use that kernel's scaled split; the last layer
-            // (into the head's 3-term product) keeps hi / lo
-            const int scaled = (g_proj_terms == 2 && g_proj_kernel != 0 && l + 1 < L) ? 1 : 0;
+            // (into the head's 3-term product) keeps hi / lo.  In modes 1 and 2 the next layer is a fused kernel, which
+            // takes 2 products whatever g_proj_kernel says; in mode 0 kernel 0 always takes 3.
+            const int scaled = (g_proj_terms == 2 && l + 1 < L && (lstm_mode() != 0 || g_proj_kernel != 0)) ? 1 : 0;
             if ((rc = lstm_tc_launch(xg, reinterpret_cast<const __half*>(pk + lo.whh), yh, yl, bc, (int)T, scaled, st))) return rc;
             a_hi = yh; a_lo = yl; lda = 2 * kHidden;
             outbuf = (outbuf == buf0) ? buf1 : buf0;
@@ -511,12 +513,13 @@ int b200vad_fbank_i16(const int16_t* wav, const int32_t* lens, int B, int64_t N,
 }
 
 size_t b200vad_model_packed_bytes(int D, int L) {
-    if (D <= 0 || L <= 0) return 0;
+    if (D <= 0 || D > B200VAD_MAX_INPUT_DIM || L <= 0) return 0;
     return model_layout(D, L).total;
 }
 
 int b200vad_model_pack_lstm(void* packed, int D, int L, int layer, int dir, const float* w_ih, const float* w_hh,
                             const float* b_ih, const float* b_hh, void* stream) {
+    B200VAD_CHECK_ARG(D <= B200VAD_MAX_INPUT_DIM, "input width D > 768 (the widest supported input, B200VAD_MAX_INPUT_DIM)");
     B200VAD_CHECK_ARG(packed && w_ih && w_hh && b_ih && b_hh, "null pointer");
     B200VAD_CHECK_ARG(D > 0 && L > 0 && layer >= 0 && layer < L && (dir == 0 || dir == 1), "bad index");
     ModelLayout m = model_layout(D, L);
@@ -534,6 +537,7 @@ int b200vad_model_pack_lstm(void* packed, int D, int L, int layer, int dir, cons
 
 int b200vad_model_pack_head(void* packed, int D, int L, const float* w1, const float* b1, const float* w2, const float* b2,
                             const float* wc, const float* bc, void* stream) {
+    B200VAD_CHECK_ARG(D <= B200VAD_MAX_INPUT_DIM, "input width D > 768 (the widest supported input, B200VAD_MAX_INPUT_DIM)");
     B200VAD_CHECK_ARG(packed && w1 && b1 && w2 && b2 && wc && bc, "null pointer");
     B200VAD_CHECK_ARG(D > 0 && L > 0, "bad shape");
     ModelLayout m = model_layout(D, L);
@@ -554,7 +558,7 @@ int b200vad_model_pack_head(void* packed, int D, int L, const float* w1, const f
 
 size_t b200vad_model_workspace_bytes(int B, int64_t T) {
     if (B <= 0 || T <= 0) return 0;
-    return (size_t)ceil64(B) * model_per_row(768, T) + 4096;   /* whole 64-sequence blocks, widest supported input (D <= 768) */
+    return (size_t)ceil64(B) * model_per_row(B200VAD_MAX_INPUT_DIM, T) + 4096;   /* whole 64-sequence blocks, widest supported input */
 }
 
 int b200vad_model_forward_f32(const void* packed, int D, int L, const float* x, int B, int64_t T, float* prob, void* ws,

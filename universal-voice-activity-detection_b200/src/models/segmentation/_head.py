@@ -50,6 +50,9 @@ class HeadMixin(PackedOwner):
         if l["hidden_size"] != 128 or not l["bidirectional"] or n["hidden_size"] != 128 or n["num_layers"] != 2:
             raise NotImplementedError("the sm_100a kernels are built for the reference defaults: BiLSTM(128) x L, "
                                       "Linear(128) x 2 (PyanNet2.py:60-67)")
+        if not 1 <= self.encoding_dim <= b200vad._lib.MAX_INPUT_DIM:
+            raise NotImplementedError(f"encoding_dim {self.encoding_dim}: the sm_100a kernels take LSTM inputs of 1 to "
+                                      f"{b200vad._lib.MAX_INPUT_DIM} channels")
         if torch.is_grad_enabled() and self.training and any(p.requires_grad for p in self.parameters()):
             raise NotImplementedError("b200vad implements inference only; call .eval() / torch.no_grad()")
         if self.training and l["num_layers"] > 1 and l.get("dropout", 0.0) > 0:
