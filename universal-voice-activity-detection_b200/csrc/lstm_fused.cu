@@ -22,11 +22,11 @@
 //     commit drains it: a single thread left the pipe idle during every barrier wait, and a thread spends ~2/3 of a part
 //     slot in waits and commits;
 //   * 16 pointwise warps: warp (pg, g) serves parts pg and pg + 4 alternately (while one part's h travels, the other is
-//     computed) and owns TMEM lane quarter g.  Lane 32 g + l of the accumulator is gate (l & 3) of unit 8 g + (l >> 2):
-//     the four gates of a cell sit in four adjacent lanes of ONE warp, so the (gate x sequence) transposition runs through a
-//     warp-private 2 KB scratch with __syncwarp only.  One warp of the group polls acc_ready and releases the other three
-//     through a named barrier, and the staged h slice goes to the sender through another (F_BAR_ACC, F_BAR_SLICE): blocked
-//     warps issue nothing, where polling ones took issue slots from the pointwise pass;
+//     computed) and owns TMEM lane quarter g.  Lane 32 g + l of the accumulator is gate l >> 3 of unit 8 g + (l & 7):
+//     two 16x256b TMEM loads then give each lane all four gates of one unit for four sequences, with no (gate x sequence)
+//     transposition through shared memory.  One warp of the group polls acc_ready and releases the other three through a
+//     named barrier, and the staged h slice goes to the sender through another (F_BAR_ACC, F_BAR_SLICE): blocked warps
+//     issue nothing, where polling ones took issue slots from the pointwise pass;
 //   * 4 exchange-sender warps (h exchange over distributed shared memory): the pointwise warps write h_s (fp16 planes,
 //     operand layout) into the CTA's own 2 KB staging slice of the part; a sender warp copies it with 16-byte st.async stores
 //     into k-block `rank` of the part's operand tile in all four CTAs (the destination mbarriers count the bytes).  The MMA K
@@ -39,7 +39,10 @@
 // the SM-to-SM port (~17 B/clk: 360-720 cycles) and ~320 issue slots per SM sub-partition.  n = 8 is all the accumulator columns
 // TMEM has left, so half of the step is unhidden latency.  Replacing 12 of the 16 acc_ready pollers and the 4 slice pollers by named
 // barriers (~160 -> ~86 polls per step and CTA) cut the one-part step to 1.18 us and the layer by 3.4 %, but not the per-part slope
-// (profiles/r03_lstm_fused_handoffs.md): the issue slots taken by polls are not what sets the per-part cost.  Exchange mechanisms tried: cp.async.bulk by a sender thread (~3000 cycles per
+// (profiles/r03_lstm_fused_handoffs.md): the issue slots taken by polls are not what sets the per-part cost.  The pointwise pass
+// is a dependent chain whose latency the step follows: taking the shared-memory transposition out of it (16x256b TMEM loads)
+// cut the layer by 13 % (profiles/r04_lstm_fused_tmem_layout.md), while making the pass 32 columns wide on pairs of parts made it
+// slower (profiles/r04_lstm_fused_pairs.md).  Exchange mechanisms tried: cp.async.bulk by a sender thread (~3000 cycles per
 // copy through the TMA unit), st.async from the pointwise warps (they stall on the port), and an exchange through the output
 // planes in L2 (TMA store + multicast TMA load: two ~1-2 us TMA round trips on the per-step chain; that variant showed
 // intermittent launch failures -- in hindsight probably the x_full race described at bar_x_full, which any delay of the x tiles
@@ -80,12 +83,11 @@ constexpr int F_BOX = FPN * 128;            // one h k-block of a part: 16 rows 
 constexpr int F_XBOX = 2 * F_BOX;           // one x TMA box: the 32 rows of a PAIR of parts (the input products run on pairs, MMA N = 32)
 constexpr int F_HTILE = FC * F_BOX;         // h operand tile of a part: 4 k-blocks (one per source CTA) = 8 KB
 constexpr int F_STAGING = 2 * FMAXP * F_BOX; // own h slices [step parity][part][16 rows][128 B] (source of the exchange copies): 32 KB
-constexpr int F_SCRATCH = 32 * 16 * 4;      // per pointwise warp: gate transposition scratch [lane 32][16 columns] fp32 = 2 KB (then the y chunk staging)
 constexpr int F_ACC_COL = 0;                // TMEM columns [0, 128): accumulators, part p at 16 p
 constexpr int F_WHH_COL = FMAXP * FPN;      // [128, 256): W_hh, k-step j at 128 + 8 j
 constexpr int F_WIH_COL = F_WHH_COL + 128;  // [256, 256 + 16 nk): W_ih plane a then plane b
 constexpr int F_MAX_STAGES = 16;
-constexpr int F_SMEM_FIXED = FMAXP * F_HTILE + F_STAGING + F_PW_WARPS * F_SCRATCH;   // 128 KB
+constexpr int F_SMEM_FIXED = FMAXP * F_HTILE + F_STAGING;   // 96 KB
 constexpr int F_SMEM_MAX = 232448;          // 227 KB per CTA
 
 struct FusedParams {
@@ -199,8 +201,7 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
     unsigned char* const smem_gen = smem_dyn + (smem_base - smem_u32(smem_dyn));
     const uint32_t h_off = 0;                                  // [part 8][k-block 4][16 rows][128 B]
     const uint32_t g_off = FMAXP * F_HTILE;                    // staging [step parity 2][part 8][16 rows][128 B]
-    const uint32_t c_off = g_off + F_STAGING;                  // scratch [pointwise warp 16][2 KB]
-    const uint32_t x_off = c_off + F_PW_WARPS * F_SCRATCH;     // [stage][plane 2][k-block][16 rows][128 B]
+    const uint32_t x_off = g_off + F_STAGING;                  // [stage][plane 2][k-block][16 rows][128 B]
     const int nk = NK > 0 ? NK : p.nk;
     const int terms = NK > 0 ? TERMS : p.terms;
     const uint32_t stage_bytes = 2u * p.kblocks * F_XBOX;     // one stage = the x tile of a pair of parts
@@ -275,8 +276,9 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
         if (warp < F_PW_WARPS && loaded_dir != dir) {
             const int wg = warp >> 2, g = warp & 3;
             const uint32_t lane_addr = tmem_base + ((uint32_t)(g * 32) << 16);
-            // TMEM lane 32 g + l holds gate (l & 3) of unit 8 g + (l >> 2) of this CTA
-            const int grow = dir * kGates + (lane & 3) * kHidden + (int)rank * FU + 8 * g + (lane >> 2);   // packed weight row of this TMEM lane
+            // TMEM lane 32 g + l holds gate l >> 3 of unit 8 g + (l & 7) of this CTA: the row pattern of a 16x256b TMEM load, which
+            // gives lane l rows l >> 2 and (l >> 2) + 8 of a 16-lane half, so that two loads bring it all four gates of unit l >> 2
+            const int grow = dir * kGates + (lane >> 3) * kHidden + (int)rank * FU + 8 * g + (lane & 7);   // packed weight row of this TMEM lane
             // W_hh: k-step j holds plane (j >> 1) & 1 of units 32 (j >> 2) + 16 (j & 1) .. + 15  (K block j >> 2 = source CTA)
             for (int j = wg; j < 16; j += 4) {
                 const int u0 = 32 * (j >> 2) + 16 * (j & 1), plane = (j >> 1) & 1;
@@ -555,18 +557,15 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
             }
         } else if ((warp >> 2) < nparts) {
             // ===================== pointwise warps: warp (pg, g) = parts pg and pg + 4, units 8 g .. 8 g + 7 of this CTA =====================
-            // lane l reads the accumulator row of gate l & 3 of unit 8 g + (l >> 2) for the part's 16 sequences, turns it into
-            // exponentials, and the four lanes of a unit transpose (gate x sequence) through the warp-private scratch, after
-            // which lane l owns all four gates of 4 cells: unit 8 g + (l >> 2), sequences 4 (l & 3) + i.
+            // Two 16x256b TMEM loads (lanes 32 g .. + 15 and 32 g + 16 .. + 31) hand lane l all four gates of unit 8 g + (l >> 2)
+            // for the 4 sequences seq(i) = 2 (l & 3) + (i & 1) + 8 (i >> 1): the gate rows are laid out for exactly that (see the
+            // weight loader), so no (gate x sequence) transposition through shared memory is needed.
             const int pg = warp >> 2, g = warp & 3;
             const int uu = lane >> 2, jj = lane & 3;
             const uint32_t lane_addr = tmem_base + ((uint32_t)(g * 32) << 16) + F_ACC_COL;
-            const float bias = __ldg(p.bias + dir * kGates + jj * kHidden + (int)rank * FU + 8 * g + uu);
-            unsigned char* const scr = smem_gen + c_off + warp * F_SCRATCH;
-            // scratch address of (row, 16-byte chunk c): conflict-free for the row-wise stores and the gate-wise loads
-            auto scr_at = [&](int row, int c) -> unsigned char* {
-                return scr + (((row * 64) + ((c ^ ((row >> 1) & 3)) << 4)) ^ (((row >> 2) & 1) << 6));
-            };
+            float bias[4];                                                     // [gate] of unit 8 g + uu
+#pragma unroll
+            for (int k = 0; k < 4; ++k) bias[k] = __ldg(p.bias + dir * kGates + k * kHidden + (int)rank * FU + 8 * g + uu);
             const float s1 = 1.f - kPlaneScale;
             const float L2E2 = 2.f * kLog2e;
             float cst[2][4];
@@ -592,27 +591,21 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
                     tc_fence_after();                                              // (commit -> mbarrier -> poller -> bar.sync -> tcgen05.ld)
                     const bool tr_on = tr_item && warp == 0 && pi == 0 && s >= F_TRACE_S0 && s < F_TRACE_S0 + F_TRACE_STEPS;
                     if (tr_on) trace[(s - F_TRACE_S0) * 16 + 2] = clock64();
-                    float z[16];
-                    tmem_ld16(lane_addr + q * FPN, z);
+                    float z[2][8];                                                 // [gates 2 h, 2 h + 1]: see tmem_ld_16x256b_x2
+                    tmem_ld_16x256b_x2(lane_addr + q * FPN, z[0]);
+                    tmem_ld_16x256b_x2(lane_addr + (16u << 16) + q * FPN, z[1]);
                     tmem_ld_wait();
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(bar_acc_free(q));                   // the next step's input product may overwrite the accumulator
                     if (tr_on) trace[(s - F_TRACE_S0) * 16 + 3] = clock64();
+                    float ev[4][4];                                                // [gate][cell i]: sequence seq(i)
 #pragma unroll
-                    for (int j = 0; j < 16; ++j) z[j] = fast_ex2(fminf(z[j] + bias, 29.f));
+                    for (int k = 0; k < 4; ++k)
+#pragma unroll
+                        for (int i = 0; i < 4; ++i)
+                            ev[k][i] = fast_ex2(fminf(z[k >> 1][4 * (i >> 1) + 2 * (k & 1) + (i & 1)] + bias[k], 29.f));
                     if (tr_on) trace[(s - F_TRACE_S0) * 16 + 4] = clock64();
-                    float ev[4][4];                                                // [gate][cell i]: sequence 4 jj + i
-#pragma unroll
-                    for (int c = 0; c < 4; ++c)
-                        *reinterpret_cast<float4*>(scr_at(lane, c)) = make_float4(z[4 * c], z[4 * c + 1], z[4 * c + 2], z[4 * c + 3]);
-                    __syncwarp();
-#pragma unroll
-                    for (int b = 0; b < 4; ++b) {
-                        const float4 v = *reinterpret_cast<const float4*>(scr_at((lane & ~3) + b, jj));
-                        ev[b][0] = v.x; ev[b][1] = v.y; ev[b][2] = v.z; ev[b][3] = v.w;
-                    }
-                    __syncwarp();
                     if (tr_on) trace[(s - F_TRACE_S0) * 16 + 5] = clock64();
                     float hv[4];
                     const f32x2 one = pack2(1.f, 1.f), mone = pack2(-1.f, -1.f), k2 = pack2(L2E2, L2E2);
@@ -638,7 +631,7 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
                     unsigned char* const stg = smem_gen + g_off + ((s & 1) * FMAXP + q) * F_BOX;
 #pragma unroll
                     for (int c = 0; c < 4; ++c) {
-                        const int row = 4 * jj + c;
+                        const int row = 2 * jj + (c & 1) + 8 * (c >> 1);
                         __half a1, a2;
                         split_scaled_f16(hv[c], s1, a1, a2);
                         unsigned char* const rp = stg + row * 128 + uu * 2;

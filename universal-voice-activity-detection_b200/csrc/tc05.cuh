@@ -322,6 +322,15 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
                  : "r"(taddr)
                  : "memory");
 }
+// 16 lanes x 16 columns: lane l of the warp gets rows r = l >> 2 and r + 8 (of the 16 lanes at taddr), columns c = 2 (l & 3) + {0, 1}
+// and c + 8: v = {(r, c), (r, c + 1), (r + 8, c), (r + 8, c + 1), (r, c + 8), (r, c + 9), (r + 8, c + 8), (r + 8, c + 9)}
+__device__ __forceinline__ void tmem_ld_16x256b_x2(uint32_t taddr, float (&v)[8]) {
+    uint32_t* r = reinterpret_cast<uint32_t*>(v);
+    asm volatile("tcgen05.ld.sync.aligned.16x256b.x2.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+                 : "r"(taddr)
+                 : "memory");
+}
 __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&r)[8]) {
     asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
                  ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
