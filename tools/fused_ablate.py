@@ -92,7 +92,7 @@ def main():
         buf = (C.c_longlong * 128)()
         lib.b200vad_lstm_fused_read_debug(buf, -128)
         names = ["mma:h_ready", "mma:issued", "pw:acc_rdy", "pw:tmem_ld", "pw:ex2", "pw:xchg", "ld:y_done", "pub:slice", "pub:done",
-                 "x:start", "pw:math", "ld:issued", "pw:done", "x:xfull", "-", "x:commit"]
+                 "x:start", "pw:math", "ld:issued", "pw:done", "x:xfull", "pub:y_done", "x:commit"]
         print(f"--- timeline of one part, {label} (cycles after the MMA thread saw h_ready; last column = step period)")
         print("      " + " ".join(f"{n:>12s}" for n in names))
         prev = None

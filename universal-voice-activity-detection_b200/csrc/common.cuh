@@ -186,6 +186,14 @@ __device__ __forceinline__ void split_scaled_f16(float x, float s1, __half& a, _
     a = __float2half_rn(x * s1);
     b = __float2half_rn(x - __half2float(a));
 }
+// split_scaled_f16 of two values at once (x in the low halves): the same operations and roundings, packed conversions
+__device__ __forceinline__ void split_scaled_f16x2(float x, float y, float s1, uint32_t& a, uint32_t& b) {
+    const __half2 a2 = __floats2half2_rn(x * s1, y * s1);
+    const float2 af = __half22float2(a2);
+    const __half2 b2 = __floats2half2_rn(x - af.x, y - af.y);
+    a = *reinterpret_cast<const uint32_t*>(&a2);
+    b = *reinterpret_cast<const uint32_t*>(&b2);
+}
 // Order-independent accumulation of InstanceNorm partial sums with atomicAdd(double): every partial is rounded to a multiple of
 // 2^-BITS, so the additions are exact (no rounding, hence no dependence on the order in which CTAs arrive) as long as the running
 // sum stays below 2^(53 - BITS); beyond that it degrades to ordinary double rounding (still accurate, no longer order-independent).

@@ -27,13 +27,15 @@
 //     transposition through shared memory.  One warp of the group polls acc_ready and releases the other three through a
 //     named barrier, and the staged h slice goes to the sender through another (F_BAR_ACC, F_BAR_SLICE): blocked warps
 //     issue nothing, where polling ones took issue slots from the pointwise pass;
-//   * 4 exchange-sender warps (h exchange over distributed shared memory): the pointwise warps write h_s (fp16 planes,
-//     operand layout) into the CTA's own 2 KB staging slice of the part; a sender warp copies it with 16-byte st.async stores
-//     into k-block `rank` of the part's operand tile in all four CTAs (the destination mbarriers count the bytes).  The MMA K
+//   * 4 exchange-sender warps (h exchange over distributed shared memory): the pointwise warps write h_s (fp32) into the CTA's
+//     own 2 KB staging slice of the part and end their pass there; a sender warp reads the slice, splits it into the two fp16
+//     planes (operand layout) and stores them with 16-byte st.async stores into k-block `rank` of the part's operand tile in all
+//     four CTAs (the destination mbarriers count the bytes), then the same chunks into the layer output planes.  The MMA K
 //     index is free as long as A and B agree: K block r (64 slots = one 128-byte swizzled row) is [h1 of units 32r..32r+31 |
 //     h2 of the same units], exactly what CTA r produces, so a CTA's contribution is ONE contiguous box.
 //
-// What bounds it (profiles/r02_lstm_fused.md): a step of a cluster with n parts in flight takes ~1.6 us + 0.26 us (n - 1): a fixed
+// What bounds it (profiles/r02_lstm_fused.md): a step of a cluster with n parts in flight took ~1.6 us + 0.26 us (n - 1) in round 2
+// (now ~1.1 us + 0.28 us (n - 1), see kStepUs in the launcher): a fixed
 // chain latency (recurrent MMAs -> accumulator read -> cell arithmetic -> h exchange -> next MMAs, ~2 900 cycles) plus a per-part
 // cost of ~475 cycles: a part needs 384 tensor-pipe cycles (16 recurrent MMAs x 8 + 16 input MMAs x 16), 6 KB out + 6 KB in over
 // the SM-to-SM port (~17 B/clk: 360-720 cycles) and ~320 issue slots per SM sub-partition.  n = 8 is all the accumulator columns
@@ -42,7 +44,9 @@
 // (profiles/r03_lstm_fused_handoffs.md): the issue slots taken by polls are not what sets the per-part cost.  The pointwise pass
 // is a dependent chain whose latency the step follows: taking the shared-memory transposition out of it (16x256b TMEM loads)
 // cut the layer by 13 % (profiles/r04_lstm_fused_tmem_layout.md), while making the pass 32 columns wide on pairs of parts made it
-// slower (profiles/r04_lstm_fused_pairs.md).  Exchange mechanisms tried: cp.async.bulk by a sender thread (~3000 cycles per
+// slower (profiles/r04_lstm_fused_pairs.md).  Moving the plane split and the layer-output store from the pass to the sender
+// warps, which were idle most of the step, took ~95 of its ~225 instructions and cut the layer by another 9 %
+// (profiles/r05_lstm_fused_sender_split.md).  Exchange mechanisms tried: cp.async.bulk by a sender thread (~3000 cycles per
 // copy through the TMA unit), st.async from the pointwise warps (they stall on the port), and an exchange through the output
 // planes in L2 (TMA store + multicast TMA load: two ~1-2 us TMA round trips on the per-step chain; that variant showed
 // intermittent launch failures -- in hindsight probably the x_full race described at bar_x_full, which any delay of the x tiles
@@ -114,7 +118,11 @@ struct FusedParams {
 constexpr int F_DBG_TAGS = 8, F_DBG_FIELDS = 3, F_DBG_WARPS = 25, F_DBG_MAX_CTAS = 148;
 __device__ long long g_fused_dbg[F_DBG_MAX_CTAS * F_DBG_WARPS * F_DBG_TAGS * F_DBG_FIELDS];
 
-// timeline probe (flags & 64): clock64 stamps of one part (part 0 of CTA 0's first item) over F_TRACE_STEPS steps
+// timeline probe (flags & 64): clock64 stamps of one part (part 0 of CTA 0's first item) over F_TRACE_STEPS steps, 16 per step:
+// recurrent issuer 0 h_ready seen, 1 MMAs committed; pointwise warp 0: 2 acc_ready, 3 accumulator read, 4 / 5 exponentials,
+// 10 cell arithmetic done, 12 pass done (fp32 h staged and handed over at the slice barrier); sender: 7 slice received, 8 exchange
+// issued, 14 layer output stored; input issuer: 9 start, 13 x_full, 15 committed.  (Until the sender split the planes, 12 came
+// after the plane split and the layer-output store of the pointwise warp, 8 was the sender's end and 14 was unused.)
 constexpr int F_TRACE_S0 = 100, F_TRACE_STEPS = 8;
 __device__ long long g_fused_trace[F_TRACE_STEPS * 16 + 128];   // + per-part stamps of the two MMA threads over two steps (flag 128)
 
@@ -164,13 +172,14 @@ __device__ __forceinline__ void mbar_wait_tag(uint32_t bar, uint32_t parity, int
 //   * F_BAR_ACC + pg (1-4), 128 threads: the 4 pointwise warps of part group pg, once per (step, part q in {pg, pg + 4} with
 //     q < nparts), after the group's poller (warp 5 pg, lane quarter g == pg: one poller per SM sub-partition) has seen
 //     acc_ready(q).  The poller's mbarrier wait keeps the bounded wait and its time-out record.
-//   * F_BAR_SLICE + pg (5-8), 160 threads: the same 4 warps and sender warp pg, once per (step s with s + 1 < T, part q in
-//     {pg, pg + 4} with q < nparts), when the part's h_s slice is staged.  Replaces an mbarrier arrive + sender poll; holding
-//     the pointwise warps until the sender arrives costs the chain nothing, because what they wait for next, acc_ready of the
-//     group's other part, needs the sender's previous send (h of that part) to have landed anyway.
-// Both sides of a barrier run the same (s, q) sequence from the same conditions (q < nparts per item, s + 1 < T for the
-// exchange), and bar.sync blocks every participant until all have arrived: no participant can arrive at generation n + 1
-// before generation n completed, so generations cannot mix.  A participation mismatch would hang instead of trapping.
+//   * F_BAR_SLICE + pg (5-8), 160 threads: the same 4 warps and sender warp pg, once per (step s < T, part q in {pg, pg + 4}
+//     with q < nparts), when the part's fp32 h_s slice is staged.  The sender turns it into the fp16 planes, exchanges them
+//     (s + 1 < T) and stores the layer output (every step, the last one included).  Replaces an mbarrier arrive + sender poll;
+//     holding the pointwise warps until the sender arrives costs the chain nothing, because what they wait for next, acc_ready
+//     of the group's other part, needs the sender's previous send (h of that part) to have landed anyway.
+// Both sides of a barrier run the same (s, q) sequence from the same conditions (q < nparts per item, every s < T), and
+// bar.sync blocks every participant until all have arrived: no participant can arrive at generation n + 1 before generation n
+// completed, so generations cannot mix.  A participation mismatch would hang instead of trapping.
 constexpr uint32_t F_BAR_ACC = 1, F_BAR_SLICE = 5;
 __device__ __forceinline__ void fused_bar(uint32_t id, uint32_t threads, int tag, long long* wacc) {
     const long long t0 = wacc ? clock64() : 0;
@@ -508,51 +517,89 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
             uint32_t cta_delta[FC];                                            // [d]: address offset of CTA (rank + d) & 3 (static indices only)
 #pragma unroll
             for (uint32_t d = 0; d < FC; ++d) cta_delta[d] = mapa_shared(smem_base, (rank + d) & (FC - 1)) - smem_base;
+            // Lane l handles rows r(j) = (l >> 2) + 8 j (j = 0, 1), 8-unit chunk k = l & 3 of the fp32 slice: groups 2 k, 2 k + 1,
+            // at the adjacent slots 2 (k ^ m) + {0, 1}, m = (r >> 1) & 3 = (l >> 3) & 3 (pointwise warps above).  The 16-byte loads
+            // go by quarter warps; a quarter is two rows of the same m and all four k, so reading half (r & 1) of the chunk first
+            // makes each load instruction cover 8 distinct slots of 16 bytes, i.e. all 32 banks.
+            const int k = lane & 3, hs = (lane >> 2) & 1;
+            const uint32_t src_lane = (uint32_t)((lane >> 2) * 128 + ((2 * (k ^ ((lane >> 3) & 3)) + hs) << 4));
+            const float s1 = 1.f - kPlaneScale;
             // ph_b: h_free phase bits
-            for (int s = 0; s + 1 < T; ++s) {
+            for (int s = 0; s < T; ++s) {
+                const int t = dir == 0 ? s : T - 1 - s;
+                const bool exchange = s + 1 < T;                                   // no h is exchanged after the last step, only y stored
                 for (int q = warp - F_W_SEND; q < nparts; q += 4) {
                     const bool trl = tr_item && q == 0 && s >= F_TRACE_S0 && s < F_TRACE_S0 + F_TRACE_STEPS;
                     fused_bar(F_BAR_SLICE + (q & 3), 160, 1, wacc);               // the part's four pointwise warps have written h_s
-                    if (lane == 0) {
-                        if (trl) trace[(s - F_TRACE_S0) * 16 + 7] = clock64();
-                        // every CTA's recurrent MMAs of step s have finished reading the part's tile (it still holds h_{s-1})
-                        FUSED_WAIT(bar_h_free(q), (ph_b >> q) & 1u, 7);
+                    if (trl) trace[(s - F_TRACE_S0) * 16 + 7] = clock64();
+                    // h_s -> the scaled split (h1 . W_hi + h2 . W'), w1 / w2[j]: the 16-byte chunks (8 units) of row r(j); this
+                    // needs no h_free and runs while the peers' recurrent MMAs may still read the operand tile
+                    uint4 w1[2], w2[2];
+#pragma unroll
+                    for (int j = 0; j < 2; ++j) {
+                        const uint32_t src = smem_base + g_off + ((s & 1) * FMAXP + q) * F_BOX + j * 1024 + src_lane;
+                        float4 a, b;
+                        asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w) : "r"(src));
+                        asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(b.x), "=f"(b.y), "=f"(b.z), "=f"(b.w) : "r"(src ^ 16u));
+                        const float4 lo = hs ? b : a, hi = hs ? a : b;             // units 8 k .. 8 k + 3 and 8 k + 4 .. 8 k + 7
+                        split_scaled_f16x2(lo.x, lo.y, s1, w1[j].x, w2[j].x);
+                        split_scaled_f16x2(lo.z, lo.w, s1, w1[j].y, w2[j].y);
+                        split_scaled_f16x2(hi.x, hi.y, s1, w1[j].z, w2[j].z);
+                        split_scaled_f16x2(hi.z, hi.w, s1, w1[j].w, w2[j].w);
                     }
-                    ph_b ^= 1u << q;
-                    __syncwarp();
-                    const uint32_t src = smem_base + g_off + ((s & 1) * FMAXP + q) * F_BOX + lane * 16;
-                    const uint32_t dst = smem_base + h_off + q * F_HTILE + rank * F_BOX + lane * 16;
-                    const uint32_t bar = bar_h_ready(q);
+                    if (exchange) {
+                        if (lane == 0) FUSED_WAIT(bar_h_free(q), (ph_b >> q) & 1u, 7);   // every CTA's recurrent MMAs of step s have read
+                        ph_b ^= 1u << q;                                                  // the part's tile (it still holds h_{s-1})
+                        __syncwarp();
+                        // operand layout: row = sequence, chunk k (h1) / 4 + k (h2) of the 128-byte row at chunk ^ (row & 7)
+                        const uint32_t bar = bar_h_ready(q);
 #pragma unroll
-                    for (int c = 0; c < F_BOX / 512; ++c) {
-                        if (PROBE && (p.flags & 1) && c >= F_BOX / 1024) break;   // timing probe: half the exchange bytes
-                        uint4 v;
-                        asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(src + c * 512));
-                        // the three peers over DSMEM; the own copy is a plain shared-memory store (it does not take the SM-to-SM port)
+                        for (int j = 0; j < 2; ++j) {
+                            if (PROBE && (p.flags & 1) && j > 0) break;                   // timing probe: half the exchange bytes
+                            const int row = (lane >> 2) + 8 * j;
+                            const uint32_t dst_row = smem_base + h_off + q * F_HTILE + rank * F_BOX + row * 128;
 #pragma unroll
-                        for (uint32_t d = 1; d < FC; ++d) {
+                            for (int pl = 0; pl < 2; ++pl) {
+                                const uint4 v = pl ? w2[j] : w1[j];
+                                const uint32_t dst = dst_row + (((4 * pl + k) ^ (row & 7)) << 4);
+                                // the three peers over DSMEM; the own copy is a plain shared-memory store (it does not take the SM-to-SM port)
+#pragma unroll
+                                for (uint32_t d = 1; d < FC; ++d) {
 #if FUSED_EXCH_PLAIN
-                            asm volatile("st.shared::cluster.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(dst + c * 512 + cta_delta[d]),
-                                         "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+                                    asm volatile("st.shared::cluster.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(dst + cta_delta[d]),
+                                                 "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 #else
-                            st_async_v4(dst + c * 512 + cta_delta[d], v, bar + cta_delta[d]);
+                                    st_async_v4(dst + cta_delta[d], v, bar + cta_delta[d]);
 #endif
+                                }
+                                asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+                            }
                         }
-                        asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(dst + c * 512), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-                    }
 #if FUSED_EXCH_PLAIN
-                    // every lane: its generic stores (local and remote) before the tensor cores' async-proxy reads, and before
-                    // lane 0's release arrives at cluster scope
-                    fence_proxy_async_all();
-                    asm volatile("fence.acq_rel.cluster;" ::: "memory");
-                    __syncwarp();
-                    if (lane < FC) mbar_arrive_cluster(mapa_shared(bar, (uint32_t)lane));   // one arrive per destination CTA (own included)
+                        // every lane: its generic stores (local and remote) before the tensor cores' async-proxy reads, and before
+                        // lane 0's release arrives at cluster scope
+                        fence_proxy_async_all();
+                        asm volatile("fence.acq_rel.cluster;" ::: "memory");
+                        __syncwarp();
+                        if (lane < FC) mbar_arrive_cluster(mapa_shared(bar, (uint32_t)lane));   // one arrive per destination CTA (own included)
 #else
-                    fence_proxy_async();                                           // own copy: generic stores before the tensor core's reads
-                    __syncwarp();
-                    if (lane == 0) mbar_complete_tx(bar, (PROBE && (p.flags & 1)) ? F_BOX / 2 : F_BOX);
+                        fence_proxy_async();                                       // own copy: generic stores before the tensor core's reads
+                        __syncwarp();
+                        if (lane == 0) mbar_complete_tx(bar, (PROBE && (p.flags & 1)) ? F_BOX / 2 : F_BOX);
 #endif
+                    }
                     if (trl) trace[(s - F_TRACE_S0) * 16 + 8] = clock64();
+                    // layer output planes (B, T, 256): the same chunks, after the exchange so that the chain does not wait on them
+#pragma unroll
+                    for (int j = 0; j < 2; ++j) {
+                        const int b = seq0 + q * FPN + (lane >> 2) + 8 * j;
+                        if (b < p.B && !(PROBE && (p.flags & 2))) {
+                            const size_t off = ((size_t)b * T + t) * (2 * kHidden) + dir * kHidden + (int)rank * FU + 8 * k;
+                            *reinterpret_cast<uint4*>(p.y_a + off) = w1[j];
+                            *reinterpret_cast<uint4*>(p.y_b + off) = w2[j];
+                        }
+                    }
+                    if (trl) trace[(s - F_TRACE_S0) * 16 + 14] = clock64();
                 }
             }
         } else if ((warp >> 2) < nparts) {
@@ -566,21 +613,20 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
             float bias[4];                                                     // [gate] of unit 8 g + uu
 #pragma unroll
             for (int k = 0; k < 4; ++k) bias[k] = __ldg(p.bias + dir * kGates + k * kHidden + (int)rank * FU + 8 * g + uu);
-            const float s1 = 1.f - kPlaneScale;
             const float L2E2 = 2.f * kLog2e;
             float cst[2][4];
 #pragma unroll
             for (int a = 0; a < 2; ++a)
 #pragma unroll
                 for (int b = 0; b < 4; ++b) cst[a][b] = 0.f;
-            // after the staging pass: lane = (sequence row lane & 15, plane lane >> 4), the 16-byte chunk of this warp's 8 units
-            const int yrow = lane & 15;
-            __half* const yplane = (lane >> 4) ? p.y_b : p.y_a;
+            // staging slice of (step parity, part): fp32 h_s, [16 rows = sequences][8 groups of 4 units][4 B].  Group G = u >> 2 of
+            // unit u sits at group slot G ^ (((row >> 1) & 3) << 1).  This lane's cells are unit u = 8 g + uu of rows 2 jj + {0, 1,
+            // 8, 9}, all with (row >> 1) & 3 = jj: one column for all four, slot 2 (g ^ jj) + (uu >> 2), bank 4 slot + (uu & 3) --
+            // over the warp's (jj, uu) 32 distinct banks per store.  A group stays 16 contiguous bytes for the sender's 16-byte loads.
+            const int stg_col = ((((2 * g + (uu >> 2)) ^ (jj << 1)) << 2) + (uu & 3)) * 4 + 2 * jj * 128;
             // ph_a: acc_ready phase bits (bit pi; used by the group's poller only)
             const bool poller = g == pg;
             for (int s = 0; s < T; ++s) {
-                const int t = dir == 0 ? s : T - 1 - s;
-                const bool exchange = s + 1 < T;
 #pragma unroll
                 for (int pi = 0; pi < 2; ++pi) {
                     const int q = pg + 4 * pi;
@@ -625,26 +671,13 @@ lstm_fused_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
                         unpack2(h2v, hv[2 * jp], hv[2 * jp + 1]);
                     }
                     if (tr_on) trace[(s - F_TRACE_S0) * 16 + 10] = clock64();
-                    // h_s planes (scaled split: h1 . W_hi + h2 . W') -> the CTA's staging slice of (step parity, part), in operand
-                    // layout: row = sequence, 2-byte element uu of chunk g (h1) / 4 + g (h2) of the 128-byte swizzled row.  The slice
-                    // of this parity was last read by the copies of step s - 2, which landed before any CTA could start step s.
-                    unsigned char* const stg = smem_gen + g_off + ((s & 1) * FMAXP + q) * F_BOX;
+                    // h_s -> the CTA's staging slice of (step parity, part); the sender splits it into the fp16 planes.  The slice of
+                    // this parity was last read by the sender at step s - 2, before its exchange of step s - 1, which landed before
+                    // any CTA could start step s.
+                    unsigned char* const stg = smem_gen + g_off + ((s & 1) * FMAXP + q) * F_BOX + stg_col;
 #pragma unroll
-                    for (int c = 0; c < 4; ++c) {
-                        const int row = 2 * jj + (c & 1) + 8 * (c >> 1);
-                        __half a1, a2;
-                        split_scaled_f16(hv[c], s1, a1, a2);
-                        unsigned char* const rp = stg + row * 128 + uu * 2;
-                        *reinterpret_cast<__half*>(rp + ((g ^ (row & 7)) << 4)) = a1;
-                        *reinterpret_cast<__half*>(rp + (((4 + g) ^ (row & 7)) << 4)) = a2;
-                    }
-                    __syncwarp();
-                    if (exchange) fused_bar(F_BAR_SLICE + pg, 160, 4, wacc);       // hand the slice to sender warp pg (it reads it with plain loads)
-                    // layer output planes (B, T, 256) = the same chunks: lane = (row, plane), this warp's 16 bytes (8 units)
-                    const uint4 v = *reinterpret_cast<const uint4*>(stg + yrow * 128 + ((((lane >> 4) * 4 + g) ^ (yrow & 7)) << 4));
-                    const int b = seq0 + q * FPN + yrow;
-                    if (b < p.B && !(PROBE && (p.flags & 2)))
-                        *reinterpret_cast<uint4*>(yplane + ((size_t)b * T + t) * (2 * kHidden) + dir * kHidden + (int)rank * FU + 8 * g) = v;
+                    for (int c = 0; c < 4; ++c) *reinterpret_cast<float*>(stg + ((c & 1) + 8 * (c >> 1)) * 128) = hv[c];
+                    fused_bar(F_BAR_SLICE + pg, 160, 4, wacc);                     // hand the slice to sender warp pg (it reads it with plain loads)
                     if (tr_on) trace[(s - F_TRACE_S0) * 16 + 12] = clock64();
                 }
             }
@@ -774,11 +807,12 @@ int lstm_fused_launch(const __half* x_a, const __half* x_b, int64_t lda, int B, 
 
     const int nc = fused_max_clusters();
     // work items: parts of 16 sequences, spread evenly over items_per_dir items per direction (<= 8 parts each); choose the
-    // count that minimises waves x step time.  Measured step time (us) of a cluster with n parts in flight (256 x 500: n = 1,
-    // 2, 4; 4096 x 800: n = 8; in between interpolated): one part runs at the unloaded latency of the chain MMA -> pointwise ->
-    // exchange, eight parts overlap 3.3 chains' worth.  Small batches (streaming: 256 sequences) therefore spread over all 33
-    // clusters with one part each (0.80 instead of 1.21 ms per layer), large ones keep eight parts per cluster.
-    static const double kStepUs[FMAXP + 1] = {0.0, 1.60, 1.93, 2.17, 2.41, 2.78, 3.16, 3.53, 3.90};
+    // count that minimises waves x step time.  Measured step time (us) of a cluster with n parts in flight (B200 at 1 000 W,
+    // `tools/lstm_modes_timing.py 256,...,2048 500 1`: one wave of n = B / 256 parts on each of 32 clusters; profiles/r05_*):
+    // one part runs at the unloaded latency of the chain MMA -> pointwise -> exchange, eight parts overlap 2.8 chains' worth.
+    // Small batches (streaming: 256 sequences) therefore spread over 32 clusters with one part each, large ones keep eight
+    // parts per cluster.
+    static const double kStepUs[FMAXP + 1] = {0.0, 1.11, 1.41, 1.53, 1.70, 2.15, 2.60, 2.73, 3.06};
     const int P = (B + FPN - 1) / FPN;
     int best_ipd = (P + FMAXP - 1) / FMAXP;
     double best_cost = 1e30;
