@@ -172,6 +172,29 @@ B200VAD_API int b200vad_threshold_median(const float* prob, int B, int64_t T, fl
 B200VAD_API int b200vad_segments(const uint8_t* dec, const int64_t* offsets, int R, int64_t T, int min_run, int32_t* counts,
                      int64_t* seg_off, int32_t* seg, int64_t cap, void* stream);
 
+/* ---- speech regions with onset / offset hysteresis, padding and minimum durations: pyannote's
+ * Binarize(onset, offset, min_duration_on, min_duration_off, pad_onset, pad_offset) in the frame domain, the same controls
+ * as silero's get_speech_timestamps.  On a stream x[0, T) of probabilities:
+ *   1. a[t] = 1 if x[t] > onset, 0 if x[t] < offset, else a[t-1] (a[-1] = 0; NaN keeps the state);
+ *   2. every maximal run [s, e) of a becomes [max(0, s - pad_onset), min(T, e + pad_offset)); overlapping or touching ones merge;
+ *   3. two consecutive regions less than min_off frames apart merge (no gap before the first or after the last is filled);
+ *   4. regions shorter than min_on frames are dropped;
+ *   5. dec[t] = 1 inside the surviving regions; each one is the triple (stream, s, e - 1), ordered by (stream, s).
+ * Differences from pyannote's loop: a region still open at the last frame ends at T (pyannote: T - 1), and padded regions are
+ * clipped to [0, T).  Every count is in frames and 0 turns its step off.  Calls refuse (B200VAD_EINVAL) a non-finite threshold,
+ * offset > onset or a negative count. */
+typedef struct b200vad_binarize_params {
+    float onset, offset;
+    int32_t pad_onset, pad_offset, min_off, min_on;
+} b200vad_binarize_params;
+/* prob: flat f32 streams, stream r = prob[offsets[r], offsets[r+1]) (offsets: (R+1) i64), or NULL = R rows of T frames; with
+ * offsets, T is the length of the flat buffer, and dec frames outside [offsets[0], offsets[R]) are written 0.  dec: u8, same
+ * layout as prob.  counts (R) i32, seg_off (R+1) i64 (seg_off[R] = total), seg (cap, 3) i32 as b200vad_segments.  A stream of n
+ * frames holds at most ceil(n / 2) regions; nothing is written past cap, and dec is complete when cap >= seg_off[R] (dec is
+ * drawn from the written triples).  No workspace, no host synchronisation: the launch sequence can be captured in a graph. */
+B200VAD_API int b200vad_binarize(const float* prob, const int64_t* offsets, int R, int64_t T, const b200vad_binarize_params* params,
+                     uint8_t* dec, int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, void* stream);
+
 /* ---- 8f-1 scoring.  VadModel.test_step stat scores (src/engines/vad_engine.py:167-202): out4 (device, i64) =
  * tp, fp, tn, fn of dec (u8, != 0 is speech) against labels (u8) over n frames. */
 B200VAD_API int b200vad_stat_scores(const uint8_t* dec, const uint8_t* labels, int64_t n, int64_t* out4, void* stream);
@@ -228,7 +251,16 @@ B200VAD_API int b200vad_pipeline_sincnet_i16(const void* packed_model, const voi
                                  int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, void* workspace, size_t ws_bytes,
                                  void* stream);
 
-/* ---- host-buffer session: the same path with HOST waveforms and HOST results -- what a caller holding
+/* ---- whole path with binarization instead of threshold / median / run-length segments: packed_sincnet = NULL selects the
+ * fbank front end (b200vad_pipeline_fbank_*, lens optional), a SincNet blob the SincNet one (b200vad_pipeline_sincnet_*, lens
+ * must be NULL); wav_i16 != 0: int16 PCM rows.  b200vad_binarize runs on prob, which is the same as the existing entries' bit for
+ * bit; cap: B * ceil(T / 2) holds every region.  Workspace: b200vad_pipeline_workspace_bytes / b200vad_pipeline_sincnet_workspace_bytes. */
+B200VAD_API int b200vad_pipeline_binarize(const void* packed_model, const void* packed_sincnet, int num_layers, const void* wav,
+                              int wav_i16, const int32_t* lens, int B, int64_t N, int64_t wav_stride,
+                              const b200vad_binarize_params* params, float* prob, uint8_t* dec, int32_t* counts, int64_t* seg_off,
+                              int32_t* seg, int64_t cap, void* workspace, size_t ws_bytes, void* stream);
+
+/* ---- host-buffer session:the same path with HOST waveforms and HOST results -- what a caller holding
  * lhotse/DataLoader batches in host memory uses (src/engines/vad_engine.py:204-211 fed by
  * src/datasets/data_module.py:194-206).  The session owns device buffers for two batches in flight and three
  * CUDA streams (H2D / compute / D2H).
@@ -256,6 +288,10 @@ B200VAD_API int b200vad_session_submit_host(b200vad_session* s, int slot, const 
 B200VAD_API int b200vad_session_submit_host_i16(b200vad_session* s, int slot, const int16_t* wav_host, int B, float thr, int kernel,
                                     uint8_t* dec_host, float* prob_host);
 B200VAD_API int b200vad_session_wait(b200vad_session* s, int slot, int32_t* seg_host, int64_t cap, int64_t* nseg);
+/* params != NULL: the following submits (and run_host calls) post-process with b200vad_binarize and ignore their thr / kernel
+ * arguments; NULL: back to threshold / median / run-length segments.  A batch already submitted keeps the policy it was
+ * submitted with.  Segment buffers hold ceil(T / 2) regions per row either way, so switching allocates nothing. */
+B200VAD_API int b200vad_session_set_binarize(b200vad_session* s, const b200vad_binarize_params* params);
 /* Device timeline of the slot's most recent batch, in ms since the session was created:
  * ms[0..4] = H2D begin, H2D end, compute begin, compute end, D2H end (CUDA events on the three streams). */
 B200VAD_API int b200vad_session_slot_times(b200vad_session* s, int slot, float* ms);
@@ -277,6 +313,9 @@ B200VAD_API int b200vad_stream_create_sincnet(int device, const void* packed_mod
                                   int num_streams, int64_t window_samples, int hop_samples, int use_graph, b200vad_stream** out);
 B200VAD_API int b200vad_stream_push(b200vad_stream* s, const float* chunk, int chunk_on_host, float thr, int kernel, float* prob_new_host,
                         uint8_t* dec_new_host, float* device_ms);
+/* params != NULL: the following pushes binarize every window's probabilities (b200vad_binarize per stream; thr / kernel of push
+ * are then ignored); NULL: back to threshold / median.  Recaptures the graph (blocking). */
+B200VAD_API int b200vad_stream_set_binarize(b200vad_stream* s, const b200vad_binarize_params* params);
 /* parity / debugging: current windows (S, window) f32 and all frame outputs (S, T) of the last push, to host buffers */
 B200VAD_API int b200vad_stream_snapshot(b200vad_stream* s, float* window_host, float* prob_host, uint8_t* dec_host);
 B200VAD_API void b200vad_stream_destroy(b200vad_stream* s);

@@ -21,6 +21,16 @@ c_void_p, c_int, c_int64, c_size_t, c_float, c_double = C.c_void_p, C.c_int, C.c
 
 MAX_INPUT_DIM = 768     # B200VAD_MAX_INPUT_DIM: the widest LSTM input the model entry points accept
 
+
+
+class BinarizeParams(C.Structure):
+    """b200vad_binarize_params: thresholds and frame counts of the binarization (include/b200vad.h)."""
+    _fields_ = [("onset", C.c_float), ("offset", C.c_float), ("pad_onset", C.c_int32), ("pad_offset", C.c_int32),
+                ("min_off", C.c_int32), ("min_on", C.c_int32)]
+
+
+_P_BIN = C.POINTER(BinarizeParams)
+
 # name -> (restype, argtypes); mirrors include/b200vad.h one to one
 PROTOTYPES = {
     "b200vad_abi_version": (c_int, []),
@@ -59,6 +69,11 @@ PROTOTYPES = {
     "b200vad_median_window": (c_int, [c_double, c_double]),
     "b200vad_threshold_median": (c_int, [c_void_p, c_int, c_int64, c_float, c_int, c_void_p, c_int, c_void_p, c_float, c_void_p]),
     "b200vad_segments": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
+    "b200vad_binarize": (c_int, [c_void_p, c_void_p, c_int, c_int64, _P_BIN, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
+    "b200vad_pipeline_binarize": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int64, c_int64, _P_BIN,
+                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
+    "b200vad_session_set_binarize": (c_int, [c_void_p, _P_BIN]),
+    "b200vad_stream_set_binarize": (c_int, [c_void_p, _P_BIN]),
     "b200vad_stat_scores": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "b200vad_score_workspace_bytes": (c_size_t, [c_int64]),
     "b200vad_score_intervals": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int64, c_int, c_void_p,

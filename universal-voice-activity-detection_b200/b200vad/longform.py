@@ -15,6 +15,11 @@ is zero padded in AUDIO (the SincNet InstanceNorm sees the zeros; no lens), per-
 of ``ceil(get_num_frames(16000 d)) + 1`` frames per recording (predict_sincnet.py:330-337), run-length encoding that keeps
 single-frame runs and whole-second timestamps (predict_sincnet.py:348-370, 492-504).  Overlapped windows need a hop of whole
 SincNet frame steps (270 samples) so that every window's frames fall on one global grid.
+
+``binarize`` (a ``b200vad.Binarize``) replaces threshold / median / run-length segments: it runs once over the recording's
+probability stream -- the stitched one for hop < window, else the concatenated window probabilities cut to the frames the
+decision stream covers -- so a region that crosses a window boundary stays one region.  Intervals are then
+[first * step + t0, (last + 1) * step + t0) seconds on the mode's frame grid (b200vad.binarize), clipped to the duration.
 """
 
 from __future__ import annotations
@@ -23,6 +28,7 @@ from typing import Optional
 
 import torch
 
+from .binarize import mode_step
 from .host import (cut_into_windows, fbank_num_frames, get_num_frames, merge_intervals_with_buffer, recording_offsets,
                    segments_to_intervals)
 
@@ -32,8 +38,8 @@ SINC_STEP = 270       # samples between SincNet frames
 class LongFormVad:
     def __init__(self, packed: torch.Tensor, num_layers: int = 4, window: int = 80000, hop: Optional[int] = None,
                  thr: float = 0.5, kernel: int = 49, max_rows: int = 4096, frame_shift: float = 0.01,
-                 sincnet_packed: Optional[torch.Tensor] = None):
-        self.packed, self.L, self.sinc = packed, num_layers, sincnet_packed
+                 sincnet_packed: Optional[torch.Tensor] = None, binarize=None):
+        self.packed, self.L, self.sinc, self.binarize = packed, num_layers, sincnet_packed, binarize
         self.window, self.hop = int(window), int(hop if hop is not None else window)
         if self.sinc is not None:
             if self.window < 991 or not (0 < self.hop <= self.window):
@@ -97,6 +103,8 @@ class LongFormVad:
             p, d, _, _ = run(tail, lens[-1:])
             probs.append(p); decs.append(d)
         prob = torch.cat(probs) if probs else wav.new_empty((0, Tw))
+        if self.binarize is not None:
+            return self._binarized(prob, N, duration, wins)
         min_run = 1 if sinc else 2      # the SincNet RLE keeps single-frame runs (predict_sincnet.py:348-370)
         if self.hop == self.window:
             # reference semantics: per-window median filter, concatenation, per-recording slice, RLE
@@ -111,3 +119,22 @@ class LongFormVad:
             seg, _ = torch.ops.b200vad.segments(stream.view(1, -1), None, min_run)
         ivs = segments_to_intervals(seg.tolist(), 1, self.fs, sincnet_durations=[duration] if sinc else None)[0]
         return {"prob": prob, "stream_dec": stream, "intervals": merge_intervals_with_buffer(ivs, duration, 0), "windows": wins}
+
+    def probability_stream(self, prob: torch.Tensor, num_samples: int, duration: float) -> torch.Tensor:
+        """The recording's probability stream that binarization runs over: the stitched stream for hop < window, else the
+        concatenated window probabilities cut to the frames the decision stream of the reference's path covers."""
+        sinc = self.sinc is not None
+        if self.hop == self.window:
+            flat = prob.reshape(-1)
+            return flat[: recording_offsets([duration], flat.numel(), self.fs, sincnet=sinc)[1]]
+        L = get_num_frames(num_samples) if sinc else fbank_num_frames(num_samples)
+        return torch.ops.b200vad.stitch_center(prob, self.hop // (SINC_STEP if sinc else 160), L)
+
+    def _binarized(self, prob, num_samples, duration, wins):
+        step, t0 = mode_step(self.sinc is not None, self.fs)
+        f = self.binarize.frames(step)
+        sp = self.probability_stream(prob, num_samples, duration)
+        dec, seg, _ = torch.ops.b200vad.binarize(sp.view(1, -1), None, f["onset"], f["offset"], f["pad_onset"], f["pad_offset"],
+                                                 f["min_off"], f["min_on"])
+        ivs = self.binarize.intervals(seg.tolist(), 1, step, t0, [duration])[0]
+        return {"prob": prob, "stream_dec": dec.view(-1), "intervals": ivs, "windows": wins}

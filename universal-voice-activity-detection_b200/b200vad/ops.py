@@ -7,9 +7,13 @@
   b200vad::segments(dec, offsets?, min_run)         -> (S, 3) i32, (R) i32 [a8/a9]
   b200vad::vad_pipeline(wav, lens?, packed, L, thr, kernel) -> prob, dec, seg, counts
   b200vad::vad_pipeline_sincnet(wav, packed_model, packed_sincnet, L, thr, kernel) -> prob, dec, seg, counts
+  b200vad::binarize(prob, offsets?, onset, offset, pad_onset, pad_offset, min_off, min_on) -> dec, seg, counts
+  b200vad::vad_pipeline_binarize(wav, lens?, packed, packed_sincnet?, L, onset, offset, pads, min durations)
+                                                    -> prob, dec, seg, counts
 
 Each op enqueues on ``torch.cuda.current_stream()`` and never synchronises, except
-``segments`` / ``vad_pipeline`` which read one int64 (the segment total) to size their output.
+``segments`` / ``binarize`` and the exact-size ``vad_pipeline*`` ops, which read one int64 (the segment total) to size
+their output.
 """
 
 from __future__ import annotations
@@ -217,6 +221,54 @@ def _(dec, offsets=None, min_run=2):
     return dec.new_empty((n, 3), dtype=torch.int32), dec.new_empty((R,), dtype=torch.int32)
 
 
+# ------------------------------------------------------------------ binarization (onset / offset hysteresis, pads, min durations)
+def _bin_params(onset, offset, pad_onset, pad_offset, min_off, min_on):
+    return _lib.BinarizeParams(float(onset), float(offset), int(pad_onset), int(pad_offset), int(min_off), int(min_on))
+
+
+@torch.library.custom_op("b200vad::binarize", mutates_args=(), device_types="cuda")
+def binarize(prob: torch.Tensor, offsets: Optional[torch.Tensor], onset: float, offset: float, pad_onset: int, pad_offset: int,
+             min_off: int, min_on: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """pyannote's Binarize in frames (include/b200vad.h): prob (R, T) rows, or a flat (n,) buffer with offsets (R+1) int64 ->
+    dec (same shape) uint8, seg (S, 3) int32 (stream, first, last) ordered by (stream, first), counts (R,) int32.  One blocking
+    read of the region total to size seg.  b200vad.Binarize converts a policy in seconds to these frame counts."""
+    prob = _prep(prob, torch.float32, "prob")
+    dev = prob.device
+    if offsets is None:
+        if prob.dim() != 2:
+            raise _lib.B200VadError("prob must be (R, T) when offsets is None")
+        R, T = prob.shape
+        cap = R * ((T + 1) // 2)
+        off_ptr = None
+    else:
+        if prob.dim() != 1:
+            raise _lib.B200VadError("prob must be a flat (n,) buffer when offsets are given")
+        offsets = _prep(offsets.to(torch.int64), torch.int64, "offsets")
+        R, T = offsets.numel() - 1, prob.numel()
+        cap = (T + R) // 2 + 1          # >= sum of ceil(len_r / 2) over R streams of at most T frames in all
+        off_ptr = offsets.data_ptr()
+    dec = torch.empty(prob.shape, dtype=torch.uint8, device=dev)
+    counts = torch.zeros(max(R, 0), dtype=torch.int32, device=dev)
+    if R <= 0:
+        return dec.zero_(), torch.empty((0, 3), dtype=torch.int32, device=dev), counts
+    seg_off = torch.empty(R + 1, dtype=torch.int64, device=dev)
+    seg = torch.empty((cap, 3), dtype=torch.int32, device=dev)
+    params = _bin_params(onset, offset, pad_onset, pad_offset, min_off, min_on)
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().b200vad_binarize(prob.data_ptr(), off_ptr, R, T, params, dec.data_ptr(), counts.data_ptr(),
+                                               seg_off.data_ptr(), seg.data_ptr(), cap, _stream_ptr(dev)), "b200vad_binarize")
+    total = int(seg_off[R].item())
+    return dec, seg[:total].clone(), counts
+
+
+@binarize.register_fake
+def _(prob, offsets, onset, offset, pad_onset, pad_offset, min_off, min_on):
+    ctx = torch.library.get_ctx()
+    n = ctx.new_dynamic_size()
+    R = prob.shape[0] if offsets is None else offsets.numel() - 1
+    return prob.new_empty(prob.shape, dtype=torch.uint8), prob.new_empty((n, 3), dtype=torch.int32), prob.new_empty((R,), dtype=torch.int32)
+
+
 # ------------------------------------------------------------------ whole path
 def _seg_per_row(T: int, sincnet: bool) -> int:
     """Most segments a row of T frames can hold: runs of >= 2 frames (fbank path) or of >= 1 frame (the SincNet RLE,
@@ -224,10 +276,12 @@ def _seg_per_row(T: int, sincnet: bool) -> int:
     return (T + 1) // 2 if sincnet else (T + 2) // 3
 
 
-def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc=None):
+def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc=None, bin=None):
     """Enqueues the whole path on the current stream; returns device buffers only (nothing synchronises):
     prob (B, T) f32, dec (B, T) u8, seg (cap, 3) i32 of which the first seg_off[B] rows are valid, counts (B,) i32,
-    seg_off (B + 1,) i64.  ``sinc``: packed SincNet blob -> the SincNet -> PyanNet path (then ``lens`` must be None)."""
+    seg_off (B + 1,) i64.  ``sinc``: packed SincNet blob -> the SincNet -> PyanNet path (then ``lens`` must be None).
+    ``bin``: BinarizeParams -> binarization instead of threshold / median / segments (thr and kernel unused; the segment
+    capacity is B * ceil(T / 2))."""
     wav = _prep_rows(wav, "wav")
     if wav.dim() != 2:
         raise _lib.B200VadError("wav must be (B, N)")
@@ -248,7 +302,7 @@ def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc=None):
         return prob, dec, torch.empty((0, 3), dtype=torch.int32, device=dev), counts, seg_off
     if B > _MAX_PIPELINE_ROWS:
         raise _lib.B200VadError(f"one pipeline launch handles at most {_MAX_PIPELINE_ROWS} rows (vad_pipeline splits larger batches)")
-    cap = B * _seg_per_row(T, sinc is not None)
+    cap = B * ((T + 1) // 2 if bin is not None else _seg_per_row(T, sinc is not None))
     seg = torch.empty((cap, 3), dtype=torch.int32, device=dev)
     with torch.cuda.device(dev):
         _ensure(dev)
@@ -261,6 +315,12 @@ def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc=None):
             minimum = L.b200vad_pipeline_workspace_bytes(B, N) - L.b200vad_model_workspace_bytes(B, T) + \
                 L.b200vad_model_workspace_bytes(1, T)
             ws = _ws(min(need, max(_MAX_WS_BYTES, minimum)), dev)
+            if bin is not None:
+                _lib.check(L.b200vad_pipeline_binarize(packed.data_ptr(), None, num_layers, wav.data_ptr(), int(wav.dtype == torch.int16),
+                                                       lens_ptr, B, N, wav.stride(0), bin, prob.data_ptr(), dec.data_ptr(),
+                                                       counts.data_ptr(), seg_off.data_ptr(), seg.data_ptr(), cap, ws.data_ptr(),
+                                                       ws.numel(), _stream_ptr(dev)), "b200vad_pipeline_binarize")
+                return prob, dec, seg, counts, seg_off
             fn = L.b200vad_pipeline_fbank_i16 if wav.dtype == torch.int16 else L.b200vad_pipeline_fbank_f32
             _lib.check(fn(packed.data_ptr(), num_layers, wav.data_ptr(), lens_ptr, B, N, wav.stride(0),
                           float(thr), int(kernel), prob.data_ptr(), dec.data_ptr(), counts.data_ptr(),
@@ -272,6 +332,12 @@ def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc=None):
             need = L.b200vad_pipeline_sincnet_workspace_bytes(B, N)
             minimum = 256 * B * T + L.b200vad_pipeline_sincnet_workspace_bytes(1, N)    # + the whole batch's layer-0 planes
             ws = _ws(min(need, max(_MAX_WS_BYTES, minimum)), dev)
+            if bin is not None:
+                _lib.check(L.b200vad_pipeline_binarize(packed.data_ptr(), sinc.data_ptr(), num_layers, wav.data_ptr(),
+                                                       int(wav.dtype == torch.int16), None, B, N, wav.stride(0), bin, prob.data_ptr(),
+                                                       dec.data_ptr(), counts.data_ptr(), seg_off.data_ptr(), seg.data_ptr(), cap,
+                                                       ws.data_ptr(), ws.numel(), _stream_ptr(dev)), "b200vad_pipeline_binarize")
+                return prob, dec, seg, counts, seg_off
             fn = L.b200vad_pipeline_sincnet_i16 if wav.dtype == torch.int16 else L.b200vad_pipeline_sincnet_f32
             _lib.check(fn(packed.data_ptr(), sinc.data_ptr(), num_layers, wav.data_ptr(), B, N, wav.stride(0),
                           float(thr), int(kernel), prob.data_ptr(), dec.data_ptr(), counts.data_ptr(),
@@ -309,16 +375,17 @@ def vad_pipeline(wav: torch.Tensor, lens: Optional[torch.Tensor], packed: torch.
     return _pipeline_exact(wav, lens, packed, num_layers, thr, kernel)
 
 
-def _pipeline_exact(wav, lens, packed, num_layers, thr, kernel, sinc=None):
+def _pipeline_exact(wav, lens, packed, num_layers, thr, kernel, sinc=None, bin=None):
     B = wav.shape[0]
     if B <= _MAX_PIPELINE_ROWS:
-        prob, dec, seg, counts, seg_off = _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc)
+        prob, dec, seg, counts, seg_off = _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc, bin)
         total = int(seg_off[B].item()) if B > 0 else 0
         return prob, dec, seg[:total].clone(), counts
     outs = []
     for b0 in range(0, B, _MAX_PIPELINE_ROWS):
         sl = slice(b0, min(B, b0 + _MAX_PIPELINE_ROWS))
-        outs.append((b0,) + _pipeline_launch(wav[sl], None if lens is None else lens[sl], packed, num_layers, thr, kernel, sinc))
+        outs.append((b0,) + _pipeline_launch(wav[sl], None if lens is None else lens[sl], packed, num_layers, thr, kernel, sinc,
+                                             bin))
     segs = []
     for b0, _, _, seg, _, seg_off in outs:
         s = seg[: int(seg_off[-1].item())].clone()
@@ -374,6 +441,53 @@ def _(wav, packed_model, packed_sincnet, num_layers, thr, kernel):
     n = ctx.new_dynamic_size()
     B, N = wav.shape
     T = _sincnet_frames(N)
+    return (wav.new_empty((B, T), dtype=torch.float32), wav.new_empty((B, T), dtype=torch.uint8), wav.new_empty((n, 3), dtype=torch.int32),
+            wav.new_empty((B,), dtype=torch.int32))
+
+
+def _pipeline_frames(wav, packed_sincnet) -> int:
+    N = wav.shape[1]
+    return (N + 80) // 160 if packed_sincnet is None else _sincnet_frames(N)
+
+
+@torch.library.custom_op("b200vad::vad_pipeline_binarize_padded", mutates_args=(), device_types="cuda")
+def vad_pipeline_binarize_padded(wav: torch.Tensor, lens: Optional[torch.Tensor], packed: torch.Tensor,
+                                 packed_sincnet: Optional[torch.Tensor], num_layers: int, onset: float, offset: float, pad_onset: int,
+                                 pad_offset: int, min_off: int, min_on: int
+                                 ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """The whole path with binarization (``binarize`` on prob) and no host synchronisation: the fbank front end, or SincNet with
+    ``packed_sincnet`` (then ``lens`` must be None); float32 or int16 PCM rows.  prob equals vad_pipeline / vad_pipeline_sincnet
+    bit for bit.  The segment list comes back at its fixed capacity B * ceil(T / 2) with seg_off (B + 1,); rows [0, seg_off[B])
+    are valid (b200vad.SegmentGatherer takes them as they are)."""
+    return _pipeline_launch(wav, lens, packed, num_layers, 0.5, 49, packed_sincnet,
+                            _bin_params(onset, offset, pad_onset, pad_offset, min_off, min_on))
+
+
+@vad_pipeline_binarize_padded.register_fake
+def _(wav, lens, packed, packed_sincnet, num_layers, onset, offset, pad_onset, pad_offset, min_off, min_on):
+    B = wav.shape[0]
+    T = _pipeline_frames(wav, packed_sincnet)
+    return (wav.new_empty((B, T), dtype=torch.float32), wav.new_empty((B, T), dtype=torch.uint8),
+            wav.new_empty((B * ((T + 1) // 2), 3), dtype=torch.int32), wav.new_empty((B,), dtype=torch.int32),
+            wav.new_empty((B + 1,), dtype=torch.int64))
+
+
+@torch.library.custom_op("b200vad::vad_pipeline_binarize", mutates_args=(), device_types="cuda")
+def vad_pipeline_binarize(wav: torch.Tensor, lens: Optional[torch.Tensor], packed: torch.Tensor, packed_sincnet: Optional[torch.Tensor],
+                          num_layers: int, onset: float, offset: float, pad_onset: int, pad_offset: int, min_off: int,
+                          min_on: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """vad_pipeline_binarize_padded with an exact-size segment list: prob, dec, seg (S, 3), counts.  One blocking read of the
+    segment total per call; batches of more than 65 535 rows are split."""
+    return _pipeline_exact(wav, lens, packed, num_layers, 0.5, 49, packed_sincnet,
+                           _bin_params(onset, offset, pad_onset, pad_offset, min_off, min_on))
+
+
+@vad_pipeline_binarize.register_fake
+def _(wav, lens, packed, packed_sincnet, num_layers, onset, offset, pad_onset, pad_offset, min_off, min_on):
+    ctx = torch.library.get_ctx()
+    n = ctx.new_dynamic_size()
+    B = wav.shape[0]
+    T = _pipeline_frames(wav, packed_sincnet)
     return (wav.new_empty((B, T), dtype=torch.float32), wav.new_empty((B, T), dtype=torch.uint8), wav.new_empty((n, 3), dtype=torch.int32),
             wav.new_empty((B,), dtype=torch.int32))
 

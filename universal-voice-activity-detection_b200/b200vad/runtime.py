@@ -78,10 +78,13 @@ class HostSession:
 
     ``sincnet_packed`` (a ``pack_sincnet`` blob; ``packed`` then holds the D = 60 LSTM stack + head) selects the SincNet ->
     PyanNet path: ``T`` = get_num_frames(num_samples) frames per row, segments keep single-frame runs.
+
+    ``binarize`` (a ``b200vad.Binarize``, or ``set_binarize`` later) replaces threshold / median / run-length segments by
+    onset / offset hysteresis, pads and minimum durations on the mode's frame grid; ``thr`` / ``kernel`` are then ignored.
     """
 
     def __init__(self, packed: torch.Tensor, num_layers: int, num_samples: int, chunk_rows: int = 1024,
-                 device: Optional[int] = None, sincnet_packed: Optional[torch.Tensor] = None):
+                 device: Optional[int] = None, sincnet_packed: Optional[torch.Tensor] = None, binarize=None):
         from .host import fbank_num_frames, get_num_frames
         from .ops import _seg_per_row
         if not packed.is_cuda or (sincnet_packed is not None and not sincnet_packed.is_cuda):
@@ -101,6 +104,20 @@ class HostSession:
             _lib.check(_lib.lib().b200vad_session_create(self.device, packed.data_ptr(), num_layers, self.chunk_rows, self.N,
                                                          C.byref(h)), "b200vad_session_create")
         self._h = h
+        self.binarize = None
+        if binarize is not None:
+            self.set_binarize(binarize)
+
+    def set_binarize(self, binarize) -> None:
+        """Post-process the following batches with ``binarize`` (a ``b200vad.Binarize``), or with threshold / median /
+        run-length segments again when None.  A batch already submitted keeps its policy."""
+        from .binarize import mode_step
+        params = None if binarize is None else binarize.params(mode_step(self.sincnet_packed is not None)[0])
+        _lib.check(_lib.lib().b200vad_session_set_binarize(self._h, params), "b200vad_session_set_binarize")
+        self.binarize = binarize
+
+    def _cap(self, B: int) -> int:
+        return B * ((self.T + 1) // 2 if self.binarize is not None else self._seg_per_row)
 
     def run(self, wav: torch.Tensor, thr: float = 0.5, kernel: int = 49, want_dec: bool = True, want_prob: bool = False,
             out: Optional[dict] = None):
@@ -113,7 +130,7 @@ class HostSession:
             out["dec"] = torch.empty((B, self.T), dtype=torch.uint8).pin_memory()
         if want_prob and ("prob" not in out or out["prob"].shape[0] < B):
             out["prob"] = torch.empty((B, self.T), dtype=torch.float32).pin_memory()
-        cap = B * self._seg_per_row
+        cap = self._cap(B)
         if "seg_buf" not in out or out["seg_buf"].shape[0] < cap:
             out["seg_buf"] = torch.empty((max(cap, 1), 3), dtype=torch.int32).pin_memory()
         nseg = C.c_int64(0)
@@ -138,7 +155,7 @@ class HostSession:
             out["dec"] = torch.empty((B, self.T), dtype=torch.uint8).pin_memory()
         if want_prob and ("prob" not in out or out["prob"].shape[0] != B):
             out["prob"] = torch.empty((B, self.T), dtype=torch.float32).pin_memory()
-        cap = B * self._seg_per_row
+        cap = self._cap(B)
         if "seg_buf" not in out or out["seg_buf"].shape[0] < cap:
             out["seg_buf"] = torch.empty((max(cap, 1), 3), dtype=torch.int32).pin_memory()
         out["_wav"] = wav          # keep the source alive until wait()

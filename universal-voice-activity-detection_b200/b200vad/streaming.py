@@ -8,6 +8,9 @@ behind ``b200vad_stream_*`` (device ring buffers + one CUDA graph replay per pus
 With ``sincnet_packed`` the path is SincNet -> PyanNet: the hop must be a multiple of 270 samples (the SincNet frame step)
 so that every push adds whole frames, and a push returns the newest ``hop // 270`` of the window's get_num_frames(window)
 frames.
+
+With ``binarize`` (a ``b200vad.Binarize``, or ``set_binarize`` between pushes) every window's probabilities go through onset /
+offset hysteresis, pads and minimum durations instead of threshold / median; ``thr`` / ``kernel`` of ``push`` are then ignored.
 """
 
 from __future__ import annotations
@@ -22,7 +25,8 @@ from . import _lib
 
 class StreamingVad:
     def __init__(self, packed: torch.Tensor, num_layers: int = 4, num_streams: int = 256, window: int = 80000, hop: int = 160,
-                 use_graph: bool = True, device: Optional[int] = None, sincnet_packed: Optional[torch.Tensor] = None):
+                 use_graph: bool = True, device: Optional[int] = None, sincnet_packed: Optional[torch.Tensor] = None,
+                 binarize=None):
         from .host import get_num_frames
         sinc = sincnet_packed is not None
         if sinc and (int(hop) <= 0 or int(hop) % 270):
@@ -45,6 +49,17 @@ class StreamingVad:
         self._h = h
         self._prob = torch.empty((self.S, self.nf), dtype=torch.float32)
         self._dec = torch.empty((self.S, self.nf), dtype=torch.uint8)
+        self.binarize = None
+        if binarize is not None:
+            self.set_binarize(binarize)
+
+    def set_binarize(self, binarize) -> None:
+        """Binarize the windows of the following pushes with ``binarize`` (a ``b200vad.Binarize``), or threshold / median them
+        again when None.  Recaptures the session's graph."""
+        from .binarize import mode_step
+        params = None if binarize is None else binarize.params(mode_step(self.sincnet_packed is not None)[0])
+        _lib.check(_lib.lib().b200vad_stream_set_binarize(self._h, params), "b200vad_stream_set_binarize")
+        self.binarize = binarize
 
     def push(self, chunk: torch.Tensor, thr: float = 0.5, kernel: int = 49):
         """chunk: (S, hop) float32, CPU or CUDA.  Returns (prob (S, nf), dec (S, nf), device_ms)."""

@@ -5,6 +5,7 @@
 #include <string.h>
 #include <stdlib.h>
 #include <algorithm>
+#include <cmath>
 #include <atomic>
 #include <mutex>
 #include <utility>
@@ -825,6 +826,27 @@ int b200vad_threshold_median(const float* prob, int B, int64_t T, float thr, int
     return threshold_median_launch(prob, B, T, thr, kernel, out, elem_bytes, near_count, near_tol, (cudaStream_t)stream);
 }
 
+// B200VAD_EINVAL unless the thresholds are finite with offset <= onset and every count is >= 0
+static int check_binarize(const b200vad_binarize_params* p) {
+    B200VAD_CHECK_ARG(p, "null binarize params");
+    B200VAD_CHECK_ARG(std::isfinite(p->onset) && std::isfinite(p->offset) && p->offset <= p->onset,
+                      "binarize: onset and offset must be finite with offset <= onset");
+    B200VAD_CHECK_ARG(p->pad_onset >= 0 && p->pad_offset >= 0 && p->min_off >= 0 && p->min_on >= 0,
+                      "binarize: pads and minimum durations must be >= 0 frames");
+    return B200VAD_OK;
+}
+
+int b200vad_binarize(const float* prob, const int64_t* offsets, int R, int64_t T, const b200vad_binarize_params* params,
+                     uint8_t* dec, int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, void* stream) {
+    int rc = check_binarize(params);
+    if (rc) return rc;
+    B200VAD_CHECK_ARG(R >= 0 && T >= 0 && cap >= 0, "bad size");
+    B200VAD_CHECK_ARG(offsets || T <= INT32_MAX, "T must fit the int32 frame indices of the triples");
+    if (R == 0) return B200VAD_OK;
+    B200VAD_CHECK_ARG(prob && dec && counts && seg_off && (seg || cap == 0), "null pointer");
+    return binarize_launch(prob, offsets, T, R, *params, 0, dec, counts, seg_off, seg, cap, (cudaStream_t)stream);
+}
+
 int b200vad_segments(const uint8_t* dec, const int64_t* offsets, int R, int64_t T, int min_run, int32_t* counts,
                      int64_t* seg_off, int32_t* seg, int64_t cap, void* stream) {
     B200VAD_CHECK_ARG(R >= 0 && cap >= 0 && min_run >= 1, "bad size");
@@ -876,9 +898,6 @@ int b200vad_stitch_center(const float* prob, int num_windows, int frames_per_win
 // PyanNet).  Both hand the LSTM its layer-0 operand as fp16 (hi, lo) planes with row pitch round8(D).
 static inline int64_t fe_frames(bool sinc, int64_t N) { return sinc ? sinc_dims(N).P3 : b200vad_fbank_num_frames(N); }
 static inline int fe_dim(bool sinc) { return sinc ? 60 : kNumMel; }
-// segments per row at most: runs of >= 2 frames (fbank) are ceil(T / 3) apart, the SincNet RLE keeps single-frame runs
-// (predict_sincnet.py:348-370): ceil(T / 2)
-static inline int64_t fe_max_seg_per_row(bool sinc, int64_t T) { return sinc ? (T + 1) / 2 : (T + 2) / 3; }
 // layout: layer-0 input (fp32 features or planes, the same bytes) | fbank row sums | model workspace; the SincNet front end's
 // workspace shares the model's region (it is dead before the model runs on the same stream)
 static size_t fe_feat_bytes(bool sinc, int B, int64_t T) { return align_up(sizeof(float) * (size_t)B * T * round8(fe_dim(sinc))); }
@@ -899,8 +918,9 @@ size_t b200vad_pipeline_sincnet_workspace_bytes(int B, int64_t N) {
 }
 
 static int pipeline_run(const void* packed, const void* sinc, int L, const void* wav, int wav_i16, const int32_t* lens, int B,
-                        int64_t N, int64_t stride, float thr, int kernel, int row_base, float* prob, uint8_t* dec, int32_t* counts,
-                        int64_t* seg_off, int32_t* seg, int64_t cap, void* ws, size_t ws_bytes, cudaStream_t st) {
+                        int64_t N, int64_t stride, float thr, int kernel, const b200vad_binarize_params* bin, int row_base, float* prob,
+                        uint8_t* dec, int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, void* ws, size_t ws_bytes,
+                        cudaStream_t st) {
     B200VAD_CHECK_ARG(packed && wav && prob && dec && counts && seg_off && ws, "null pointer");
     B200VAD_CHECK_ARG((reinterpret_cast<uintptr_t>(ws) & 255) == 0, "workspace must be 256-byte aligned");
     const int64_t T = fe_frames(sinc != nullptr, N);
@@ -935,6 +955,7 @@ static int pipeline_run(const void* packed, const void* sinc, int L, const void*
     if (rc) return rc;
     rc = model_forward(packed, D, L, planes ? nullptr : feats, f_hi, f_lo, B, T, prob, w, ws_bytes - used, st);
     if (rc) return rc;
+    if (bin) return binarize_launch(prob, nullptr, T, B, *bin, row_base, dec, counts, seg_off, seg, cap, st);
     rc = threshold_median_launch(prob, B, T, thr, kernel, dec, 1, nullptr, 0.f, st);
     if (rc) return rc;
     return segments_launch(dec, nullptr, T, B, sinc ? 1 : 2, row_base, counts, seg_off, seg, cap, st);
@@ -944,7 +965,7 @@ int b200vad_pipeline_fbank_f32(const void* packed, int L, const float* wav, cons
                                int64_t stride, float thr, int kernel, float* prob, uint8_t* dec, int32_t* counts,
                                int64_t* seg_off, int32_t* seg, int64_t cap, void* ws, size_t ws_bytes, void* stream) {
     B200VAD_CHECK_ARG(B >= 0 && B <= 65535 && N >= 1 && stride >= 1, "bad shape");
-    return pipeline_run(packed, nullptr, L, wav, 0, lens, B, N, stride, thr, kernel, 0, prob, dec, counts, seg_off, seg, cap, ws,
+    return pipeline_run(packed, nullptr, L, wav, 0, lens, B, N, stride, thr, kernel, nullptr, 0, prob, dec, counts, seg_off, seg, cap, ws,
                         ws_bytes, (cudaStream_t)stream);
 }
 
@@ -952,7 +973,7 @@ int b200vad_pipeline_fbank_i16(const void* packed, int L, const int16_t* wav, co
                                int64_t stride, float thr, int kernel, float* prob, uint8_t* dec, int32_t* counts,
                                int64_t* seg_off, int32_t* seg, int64_t cap, void* ws, size_t ws_bytes, void* stream) {
     B200VAD_CHECK_ARG(B >= 0 && B <= 65535 && N >= 1 && stride >= 1, "bad shape");
-    return pipeline_run(packed, nullptr, L, wav, 1, lens, B, N, stride, thr, kernel, 0, prob, dec, counts, seg_off, seg, cap, ws,
+    return pipeline_run(packed, nullptr, L, wav, 1, lens, B, N, stride, thr, kernel, nullptr, 0, prob, dec, counts, seg_off, seg, cap, ws,
                         ws_bytes, (cudaStream_t)stream);
 }
 
@@ -962,7 +983,7 @@ static int pipeline_sincnet_entry(const void* packed, const void* sinc, int L, c
     B200VAD_CHECK_ARG(sinc, "null pointer");
     B200VAD_CHECK_ARG(L > 0 && B >= 0 && B <= 65535 && stride >= 1 && cap >= 0, "bad shape");
     B200VAD_CHECK_ARG(N >= 991, "waveform shorter than the SincNet receptive field (991 samples)");
-    return pipeline_run(packed, sinc, L, wav, wav_i16, nullptr, B, N, stride, thr, kernel, 0, prob, dec, counts, seg_off, seg, cap, ws,
+    return pipeline_run(packed, sinc, L, wav, wav_i16, nullptr, B, N, stride, thr, kernel, nullptr, 0, prob, dec, counts, seg_off, seg, cap, ws,
                         ws_bytes, (cudaStream_t)stream);
 }
 int b200vad_pipeline_sincnet_f32(const void* packed_model, const void* packed_sincnet, int num_layers, const float* wav, int B,
@@ -976,6 +997,21 @@ int b200vad_pipeline_sincnet_i16(const void* packed_model, const void* packed_si
                                  int64_t* seg_off, int32_t* seg, int64_t cap, void* ws, size_t ws_bytes, void* stream) {
     return pipeline_sincnet_entry(packed_model, packed_sincnet, num_layers, wav, 1, B, N, wav_stride, thr, kernel, prob, dec, counts,
                                   seg_off, seg, cap, ws, ws_bytes, stream);
+}
+
+int b200vad_pipeline_binarize(const void* packed_model, const void* packed_sincnet, int num_layers, const void* wav, int wav_i16,
+                              const int32_t* lens, int B, int64_t N, int64_t wav_stride, const b200vad_binarize_params* params,
+                              float* prob, uint8_t* dec, int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, void* ws,
+                              size_t ws_bytes, void* stream) {
+    int rc = check_binarize(params);
+    if (rc) return rc;
+    B200VAD_CHECK_ARG(num_layers > 0 && B >= 0 && B <= 65535 && N >= 1 && wav_stride >= 1 && cap >= 0, "bad shape");
+    if (packed_sincnet) {
+        B200VAD_CHECK_ARG(!lens, "the SincNet path takes no lens");
+        B200VAD_CHECK_ARG(N >= 991, "waveform shorter than the SincNet receptive field (991 samples)");
+    }
+    return pipeline_run(packed_model, packed_sincnet, num_layers, wav, wav_i16 != 0, lens, B, N, wav_stride, 0.f, 0, params, 0, prob,
+                        dec, counts, seg_off, seg, cap, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------- host-buffer session
@@ -1000,6 +1036,8 @@ struct b200vad_session {
     int L;
     int chunk;
     int64_t N, T, max_seg_per_row;
+    bool bin_on;            // b200vad_session_set_binarize
+    b200vad_binarize_params bin;
     cudaStream_t copy_stream, compute_stream, d2h_stream, seg_stream;
     cudaEvent_t epoch;      // recorded at creation; slot event times are reported relative to it
     SessionSlot slot[2];
@@ -1018,7 +1056,8 @@ static int session_create(int device, const void* packed_device, const void* sin
     memset(s, 0, sizeof(*s));
     s->device = device; s->packed = packed_device; s->sinc = sinc; s->L = num_layers; s->chunk = max_chunk_rows; s->N = N;
     s->T = fe_frames(sinc != nullptr, N);
-    s->max_seg_per_row = fe_max_seg_per_row(sinc != nullptr, s->T);
+    // segments per row at most: ceil(T / 2) single-frame runs (the SincNet RLE, binarization); the fbank RLE needs ceil(T / 3)
+    s->max_seg_per_row = (s->T + 1) / 2;
     cudaError_t e = cudaSuccess;
     auto ok = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
     ok(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
@@ -1072,7 +1111,8 @@ static int session_submit(b200vad_session* s, int slot, const void* wav_host, in
     B200VAD_CUDA(cudaEventRecord(sl.copied, s->copy_stream));
     B200VAD_CUDA(cudaStreamWaitEvent(s->compute_stream, sl.copied, 0));
     B200VAD_CUDA(cudaEventRecord(sl.compute_begin, s->compute_stream));
-    int rc = pipeline_run(s->packed, s->sinc, s->L, sl.wav_dev, wav_i16, nullptr, B, N, N, thr, kernel, row_base, sl.prob_dev, sl.dec_dev,
+    int rc = pipeline_run(s->packed, s->sinc, s->L, sl.wav_dev, wav_i16, nullptr, B, N, N, thr, kernel, s->bin_on ? &s->bin : nullptr,
+                          row_base, sl.prob_dev, sl.dec_dev,
                           sl.counts_dev, sl.seg_off_dev, sl.seg_dev, (int64_t)B * s->max_seg_per_row, s->ws, s->ws_bytes,
                           s->compute_stream);
     if (rc) return rc;
@@ -1134,6 +1174,17 @@ int b200vad_session_wait(b200vad_session* s, int slot, int32_t* seg_host, int64_
     }
     B200VAD_CUDA(cudaSetDevice(s->device));
     return session_wait(s, slot, seg_host, cap, nseg);
+}
+
+int b200vad_session_set_binarize(b200vad_session* s, const b200vad_binarize_params* params) {
+    B200VAD_CHECK_ARG(s, "null pointer");
+    if (params) {
+        int rc = check_binarize(params);
+        if (rc) return rc;
+        s->bin = *params;
+    }
+    s->bin_on = params != nullptr;
+    return B200VAD_OK;
 }
 
 int b200vad_session_slot_times(b200vad_session* s, int slot, float* ms) {
@@ -1224,6 +1275,8 @@ struct b200vad_stream {
     int64_t W, T;
     float thr;
     int kernel;
+    bool bin_on;            // b200vad_stream_set_binarize
+    b200vad_binarize_params bin;
     bool use_graph;
     cudaStream_t st;
     cudaGraph_t graph;
@@ -1232,6 +1285,8 @@ struct b200vad_stream {
     float *ring, *lin, *chunk, *feats, *prob, *prob_new, *prob_new_host;
     double* sums;
     uint8_t *dec, *dec_new, *dec_new_host;
+    int32_t *counts, *seg;  // binarization: per-stream region counts and triples (S * ceil(T / 2))
+    int64_t* seg_off;
     void* ws;
     size_t ws_bytes;
 };
@@ -1245,7 +1300,9 @@ static int stream_forward(b200vad_stream* s) {
     if (rc) return rc;
     rc = model_forward(s->packed, D, s->L, nullptr, f_hi, f_lo, s->S, s->T, s->prob, s->ws, s->ws_bytes, s->st);
     if (rc) return rc;
-    rc = threshold_median_launch(s->prob, s->S, s->T, s->thr, s->kernel, s->dec, 1, nullptr, 0.f, s->st);
+    rc = s->bin_on ? binarize_launch(s->prob, nullptr, s->T, s->S, s->bin, 0, s->dec, s->counts, s->seg_off, s->seg,
+                                     (int64_t)s->S * ((s->T + 1) / 2), s->st)
+                   : threshold_median_launch(s->prob, s->S, s->T, s->thr, s->kernel, s->dec, 1, nullptr, 0.f, s->st);
     if (rc) return rc;
     return stream_newest_launch(s->prob, s->dec, s->S, s->T, s->nf, s->prob_new, s->dec_new, s->st);
 }
@@ -1300,6 +1357,9 @@ static int stream_create(int device, const void* packed_device, const void* sinc
     ok(cudaMalloc(&s->dec, S * T));
     ok(cudaMalloc(&s->prob_new, sizeof(float) * S * s->nf));
     ok(cudaMalloc(&s->dec_new, S * s->nf));
+    ok(cudaMalloc(&s->counts, sizeof(int32_t) * S));
+    ok(cudaMalloc(&s->seg_off, sizeof(int64_t) * (S + 1)));
+    ok(cudaMalloc(&s->seg, sizeof(int32_t) * 3 * S * ((T + 1) / 2)));
     ok(cudaMallocHost(&s->prob_new_host, sizeof(float) * S * s->nf));
     ok(cudaMallocHost(&s->dec_new_host, S * s->nf));
     s->ws_bytes = b200vad_model_workspace_bytes(s->S, s->T);
@@ -1330,10 +1390,10 @@ int b200vad_stream_create_sincnet(int device, const void* packed_model, const vo
 int b200vad_stream_push(b200vad_stream* s, const float* chunk, int chunk_on_host, float thr, int kernel, float* prob_new_host,
                         uint8_t* dec_new_host, float* device_ms) {
     B200VAD_CHECK_ARG(s && chunk, "null pointer");
-    B200VAD_CHECK_ARG(kernel >= 1 && (kernel & 1), "median kernel must be odd");
+    B200VAD_CHECK_ARG(s->bin_on || (kernel >= 1 && (kernel & 1)), "median kernel must be odd");
     B200VAD_CUDA(cudaSetDevice(s->device));
     int rc;
-    if (thr != s->thr || kernel != s->kernel) {
+    if (!s->bin_on && (thr != s->thr || kernel != s->kernel)) {
         s->thr = thr; s->kernel = kernel;
         if (s->use_graph && (rc = stream_capture(s))) return rc;
     }
@@ -1362,6 +1422,18 @@ int b200vad_stream_push(b200vad_stream* s, const float* chunk, int chunk_on_host
     return B200VAD_OK;
 }
 
+int b200vad_stream_set_binarize(b200vad_stream* s, const b200vad_binarize_params* params) {
+    B200VAD_CHECK_ARG(s, "null pointer");
+    if (params) {
+        int rc = check_binarize(params);
+        if (rc) return rc;
+        s->bin = *params;
+    }
+    s->bin_on = params != nullptr;
+    B200VAD_CUDA(cudaSetDevice(s->device));
+    return s->use_graph ? stream_capture(s) : B200VAD_OK;
+}
+
 /* debugging / parity: copy the current buffered windows (S, window) and all frame outputs to the host */
 int b200vad_stream_snapshot(b200vad_stream* s, float* window_host, float* prob_host, uint8_t* dec_host) {
     B200VAD_CHECK_ARG(s, "null pointer");
@@ -1379,7 +1451,8 @@ void b200vad_stream_destroy(b200vad_stream* s) {
     if (s->st) cudaStreamSynchronize(s->st);
     if (s->exec) cudaGraphExecDestroy(s->exec);
     if (s->graph) cudaGraphDestroy(s->graph);
-    void* dev_ptrs[] = {s->ring, s->lin, s->chunk, s->feats, s->sums, s->prob, s->dec, s->prob_new, s->dec_new, s->ws};
+    void* dev_ptrs[] = {s->ring, s->lin, s->chunk, s->feats, s->sums, s->prob, s->dec, s->prob_new, s->dec_new, s->counts, s->seg_off,
+                        s->seg, s->ws};
     for (void* p : dev_ptrs) if (p) cudaFree(p);
     if (s->prob_new_host) cudaFreeHost(s->prob_new_host);
     if (s->dec_new_host) cudaFreeHost(s->dec_new_host);

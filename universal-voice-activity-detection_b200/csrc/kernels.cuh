@@ -1,6 +1,7 @@
 // Internal launcher interface shared by the translation units of libb200vad.so.
 #pragma once
 #include "common.cuh"
+#include "../../include/b200vad.h"
 
 namespace b200vad {
 
@@ -81,6 +82,9 @@ int threshold_median_launch(const float* prob, int B, int64_t T, float thr, int 
 // offsets == nullptr: R uniform rows of uniform_T frames
 int segments_launch(const uint8_t* dec, const int64_t* offsets, int64_t uniform_T, int R, int min_run, int row_base,
                     int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, cudaStream_t stream);
+// offsets == nullptr: R rows of T frames; else T = frames of the flat buffer (dec is written over [0, T)).  p is validated.
+int binarize_launch(const float* prob, const int64_t* offsets, int64_t T, int R, const b200vad_binarize_params& p, int row_base,
+                    uint8_t* dec, int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, cudaStream_t stream);
 int sinc_filters_launch(const float* low, const float* band, const float* window, const float* n, float* out, cudaStream_t s);
 int repack_conv_launch(const float* w, int Cout, int Cin, int k, float* out, cudaStream_t s);
 int wave_instnorm_launch(const float* wav, int B, int64_t N, int64_t stride, const float* gamma, const float* beta,

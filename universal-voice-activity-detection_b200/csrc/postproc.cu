@@ -214,4 +214,282 @@ int segments_launch(const uint8_t* dec, const int64_t* offsets, int64_t uniform_
     return B200VAD_OK;
 }
 
+// ---------------------------------------------------------------- binarization (onset / offset hysteresis, pads, min durations)
+// pyannote's Binarize in the frame domain (include/b200vad.h states the contract).  Steps 2-4 of the contract collapse into one
+// rule on the hysteresis output a[]: two consecutive regions [s1, e1), [s2, e2) belong to one group iff their gap
+// s2 - e1 < G = pad_onset + pad_offset + max(min_off, 1) (padded gap below max(min_off, 1): they overlap, touch or the gap is
+// filled).  A group [S, E) becomes [max(0, S - pad_onset), min(len, E + pad_offset)) and survives iff that is >= min_on
+// frames long.  So a group is closed when the NEXT group starts (or at the end of the stream), and no pad or duration needs a
+// halo: the kernel carries four numbers across chunks (hysteresis state, last region end, open group start, groups so far).
+//
+// One CTA per stream walks it in chunks of 2048 frames = 64 words of 32; every per-frame step is a ballot and every
+// cross-word step is a 64-entry scan by warp 0, so a chunk costs a fixed handful of barriers whatever its content.
+// Pass 1 counts, scan_counts_kernel orders the output by (r, s), pass 2 writes, binarize_raster_kernel fills dec from the
+// triples (a padded group can reach any distance back or forth, so dec is written once all groups are known).
+constexpr int kBinThreads = 256;
+constexpr int kBinWords = 64;                       // words per chunk
+constexpr int kBinChunk = 32 * kBinWords;           // frames per chunk
+constexpr int kBinRounds = kBinChunk / kBinThreads; // frames per thread per chunk
+
+// position of the last set bit of each of the 64 words before w, as an exclusive running "last" over the chunk (or `carry`);
+// warp 0, lane l owns words l and l + 32.  pos(w) = the word's own last position or -1.
+__device__ __forceinline__ void last_pos_scan(int lane, int64_t pos_lo, int64_t pos_hi, int64_t carry, int64_t* out /* [65] */) {
+    int64_t v = pos_lo;                              // inclusive running max over words 0..l (positions increase with w)
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        int64_t n = __shfl_up_sync(0xffffffffu, v, o);
+        if (lane >= o) v = max(v, n);
+    }
+    int64_t lo_incl = max(v, carry);
+    int64_t lo_tot = __shfl_sync(0xffffffffu, lo_incl, 31);
+    v = pos_hi;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        int64_t n = __shfl_up_sync(0xffffffffu, v, o);
+        if (lane >= o) v = max(v, n);
+    }
+    int64_t hi_incl = max(v, lo_tot);
+    int64_t lo_excl = __shfl_up_sync(0xffffffffu, lo_incl, 1);
+    int64_t hi_excl = __shfl_up_sync(0xffffffffu, hi_incl, 1);
+    out[lane] = lane ? lo_excl : carry;
+    out[lane + 32] = lane ? hi_excl : lo_tot;
+    if (lane == 31) out[64] = hi_incl;
+}
+
+template <bool WRITE>
+__global__ void __launch_bounds__(kBinThreads)
+binarize_kernel(const float* __restrict__ prob, const int64_t* __restrict__ offsets, int64_t uniform_T, b200vad_binarize_params p,
+                int row_base, int32_t* __restrict__ counts, const int64_t* __restrict__ seg_off, int32_t* __restrict__ seg, int64_t cap) {
+    const int r = blockIdx.x;
+    const int64_t beg = offsets ? offsets[r] : (int64_t)r * uniform_T;
+    const int64_t len = offsets ? offsets[r + 1] - beg : uniform_T;
+    const float* x = prob + beg;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int64_t gap_break = (int64_t)p.pad_onset + p.pad_offset + max(p.min_off, 1);
+    __shared__ unsigned s1w[kBinWords], s0w[kBinWords], aw[kBinWords], stw[kBinWords], enw[kBinWords], gsw[kBinWords], emw[kBinWords];
+    __shared__ int cin[kBinWords + 1];
+    __shared__ int64_t last_end[kBinWords + 1], last_gs[kBinWords + 1];
+    __shared__ int emit_off[kBinWords + 1];
+    __shared__ int c_a;                // hysteresis state before the chunk
+    __shared__ int64_t c_end, c_gs;    // last region end, start of the open group (-1: none)
+    __shared__ int64_t c_count;        // surviving groups so far
+    if (tid == 0) { c_a = 0; c_end = -1; c_gs = -1; c_count = 0; }
+    __syncthreads();
+    const int64_t out_base = WRITE ? seg_off[r] : 0;
+    // a group [gs, ge) of raw frames -> 1 if it survives, with its padded, clipped bounds
+    auto survive = [&](int64_t gs, int64_t ge, int64_t& a, int64_t& b) {
+        a = gs - p.pad_onset;
+        if (a < 0) a = 0;
+        b = ge + p.pad_offset;
+        if (b > len) b = len;
+        return b - a >= p.min_on;
+    };
+    for (int64_t base = 0; base < len; base += kBinChunk) {
+        // 1. the frames that set the state to 1 / to 0
+#pragma unroll
+        for (int k = 0; k < kBinRounds; ++k) {
+            const int64_t t = base + k * kBinThreads + tid;
+            const float v = t < len ? __ldg(x + t) : 0.f;
+            const unsigned m1 = __ballot_sync(0xffffffffu, t < len && v > p.onset);
+            const unsigned m0 = __ballot_sync(0xffffffffu, t < len && v < p.offset);
+            if (lane == 0) { s1w[k * 8 + warp] = m1; s0w[k * 8 + warp] = m0; }
+        }
+        __syncthreads();
+        // 2. hysteresis state entering every word: the value of the last setting frame before it
+        if (warp == 0) {
+            auto last_val = [&](int w) { unsigned s = s1w[w] | s0w[w]; return (int)((s1w[w] >> (31 - __clz(s))) & 1u); };
+            const unsigned h_lo = __ballot_sync(0xffffffffu, (s1w[lane] | s0w[lane]) != 0);
+            const unsigned h_hi = __ballot_sync(0xffffffffu, (s1w[lane + 32] | s0w[lane + 32]) != 0);
+            const unsigned long long H = (unsigned long long)h_lo | ((unsigned long long)h_hi << 32);
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                const int w = lane + 32 * h;
+                const unsigned long long m = H & ((1ull << w) - 1ull);
+                cin[w] = m ? last_val(63 - __clzll(m)) : c_a;
+            }
+            if (lane == 0) cin[kBinWords] = H ? last_val(63 - __clzll(H)) : c_a;
+        }
+        __syncthreads();
+        // 3. a[] per frame: the last setting frame at or before it in the word, else the word's carry-in
+#pragma unroll
+        for (int k = 0; k < kBinRounds; ++k) {
+            const int w = k * 8 + warp;
+            const unsigned s = (s1w[w] | s0w[w]) & (0xffffffffu >> (31 - lane));
+            const int a = s ? (int)((s1w[w] >> (31 - __clz(s))) & 1u) : cin[w];
+            const unsigned m = __ballot_sync(0xffffffffu, a && base + k * kBinThreads + tid < len);
+            if (lane == 0) aw[w] = m;
+        }
+        __syncthreads();
+        // 4. region starts and ends (an end is the first 0 after a run; the end at len is the flush below); last end before each word
+        if (warp == 0) {
+            int64_t pos[2];
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                const int w = lane + 32 * h;
+                const unsigned prev = w ? aw[w - 1] >> 31 : (unsigned)c_a;
+                const int64_t t0 = base + 32 * w;
+                const unsigned valid = t0 >= len ? 0u : (len - t0 >= 32 ? 0xffffffffu : (1u << (len - t0)) - 1u);
+                const unsigned shifted = (aw[w] << 1) | prev;
+                stw[w] = aw[w] & ~shifted;
+                enw[w] = ~aw[w] & shifted & valid;
+                pos[h] = enw[w] ? t0 + 31 - __clz(enw[w]) : -1;
+            }
+            last_pos_scan(lane, pos[0], pos[1], c_end, last_end);
+        }
+        __syncthreads();
+        // 5. group starts: the first region, or a region whose gap to the previous region end is >= gap_break
+#pragma unroll
+        for (int k = 0; k < kBinRounds; ++k) {
+            const int w = k * 8 + warp;
+            const int64_t t = base + k * kBinThreads + tid;
+            int g = 0;
+            if ((stw[w] >> lane) & 1u) {
+                const unsigned below = enw[w] & ((1u << lane) - 1u);
+                const int64_t pe = below ? base + 32 * w + 31 - __clz(below) : last_end[w];
+                g = pe < 0 || t - pe >= gap_break;
+            }
+            const unsigned m = __ballot_sync(0xffffffffu, g);
+            if (lane == 0) gsw[w] = m;
+        }
+        __syncthreads();
+        if (warp == 0) {
+            int64_t pos[2];
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                const int w = lane + 32 * h;
+                pos[h] = gsw[w] ? base + 32 * w + 31 - __clz(gsw[w]) : -1;
+            }
+            last_pos_scan(lane, pos[0], pos[1], c_gs, last_gs);
+        }
+        __syncthreads();
+        // 6. every group start closes the group before it: [previous group start, last region end before this start)
+        int64_t gs_prev[kBinRounds], ge_prev[kBinRounds];
+#pragma unroll
+        for (int k = 0; k < kBinRounds; ++k) {
+            const int w = k * 8 + warp;
+            int e = 0;
+            gs_prev[k] = -1; ge_prev[k] = -1;
+            if ((gsw[w] >> lane) & 1u) {
+                const unsigned gb = gsw[w] & ((1u << lane) - 1u), eb = enw[w] & ((1u << lane) - 1u);
+                gs_prev[k] = gb ? base + 32 * w + 31 - __clz(gb) : last_gs[w];
+                ge_prev[k] = eb ? base + 32 * w + 31 - __clz(eb) : last_end[w];
+                int64_t a, b;
+                e = gs_prev[k] >= 0 && survive(gs_prev[k], ge_prev[k], a, b);
+            }
+            const unsigned m = __ballot_sync(0xffffffffu, e);
+            if (lane == 0) emw[w] = m;
+        }
+        __syncthreads();
+        if (warp == 0) {
+            const int c_lo = __popc(emw[lane]), c_hi = __popc(emw[lane + 32]);
+            int v = c_lo;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                int n = __shfl_up_sync(0xffffffffu, v, o);
+                if (lane >= o) v += n;
+            }
+            const int lo_tot = __shfl_sync(0xffffffffu, v, 31);
+            emit_off[lane] = v - c_lo;
+            int u = c_hi;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                int n = __shfl_up_sync(0xffffffffu, u, o);
+                if (lane >= o) u += n;
+            }
+            emit_off[lane + 32] = lo_tot + u - c_hi;
+            if (lane == 31) emit_off[kBinWords] = lo_tot + u;
+        }
+        __syncthreads();
+        if (WRITE) {
+#pragma unroll
+            for (int k = 0; k < kBinRounds; ++k) {
+                const int w = k * 8 + warp;
+                if ((emw[w] >> lane) & 1u) {
+                    const int64_t o = out_base + c_count + emit_off[w] + __popc(emw[w] & ((1u << lane) - 1u));
+                    int64_t a, b;
+                    survive(gs_prev[k], ge_prev[k], a, b);
+                    if (o < cap) {
+                        seg[o * 3 + 0] = r + row_base;
+                        seg[o * 3 + 1] = (int)a;
+                        seg[o * 3 + 2] = (int)(b - 1);
+                    }
+                }
+            }
+        }
+        __syncthreads();
+        if (tid == 0) {
+            c_a = cin[kBinWords];
+            c_end = last_end[kBinWords];
+            c_gs = last_gs[kBinWords];
+            c_count += emit_off[kBinWords];
+        }
+        __syncthreads();
+    }
+    if (tid == 0) {
+        // the last group ends at the last region end, or at len if a region is still open
+        int64_t a, b;
+        const int64_t ge = c_a ? len : c_end;
+        const bool last = c_gs >= 0 && survive(c_gs, ge, a, b);
+        if (!WRITE) {
+            counts[r] = (int32_t)(c_count + last);
+        } else if (last) {
+            const int64_t o = out_base + c_count;
+            if (o < cap) {
+                seg[o * 3 + 0] = r + row_base;
+                seg[o * 3 + 1] = (int)a;
+                seg[o * 3 + 2] = (int)(b - 1);
+            }
+        }
+    }
+}
+
+// dec[i] = 1 iff frame i lies in one of its stream's (disjoint, sorted) written groups: a binary search per frame
+__global__ void __launch_bounds__(256)
+binarize_raster_kernel(const int64_t* __restrict__ offsets, int64_t uniform_T, int R, int64_t total, const int64_t* __restrict__ seg_off,
+                       const int32_t* __restrict__ seg, int64_t cap, uint8_t* __restrict__ dec) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    int r;
+    int64_t t;
+    if (offsets) {
+        // the last stream starting at or before i (skips empty streams); frames outside [offsets[0], offsets[R]) are no stream's
+        if (i < offsets[0] || i >= offsets[R]) { dec[i] = 0; return; }
+        int lo = 0, hi = R - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (offsets[mid] <= i) lo = mid; else hi = mid - 1;
+        }
+        r = lo;
+        t = i - offsets[r];
+    } else {
+        r = (int)(i / uniform_T);
+        t = i - (int64_t)r * uniform_T;
+    }
+    int64_t lo = seg_off[r], hi = min(seg_off[r + 1], cap) - 1;   // last group with start <= t
+    int64_t found = -1;
+    while (lo <= hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (seg[mid * 3 + 1] <= t) { found = mid; lo = mid + 1; } else hi = mid - 1;
+    }
+    dec[i] = found >= 0 && t <= seg[found * 3 + 2];
+}
+
+int binarize_launch(const float* prob, const int64_t* offsets, int64_t T, int R, const b200vad_binarize_params& p, int row_base,
+                    uint8_t* dec, int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, cudaStream_t stream) {
+    if (R == 0) return B200VAD_OK;
+    const int64_t uniform_T = offsets ? 0 : T;
+    binarize_kernel<false><<<R, kBinThreads, 0, stream>>>(prob, offsets, uniform_T, p, row_base, counts, nullptr, nullptr, 0);
+    B200VAD_LAUNCH_CHECK();
+    scan_counts_kernel<<<1, 1024, 0, stream>>>(counts, R, seg_off);
+    B200VAD_LAUNCH_CHECK();
+    binarize_kernel<true><<<R, kBinThreads, 0, stream>>>(prob, offsets, uniform_T, p, row_base, counts, seg_off, seg, cap);
+    B200VAD_LAUNCH_CHECK();
+    const int64_t total = offsets ? T : (int64_t)R * T;
+    if (total > 0) {
+        binarize_raster_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(offsets, uniform_T, R, total, seg_off, seg, cap, dec);
+        B200VAD_LAUNCH_CHECK();
+    }
+    return B200VAD_OK;
+}
+
 }  // namespace b200vad
