@@ -195,6 +195,42 @@ typedef struct b200vad_binarize_params {
 B200VAD_API int b200vad_binarize(const float* prob, const int64_t* offsets, int R, int64_t T, const b200vad_binarize_params* params,
                      uint8_t* dec, int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, void* stream);
 
+/* ---- streaming speech start / end events: the binarization above, carried across pushes.  A stream's TIMELINE is the sequence
+ * of frames it was given since its state was last zeroed; frame tau is column k of the call that passed it.  Events are defined
+ * so that, once the stream ends, its (start, end) pairs are exactly the regions b200vad_binarize gives on the whole timeline
+ * (T = the timeline length then).  With gap_break = pad_onset + pad_offset + max(min_off, 1), the regions of a[] fall into
+ * groups (a region starts a new group iff it is the first or starts >= gap_break frames after the previous region's end); a
+ * group [gs, ge) becomes the region [s, e) = [max(0, gs - pad_onset), min(T, ge + pad_offset)) and survives iff e - s >= min_on.
+ *   start(s): emitted at the first frame t of the group at which it survives whatever comes next.  The worst case is the stream
+ *             ending right after t: min(t + 1, ge + pad_offset) - s >= min_on, with ge = t + 1 while a[t] = 1 and the last
+ *             region end otherwise.  Equivalently, t is the first frame at which the regions of timeline[0, t] contain one that
+ *             starts at s (padded regions of different groups are disjoint, so at most one does).
+ *   end(e):   e = ge + pad_offset (exclusive), for a group whose start was emitted, emitted at frame ge + gap_break - 1: from
+ *             there on no onset can join the group.  At that frame t + 1 > e, so e needs no clipping.  Equivalently, t is the
+ *             first frame at which the regions of timeline[0, t] followed by max(min_on, 1) frames of +inf have [s, e)
+ *             followed by another region: the +inf run either joins the group (then the group's region is the last one) or
+ *             is a surviving region of its own.
+ *   end of stream: the open group is closed at T with clipping, as b200vad_binarize closes its last group: if its start was
+ *             emitted, end(min(T, ge + pad_offset)) with ge = T while a[T - 1] = 1.  A group whose start was not emitted does
+ *             not survive: at frame T - 1 the start test above evaluated min(T, ge + pad_offset) - s >= min_on, which is the
+ *             survival test itself.  So an end of stream emits at most one event.
+ * At most one event per frame: a frame confirms a start only for the open group, and an end only for that same group.  The
+ * start bound reaches its final value ge + pad_offset - s at frame ge + pad_offset - 1 <= ge + gap_break - 2 (gap_break >=
+ * pad_offset + 1), so a group that survives has its start emitted before the frame that emits its end.  A call of nf frames
+ * emits at most nf events, nf + 1 with an end of stream.  Event frames (s, then e, then the next group's s > e) increase
+ * within a stream, and no event is ever retracted: a group's left edge is fixed once it opens.
+ *
+ * State: (S, 5) i64 per stream, all zero = a fresh stream: [0] hysteresis a of the last frame, [1] last region end, [2] open
+ * group start gs, [3] group status (0 none open, 1 open, 2 open and its start emitted), [4] timeline length.
+ * b200vad_regions_step advances stream r by the nf frames prob[r * row_stride + k], k < nf, and writes its events to
+ * ev (S, cap_per_stream, 2) i64 as (frame, kind: 1 start, 0 end) in frame order, ev_counts[r] = events of the call (entries past
+ * cap_per_stream are counted, not written; nf + 1 always suffices).  flush (S) u8, optional: after its frames, a stream with
+ * flush[r] != 0 ends (the end-of-stream rule) and its state is zeroed.  nf = 0 only flushes.  All pointers device; no
+ * workspace, no host synchronisation: it can be captured in a graph, and each replay carries the state forward. */
+B200VAD_API int b200vad_regions_step(const float* prob, int S, int nf, int64_t row_stride, const b200vad_binarize_params* params,
+                         int64_t* state, const uint8_t* flush, int64_t* ev, int32_t* ev_counts, int64_t cap_per_stream,
+                         void* stream);
+
 /* ---- 8f-1 scoring.  VadModel.test_step stat scores (src/engines/vad_engine.py:167-202): out4 (device, i64) =
  * tp, fp, tn, fn of dec (u8, != 0 is speech) against labels (u8) over n frames. */
 B200VAD_API int b200vad_stat_scores(const uint8_t* dec, const uint8_t* labels, int64_t n, int64_t* out4, void* stream);
@@ -316,6 +352,20 @@ B200VAD_API int b200vad_stream_push(b200vad_stream* s, const float* chunk, int c
 /* params != NULL: the following pushes binarize every window's probabilities (b200vad_binarize per stream; thr / kernel of push
  * are then ignored); NULL: back to threshold / median.  Recaptures the graph (blocking). */
 B200VAD_API int b200vad_stream_set_binarize(b200vad_stream* s, const b200vad_binarize_params* params);
+/* Speech start / end events (b200vad_regions_step) on every stream's timeline of prob_new frames.  params != NULL turns them on
+ * or changes the policy, NULL turns them off.  Every stream's open group is first ended under the old policy; tracking restarts
+ * from the next frame, with frame indices continuing along the timeline.  Recaptures the graph (blocking).  With events on, a
+ * push runs b200vad_regions_step on prob_new inside its graph and copies the events back in one extra copy; with them off the
+ * push is unchanged. */
+B200VAD_API int b200vad_stream_set_events(b200vad_stream* s, const b200vad_binarize_params* params);
+/* End the n distinct slots streams[0, n) between pushes: their open groups end (end events when events are on), their rows of
+ * the ring and the window are zeroed and their timelines restart at frame 0, so a new caller in a slot sees what a fresh
+ * session sees.  Other slots are untouched.  Blocking.  An index out of [0, num_streams) or a repeated one: B200VAD_EINVAL. */
+B200VAD_API int b200vad_stream_end(b200vad_stream* s, const int32_t* streams, int n);
+/* Drain the events collected since the last call as (stream, kind: 1 start / 0 end, frame) i64 triples, ordered by push, then
+ * stream, then frame: at most cap, oldest first, *n = triples written; the rest stay queued.  ev_host = NULL with cap = 0 sets
+ * *n to the number queued and drains nothing. */
+B200VAD_API int b200vad_stream_events(b200vad_stream* s, int64_t* ev_host, int64_t cap, int64_t* n);
 /* parity / debugging: current windows (S, window) f32 and all frame outputs (S, T) of the last push, to host buffers */
 B200VAD_API int b200vad_stream_snapshot(b200vad_stream* s, float* window_host, float* prob_host, uint8_t* dec_host);
 B200VAD_API void b200vad_stream_destroy(b200vad_stream* s);

@@ -74,6 +74,10 @@ PROTOTYPES = {
                                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
     "b200vad_session_set_binarize": (c_int, [c_void_p, _P_BIN]),
     "b200vad_stream_set_binarize": (c_int, [c_void_p, _P_BIN]),
+    "b200vad_regions_step": (c_int, [c_void_p, c_int, c_int, c_int64, _P_BIN, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
+    "b200vad_stream_set_events": (c_int, [c_void_p, _P_BIN]),
+    "b200vad_stream_end": (c_int, [c_void_p, c_void_p, c_int]),
+    "b200vad_stream_events": (c_int, [c_void_p, c_void_p, c_int64, C.POINTER(c_int64)]),
     "b200vad_stat_scores": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "b200vad_score_workspace_bytes": (c_size_t, [c_int64]),
     "b200vad_score_intervals": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int64, c_int, c_void_p,

@@ -31,6 +31,26 @@ def mode_step(sincnet: bool, frame_shift: float = 0.01):
     return (SINC_STEP, SINC_T0) if sincnet else (float(frame_shift), FBANK_T0)
 
 
+def stream_event_seconds(frames, sincnet: bool, window: int) -> np.ndarray:
+    """Timeline frames of a streaming session (b200vad_stream_events) -> seconds since the stream's first sample.
+
+    A push that brings the stream to n samples returns the newest nf = hop / step_samples frames of the window of the last
+    ``window`` samples, which starts at sample n - window; timeline frame tau of that push is window frame j = T - nf + k with
+    n = (tau - k + nf) * hop / nf.  Window frame j lies at j * step + t0 seconds after the window's start, so tau lies at
+    (n - window) / 16000 + j * step + t0, and the push-dependent terms cancel:
+
+      fbank   : T = window / 160 frames of 160 samples, t0 = 0:  tau * 0.01 s.  Every newest frame lands on the stream's 10 ms grid.
+      SincNet : step = 270 / 16000, t0 = 496 / 16000, T = get_num_frames(window):
+                tau * 270 / 16000 + (270 * T - window + 496) / 16000 s.  get_num_frames(window) * 270 <= window - 721 (the
+                receptive field is 991 samples), so the offset is negative for every window; the result is clipped at 0.
+    """
+    frames = np.asarray(frames, dtype=np.float64)
+    if not sincnet:
+        return frames * 0.01
+    from .host import get_num_frames
+    return np.maximum(frames * SINC_STEP + (270 * get_num_frames(int(window)) - int(window) + 496) / 16000, 0.0)
+
+
 class Binarize:
     """Binarize(onset=0.5, offset=None, min_duration_on=0.0, min_duration_off=0.0, pad_onset=0.0, pad_offset=0.0).
 

@@ -10,6 +10,8 @@
   b200vad::binarize(prob, offsets?, onset, offset, pad_onset, pad_offset, min_off, min_on) -> dec, seg, counts
   b200vad::vad_pipeline_binarize(wav, lens?, packed, packed_sincnet?, L, onset, offset, pads, min durations)
                                                     -> prob, dec, seg, counts
+  b200vad::regions_step(prob, state, onset, offset, pad_onset, pad_offset, min_off, min_on, flush?)
+                                                    -> ev (S, nf + 1, 2) i64, counts (S,) i32; mutates state
 
 Each op enqueues on ``torch.cuda.current_stream()`` and never synchronises, except
 ``segments`` / ``binarize`` and the exact-size ``vad_pipeline*`` ops, which read one int64 (the segment total) to size
@@ -267,6 +269,43 @@ def _(prob, offsets, onset, offset, pad_onset, pad_offset, min_off, min_on):
     n = ctx.new_dynamic_size()
     R = prob.shape[0] if offsets is None else offsets.numel() - 1
     return prob.new_empty(prob.shape, dtype=torch.uint8), prob.new_empty((n, 3), dtype=torch.int32), prob.new_empty((R,), dtype=torch.int32)
+
+
+@torch.library.custom_op("b200vad::regions_step", mutates_args=("state",), device_types="cuda")
+def regions_step(prob: torch.Tensor, state: torch.Tensor, onset: float, offset: float, pad_onset: int, pad_offset: int, min_off: int,
+                 min_on: int, flush: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Speech start / end events on streams fed a chunk at a time (include/b200vad.h, b200vad_regions_step): prob (S, nf) f32
+    are the next nf frames of S streams, state (S, 5) int64 (zeros = fresh streams) is advanced in place.  Returns ev
+    (S, nf + 1, 2) int64 rows (frame, kind: 1 start / 0 end), of which the first counts[r] of stream r are valid (the rest
+    unspecified), and counts (S,) int32.  flush (S,) bool, optional: those streams end after their frames (their open group is
+    closed, their state zeroed).  Never synchronises."""
+    prob = _prep(prob, torch.float32, "prob")
+    if prob.dim() != 2:
+        raise _lib.B200VadError("prob must be (S, nf)")
+    S, nf = prob.shape
+    if state.dtype != torch.int64 or tuple(state.shape) != (S, 5) or not state.is_contiguous() or state.device != prob.device:
+        raise _lib.B200VadError("state must be a contiguous (S, 5) int64 tensor on prob's device")
+    dev = prob.device
+    flush_ptr = None
+    if flush is not None:
+        if flush.numel() != S:
+            raise _lib.B200VadError("flush must hold one flag per stream")
+        flush = _prep(flush.reshape(S).to(torch.uint8), torch.uint8, "flush")
+        flush_ptr = flush.data_ptr()
+    ev = torch.empty((S, nf + 1, 2), dtype=torch.int64, device=dev)
+    counts = torch.empty(S, dtype=torch.int32, device=dev)
+    params = _bin_params(onset, offset, pad_onset, pad_offset, min_off, min_on)
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().b200vad_regions_step(prob.data_ptr() if prob.numel() else None, S, nf, nf, params, state.data_ptr(),
+                                                   flush_ptr, ev.data_ptr(), counts.data_ptr(), nf + 1, _stream_ptr(dev)),
+                   "b200vad_regions_step")
+    return ev, counts
+
+
+@regions_step.register_fake
+def _(prob, state, onset, offset, pad_onset, pad_offset, min_off, min_on, flush=None):
+    S, nf = prob.shape
+    return prob.new_empty((S, nf + 1, 2), dtype=torch.int64), prob.new_empty((S,), dtype=torch.int32)
 
 
 # ------------------------------------------------------------------ whole path

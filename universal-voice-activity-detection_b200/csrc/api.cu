@@ -847,6 +847,17 @@ int b200vad_binarize(const float* prob, const int64_t* offsets, int R, int64_t T
     return binarize_launch(prob, offsets, T, R, *params, 0, dec, counts, seg_off, seg, cap, (cudaStream_t)stream);
 }
 
+int b200vad_regions_step(const float* prob, int S, int nf, int64_t row_stride, const b200vad_binarize_params* params,
+                         int64_t* state, const uint8_t* flush, int64_t* ev, int32_t* ev_counts, int64_t cap_per_stream,
+                         void* stream) {
+    int rc = check_binarize(params);
+    if (rc) return rc;
+    B200VAD_CHECK_ARG(S >= 0 && nf >= 0 && row_stride >= nf && cap_per_stream >= 0, "bad size");
+    if (S == 0) return B200VAD_OK;
+    B200VAD_CHECK_ARG(state && ev_counts && (prob || nf == 0) && (ev || cap_per_stream == 0), "null pointer");
+    return regions_step_launch(prob, S, nf, row_stride, *params, state, flush, ev, ev_counts, cap_per_stream, (cudaStream_t)stream);
+}
+
 int b200vad_segments(const uint8_t* dec, const int64_t* offsets, int R, int64_t T, int min_run, int32_t* counts,
                      int64_t* seg_off, int32_t* seg, int64_t cap, void* stream) {
     B200VAD_CHECK_ARG(R >= 0 && cap >= 0 && min_run >= 1, "bad size");
@@ -1289,9 +1300,22 @@ struct b200vad_stream {
     int64_t* seg_off;
     void* ws;
     size_t ws_bytes;
+    // speech events (b200vad_stream_set_events): device state (S, 5) and flush mask (S); one buffer holding ev (S, nf + 1, 2)
+    // then ev_counts (S), copied to its pinned twin by one copy per push; the drained triples queue on the host
+    bool ev_on;
+    b200vad_binarize_params evp;
+    int64_t* ev_state;
+    uint8_t *ev_flush, *ev_flush_host;
+    void *ev_dev, *ev_host;
+    int64_t pushes;         // pushes so far; stream i's timeline holds (pushes - born[i]) * nf frames
+    int64_t *born, *ev_base; // per stream: push at which its timeline began, timeline frame of its event tracking's frame 0
+    int64_t *ev_list, ev_n, ev_cap;
 };
 
-static int stream_forward(b200vad_stream* s) {
+static inline size_t stream_ev_bytes(const b200vad_stream* s) { return sizeof(int64_t) * (size_t)s->S * (s->nf + 1) * 2; }
+
+// warm_up: the events step runs on 0 frames, which leaves its state as it is
+static int stream_forward(b200vad_stream* s, bool warm_up = false) {
     const int D = fe_dim(s->sinc != nullptr);
     __half* f_hi = reinterpret_cast<__half*>(s->feats);
     __half* f_lo = f_hi + (size_t)s->S * s->T * round8(D);
@@ -1304,13 +1328,49 @@ static int stream_forward(b200vad_stream* s) {
                                      (int64_t)s->S * ((s->T + 1) / 2), s->st)
                    : threshold_median_launch(s->prob, s->S, s->T, s->thr, s->kernel, s->dec, 1, nullptr, 0.f, s->st);
     if (rc) return rc;
-    return stream_newest_launch(s->prob, s->dec, s->S, s->T, s->nf, s->prob_new, s->dec_new, s->st);
+    rc = stream_newest_launch(s->prob, s->dec, s->S, s->T, s->nf, s->prob_new, s->dec_new, s->st);
+    if (rc || !s->ev_on) return rc;
+    int64_t* ev = static_cast<int64_t*>(s->ev_dev);
+    return regions_step_launch(s->prob_new, s->S, warm_up ? 0 : s->nf, s->nf, s->evp, s->ev_state, nullptr, ev,
+                               reinterpret_cast<int32_t*>(reinterpret_cast<char*>(ev) + stream_ev_bytes(s)), s->nf + 1, s->st);
+}
+
+// after the events of one call are in ev_host: queue them as (stream, kind, timeline frame) triples, in stream then frame order
+static int stream_queue_events(b200vad_stream* s) {
+    const int64_t* ev = static_cast<const int64_t*>(s->ev_host);
+    const int32_t* counts = reinterpret_cast<const int32_t*>(static_cast<const char*>(s->ev_host) + stream_ev_bytes(s));
+    for (int i = 0; i < s->S; ++i) {
+        for (int j = 0; j < counts[i]; ++j) {
+            if (s->ev_n == s->ev_cap) {
+                const int64_t cap = std::max<int64_t>(1024, 2 * s->ev_cap);
+                int64_t* p = static_cast<int64_t*>(realloc(s->ev_list, sizeof(int64_t) * 3 * cap));
+                if (!p) { set_error("stream events: out of host memory"); return B200VAD_ENOMEM; }
+                s->ev_list = p; s->ev_cap = cap;
+            }
+            const int64_t* e = ev + ((int64_t)i * (s->nf + 1) + j) * 2;
+            int64_t* o = s->ev_list + 3 * s->ev_n++;
+            o[0] = i; o[1] = e[1]; o[2] = s->ev_base[i] + e[0];
+        }
+    }
+    return B200VAD_OK;
+}
+
+// end the groups of the streams in ev_flush_host under the current policy (events on), and queue their end events.  Blocking.
+static int stream_flush_events(b200vad_stream* s) {
+    B200VAD_CUDA(cudaMemcpyAsync(s->ev_flush, s->ev_flush_host, s->S, cudaMemcpyHostToDevice, s->st));
+    int64_t* ev = static_cast<int64_t*>(s->ev_dev);
+    int rc = regions_step_launch(nullptr, s->S, 0, 0, s->evp, s->ev_state, s->ev_flush, ev,
+                                 reinterpret_cast<int32_t*>(reinterpret_cast<char*>(ev) + stream_ev_bytes(s)), s->nf + 1, s->st);
+    if (rc) return rc;
+    B200VAD_CUDA(cudaMemcpyAsync(s->ev_host, s->ev_dev, stream_ev_bytes(s) + sizeof(int32_t) * s->S, cudaMemcpyDeviceToHost, s->st));
+    B200VAD_CUDA(cudaStreamSynchronize(s->st));
+    return stream_queue_events(s);
 }
 
 static int stream_capture(b200vad_stream* s) {
     if (s->exec) { cudaGraphExecDestroy(s->exec); s->exec = nullptr; }
     if (s->graph) { cudaGraphDestroy(s->graph); s->graph = nullptr; }
-    int rc = stream_forward(s);                         // warm-up: one-time function attributes, table init
+    int rc = stream_forward(s, true);                   // warm-up: one-time function attributes, table init
     if (rc) return rc;
     B200VAD_CUDA(cudaStreamSynchronize(s->st));
     B200VAD_CUDA(cudaStreamBeginCapture(s->st, cudaStreamCaptureModeThreadLocal));
@@ -1362,12 +1422,21 @@ static int stream_create(int device, const void* packed_device, const void* sinc
     ok(cudaMalloc(&s->seg, sizeof(int32_t) * 3 * S * ((T + 1) / 2)));
     ok(cudaMallocHost(&s->prob_new_host, sizeof(float) * S * s->nf));
     ok(cudaMallocHost(&s->dec_new_host, S * s->nf));
+    ok(cudaMalloc(&s->ev_state, sizeof(int64_t) * S * 5));
+    ok(cudaMalloc(&s->ev_flush, S));
+    ok(cudaMallocHost(&s->ev_flush_host, S));
+    ok(cudaMalloc(&s->ev_dev, stream_ev_bytes(s) + sizeof(int32_t) * S));
+    ok(cudaMallocHost(&s->ev_host, stream_ev_bytes(s) + sizeof(int32_t) * S));
+    s->born = static_cast<int64_t*>(calloc(S, sizeof(int64_t)));
+    s->ev_base = static_cast<int64_t*>(calloc(S, sizeof(int64_t)));
+    if (!s->born || !s->ev_base) ok(cudaErrorMemoryAllocation);
     s->ws_bytes = b200vad_model_workspace_bytes(s->S, s->T);
     if (sinc)   // the front end's workspace is dead before the model runs on the same stream
         s->ws_bytes = std::max(s->ws_bytes, (size_t)std::min<int64_t>(s->S, sinc_chunk_rows(s->W)) * sinc_ws_per_row(s->W) + 4096);
     ok(cudaMalloc(&s->ws, s->ws_bytes));
     if (e == cudaSuccess) ok(cudaMemsetAsync(s->ring, 0, sizeof(float) * S * 2 * W, s->st));
     if (e == cudaSuccess) ok(cudaMemsetAsync(s->lin, 0, sizeof(float) * S * W, s->st));
+    if (e == cudaSuccess) ok(cudaMemsetAsync(s->ev_state, 0, sizeof(int64_t) * S * 5, s->st));
     if (e != cudaSuccess) {
         set_error("b200vad_stream_create: %s", cudaGetErrorString(e));
         b200vad_stream_destroy(s);
@@ -1414,10 +1483,14 @@ int b200vad_stream_push(b200vad_stream* s, const float* chunk, int chunk_on_host
     const size_t n = (size_t)s->S * s->nf;
     B200VAD_CUDA(cudaMemcpyAsync(s->prob_new_host, s->prob_new, sizeof(float) * n, cudaMemcpyDeviceToHost, s->st));
     B200VAD_CUDA(cudaMemcpyAsync(s->dec_new_host, s->dec_new, n, cudaMemcpyDeviceToHost, s->st));
+    if (s->ev_on)
+        B200VAD_CUDA(cudaMemcpyAsync(s->ev_host, s->ev_dev, stream_ev_bytes(s) + sizeof(int32_t) * s->S, cudaMemcpyDeviceToHost, s->st));
     B200VAD_CUDA(cudaEventRecord(s->e1, s->st));
     B200VAD_CUDA(cudaEventSynchronize(s->e1));
+    ++s->pushes;
     if (prob_new_host) memcpy(prob_new_host, s->prob_new_host, sizeof(float) * n);
     if (dec_new_host) memcpy(dec_new_host, s->dec_new_host, n);
+    if (s->ev_on && (rc = stream_queue_events(s))) return rc;
     if (device_ms) B200VAD_CUDA(cudaEventElapsedTime(device_ms, s->e0, s->e1));
     return B200VAD_OK;
 }
@@ -1432,6 +1505,62 @@ int b200vad_stream_set_binarize(b200vad_stream* s, const b200vad_binarize_params
     s->bin_on = params != nullptr;
     B200VAD_CUDA(cudaSetDevice(s->device));
     return s->use_graph ? stream_capture(s) : B200VAD_OK;
+}
+
+int b200vad_stream_set_events(b200vad_stream* s, const b200vad_binarize_params* params) {
+    B200VAD_CHECK_ARG(s, "null pointer");
+    if (params) {
+        int rc = check_binarize(params);
+        if (rc) return rc;
+    }
+    B200VAD_CUDA(cudaSetDevice(s->device));
+    if (s->ev_on) {             // end every stream's open group under the old policy; this zeroes the state
+        memset(s->ev_flush_host, 1, s->S);
+        int rc = stream_flush_events(s);
+        if (rc) return rc;
+    }
+    s->ev_on = params != nullptr;
+    if (params) s->evp = *params;
+    for (int i = 0; i < s->S; ++i) s->ev_base[i] = (s->pushes - s->born[i]) * s->nf;
+    return s->use_graph ? stream_capture(s) : B200VAD_OK;
+}
+
+int b200vad_stream_end(b200vad_stream* s, const int32_t* streams, int n) {
+    B200VAD_CHECK_ARG(s && (streams || n == 0), "null pointer");
+    B200VAD_CHECK_ARG(n >= 0 && n <= s->S, "bad count");
+    memset(s->ev_flush_host, 0, s->S);
+    for (int j = 0; j < n; ++j) {
+        B200VAD_CHECK_ARG(streams[j] >= 0 && streams[j] < s->S, "stream index out of range");
+        B200VAD_CHECK_ARG(!s->ev_flush_host[streams[j]], "repeated stream index");
+        s->ev_flush_host[streams[j]] = 1;
+    }
+    if (n == 0) return B200VAD_OK;
+    B200VAD_CUDA(cudaSetDevice(s->device));
+    if (s->ev_on) {
+        int rc = stream_flush_events(s);
+        if (rc) return rc;
+    }
+    for (int j = 0; j < n; ++j) {
+        const int i = streams[j];
+        B200VAD_CUDA(cudaMemsetAsync(s->ring + (size_t)i * 2 * s->W, 0, sizeof(float) * 2 * s->W, s->st));
+        B200VAD_CUDA(cudaMemsetAsync(s->lin + (size_t)i * s->W, 0, sizeof(float) * s->W, s->st));
+        s->born[i] = s->pushes;
+        s->ev_base[i] = 0;
+    }
+    B200VAD_CUDA(cudaStreamSynchronize(s->st));
+    return B200VAD_OK;
+}
+
+int b200vad_stream_events(b200vad_stream* s, int64_t* ev_host, int64_t cap, int64_t* n) {
+    B200VAD_CHECK_ARG(s && n && (ev_host || cap == 0) && cap >= 0, "bad argument");
+    if (!ev_host) { *n = s->ev_n; return B200VAD_OK; }
+    const int64_t k = std::min(cap, s->ev_n);
+    if (k == 0) { *n = 0; return B200VAD_OK; }
+    memcpy(ev_host, s->ev_list, sizeof(int64_t) * 3 * k);
+    memmove(s->ev_list, s->ev_list + 3 * k, sizeof(int64_t) * 3 * (s->ev_n - k));
+    s->ev_n -= k;
+    *n = k;
+    return B200VAD_OK;
 }
 
 /* debugging / parity: copy the current buffered windows (S, window) and all frame outputs to the host */
@@ -1452,10 +1581,11 @@ void b200vad_stream_destroy(b200vad_stream* s) {
     if (s->exec) cudaGraphExecDestroy(s->exec);
     if (s->graph) cudaGraphDestroy(s->graph);
     void* dev_ptrs[] = {s->ring, s->lin, s->chunk, s->feats, s->sums, s->prob, s->dec, s->prob_new, s->dec_new, s->counts, s->seg_off,
-                        s->seg, s->ws};
+                        s->seg, s->ws, s->ev_state, s->ev_flush, s->ev_dev};
     for (void* p : dev_ptrs) if (p) cudaFree(p);
-    if (s->prob_new_host) cudaFreeHost(s->prob_new_host);
-    if (s->dec_new_host) cudaFreeHost(s->dec_new_host);
+    void* host_ptrs[] = {s->prob_new_host, s->dec_new_host, s->ev_flush_host, s->ev_host};
+    for (void* p : host_ptrs) if (p) cudaFreeHost(p);
+    free(s->born); free(s->ev_base); free(s->ev_list);
     if (s->e0) cudaEventDestroy(s->e0);
     if (s->e1) cudaEventDestroy(s->e1);
     if (s->st) cudaStreamDestroy(s->st);

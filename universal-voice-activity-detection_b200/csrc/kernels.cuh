@@ -85,6 +85,9 @@ int segments_launch(const uint8_t* dec, const int64_t* offsets, int64_t uniform_
 // offsets == nullptr: R rows of T frames; else T = frames of the flat buffer (dec is written over [0, T)).  p is validated.
 int binarize_launch(const float* prob, const int64_t* offsets, int64_t T, int R, const b200vad_binarize_params& p, int row_base,
                     uint8_t* dec, int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, cudaStream_t stream);
+// b200vad_regions_step on validated arguments (prob may be null when nf == 0)
+int regions_step_launch(const float* prob, int S, int nf, int64_t row_stride, const b200vad_binarize_params& p, int64_t* state,
+                        const uint8_t* flush, int64_t* ev, int32_t* ev_counts, int64_t cap, cudaStream_t stream);
 int sinc_filters_launch(const float* low, const float* band, const float* window, const float* n, float* out, cudaStream_t s);
 int repack_conv_launch(const float* w, int Cout, int Cin, int k, float* out, cudaStream_t s);
 int wave_instnorm_launch(const float* wav, int B, int64_t N, int64_t stride, const float* gamma, const float* beta,

@@ -492,4 +492,105 @@ int binarize_launch(const float* prob, const int64_t* offsets, int64_t T, int R,
     return B200VAD_OK;
 }
 
+
+// ---------------------------------------------------------------- streaming speech events (include/b200vad.h states the contract)
+// One warp per stream walks its new frames 32 at a time, with the group rule of binarize_kernel.  Per word, every lane owns one
+// frame and finds from ballots of the word and the carried state: the hysteresis value (last setting frame at or before it),
+// region starts and ends, the last region end at or before it, whether a rise starts a new group (no group open, or >= gap_break
+// frames after that end), whether its frame closes the open group (a[t] = 0 and t = last end + gap_break - 1), the group in
+// effect during its frame and that group's start test.  A start is the first frame of a group whose test passes; an end is a
+// close whose test passes.  So a word costs a fixed handful of ballots and the events come out compacted, in frame order.
+constexpr int kEvWarps = 4;
+
+__global__ void __launch_bounds__(32 * kEvWarps)
+regions_step_kernel(const float* __restrict__ prob, int S, int nf, int64_t row_stride, b200vad_binarize_params p,
+                    int64_t* __restrict__ state, const uint8_t* __restrict__ flush, int64_t* __restrict__ ev,
+                    int32_t* __restrict__ ev_counts, int64_t cap) {
+    const int r = blockIdx.x * kEvWarps + (threadIdx.x >> 5);
+    if (r >= S) return;
+    const int lane = threadIdx.x & 31;
+    const unsigned lt = (1u << lane) - 1u, le = lt | (1u << lane);
+    const int64_t gap_break = (int64_t)p.pad_onset + p.pad_offset + max(p.min_off, 1);
+    int64_t* st = state + (int64_t)r * 5;
+    int h = (int)st[0], status = (int)st[3];
+    int64_t last_end = st[1], gs = st[2];
+    const int64_t len = st[4];
+    const float* x = prob + (int64_t)r * row_stride;
+    int64_t* out = ev + (int64_t)r * cap * 2;
+    int64_t n = 0;
+    auto last = [](unsigned m) { return 31 - __clz(m); };
+    for (int base = 0; base < nf; base += 32) {
+        const int nv = min(32, nf - base);
+        const bool valid = lane < nv;
+        const unsigned vm = nv == 32 ? 0xffffffffu : (1u << nv) - 1u;
+        const int64_t t0 = len + base, t = t0 + lane;
+        const float v = valid ? __ldg(x + base + lane) : 0.f;
+        const unsigned m1 = __ballot_sync(0xffffffffu, valid && v > p.onset);
+        const unsigned m0 = __ballot_sync(0xffffffffu, valid && v < p.offset);
+        const unsigned sm = (m1 | m0) & le;
+        const int a = sm ? (int)((m1 >> last(sm)) & 1u) : h;
+        const unsigned A = __ballot_sync(0xffffffffu, a) & vm;
+        const unsigned shifted = (A << 1) | (unsigned)h;
+        const unsigned rise = A & ~shifted, fall = ~A & shifted & vm;
+        // last region end before / at or before t; the carried one counts only while its group is open (-1: none)
+        const int64_t pe_carry = status ? last_end : -1;
+        const int64_t pe_lt = (fall & lt) ? t0 + last(fall & lt) : pe_carry;
+        const int64_t pe_le = (fall & le) ? t0 + last(fall & le) : pe_carry;
+        const bool g = valid && ((rise >> lane) & 1u) && (pe_lt < 0 || t - pe_lt >= gap_break);
+        const bool c = valid && !a && pe_le >= 0 && t - pe_le + 1 == gap_break;
+        const unsigned G = __ballot_sync(0xffffffffu, g), C = __ballot_sync(0xffffffffu, c);
+        // the group open during frame t: the latest of a group start at or before t and a close before t decides
+        const unsigned gle = G & le, clt = C & lt;
+        const bool open = valid && (gle ? (!clt || last(gle) > last(clt)) : (!clt && status != 0));
+        const int64_t gst = gle ? t0 + last(gle) : gs;
+        const int64_t s = max(gst - (int64_t)p.pad_onset, (int64_t)0);
+        bool pass = false;
+        if (open) {
+            const int64_t ge = a ? t + 1 : pe_le;
+            pass = min(t + 1, ge + (int64_t)p.pad_offset) - s >= (int64_t)p.min_on;
+        }
+        const unsigned P = __ballot_sync(0xffffffffu, pass);
+        const bool passed_before = lane ? ((P >> (lane - 1)) & 1u) : status == 2;
+        const bool start = pass && (g || !passed_before);
+        const bool end = c && pass;
+        const unsigned E = __ballot_sync(0xffffffffu, start || end);
+        if (start || end) {
+            const int64_t o = n + __popc(E & lt);
+            if (o < cap) {
+                out[2 * o] = start ? s : pe_le + p.pad_offset;
+                out[2 * o + 1] = start;
+            }
+        }
+        n += __popc(E);
+        const int L = nv - 1;           // the state after the word is the one after its last frame
+        h = __shfl_sync(0xffffffffu, a, L);
+        last_end = __shfl_sync(0xffffffffu, pe_le, L);
+        gs = __shfl_sync(0xffffffffu, gst, L);
+        status = __shfl_sync(0xffffffffu, open && !c ? (pass ? 2 : 1) : 0, L);
+    }
+    if (lane != 0) return;
+    if (flush && flush[r]) {
+        // end of stream: only a group whose start was emitted survives (the start test at the last frame is the survival test)
+        if (status == 2) {
+            const int64_t T = len + nf;
+            const int64_t e = min(T, (h ? T : last_end) + (int64_t)p.pad_offset);
+            if (n < cap) { out[2 * n] = e; out[2 * n + 1] = 0; }
+            ++n;
+        }
+        st[0] = st[1] = st[2] = st[3] = st[4] = 0;
+    } else {
+        st[0] = h; st[1] = last_end; st[2] = gs; st[3] = status; st[4] = len + nf;
+    }
+    ev_counts[r] = (int32_t)n;
+}
+
+int regions_step_launch(const float* prob, int S, int nf, int64_t row_stride, const b200vad_binarize_params& p, int64_t* state,
+                        const uint8_t* flush, int64_t* ev, int32_t* ev_counts, int64_t cap, cudaStream_t stream) {
+    if (S == 0) return B200VAD_OK;
+    regions_step_kernel<<<(S + kEvWarps - 1) / kEvWarps, 32 * kEvWarps, 0, stream>>>(prob, S, nf, row_stride, p, state, flush, ev,
+                                                                                     ev_counts, cap);
+    B200VAD_LAUNCH_CHECK();
+    return B200VAD_OK;
+}
+
 }  // namespace b200vad
