@@ -163,6 +163,11 @@ B200VAD_API int b200vad_sincnet_forward_f32(const void* packed, const float* wav
 B200VAD_API int b200vad_median_window(double speech_window, double window);
 B200VAD_API int b200vad_threshold_median(const float* prob, int B, int64_t T, float thr, int kernel, void* out, int elem_bytes,
                              int32_t* near_count, float near_tol, void* stream);
+/* The same filter on R ragged streams of a flat buffer: stream r = prob[offsets[r], offsets[r+1]) (offsets: (R+1) i64 device),
+ * zero padded at its own edges, decisions written as u8 to the same offsets of out.  max_len >= every stream's length (it sizes
+ * the grid).  R <= 65535 per call; equals b200vad_threshold_median on each stream taken as one row. */
+B200VAD_API int b200vad_threshold_median_streams(const float* prob, const int64_t* offsets, int R, int64_t max_len, float thr, int kernel,
+                                     uint8_t* out, void* stream);
 
 /* ---- a8/a9: run-length segment extraction (src/scripts/predict.py:447-458, 472-490).
  * dec: flat uint8 decisions; stream r = dec[offsets[r], offsets[r+1]) (offsets: (R+1) i64,
@@ -255,6 +260,14 @@ B200VAD_API int b200vad_synth_corpus(float* wav, int64_t first_utt, int rows, in
  * starting at global frame w * hop_frames -> out (L) f32, every frame taken from the window whose centre is nearest. */
 B200VAD_API int b200vad_stitch_center(const float* prob, int num_windows, int frames_per_window, int hop_frames, float* out, int64_t L,
                           void* stream);
+/* The same stitching for R recordings at once: recording r has the windows [win_off[r], win_off[r+1]) of prob
+ * (W_total, frames_per_window) and its stream is out[frame_off[r], frame_off[r+1]) (win_off, frame_off: (R+1) i64 device);
+ * frames no window covers, and every frame of a recording without windows, are 0.  max_len >= every stream's length (it sizes
+ * the grid).  elem_bytes: 4 (f32 probabilities) or 1 (u8 decisions).  With hop_frames = frames_per_window this is the
+ * reference's "concatenate the windows, keep the first n frames" slice (src/scripts/predict.py:447-458) taken per recording.
+ * R <= 65535 per call; recording r equals b200vad_stitch_center on its own windows. */
+B200VAD_API int b200vad_stitch_center_streams(const void* prob, int elem_bytes, const int64_t* win_off, const int64_t* frame_off, int R,
+                                  int frames_per_window, int hop_frames, int64_t max_len, void* out, void* stream);
 
 /* ---- whole path on device buffers: fbank -> PyanNet2 -> threshold/median -> segments */
 B200VAD_API size_t b200vad_pipeline_workspace_bytes(int B, int64_t N);
@@ -295,6 +308,22 @@ B200VAD_API int b200vad_pipeline_binarize(const void* packed_model, const void* 
                               int wav_i16, const int32_t* lens, int B, int64_t N, int64_t wav_stride,
                               const b200vad_binarize_params* params, float* prob, uint8_t* dec, int32_t* counts, int64_t* seg_off,
                               int32_t* seg, int64_t cap, void* workspace, size_t ws_bytes, void* stream);
+
+/* ---- whole path on rows addressed through a table: windows of many recordings in one launch.  rows: (B) device array of
+ * device pointers (f32, or int16 PCM with wav_i16 != 0), row b starting at rows[b]; lens: (B) i32 device, the valid samples
+ * of each row (required).  A row never reads at or past lens[b], so rows may be separate allocations or views that end where
+ * the next recording's samples begin.  N is the window length every row is processed at:
+ *   fbank   (packed_sincnet = NULL): features past the row's frames are LOG_EPS, as lens means for b200vad_pipeline_fbank_*;
+ *   SincNet (packed_sincnet given, N >= 991): samples at index >= lens[b] are read as 0, the reference's zero-padded tail
+ *           window, which its InstanceNorm sees.  Adding 0 changes no partial sum, so prob equals that of the row copied into
+ *           a zero-padded buffer, bit for bit.
+ * params = NULL: threshold / median / segments as b200vad_pipeline_fbank_* / b200vad_pipeline_sincnet_*; else binarization
+ * as b200vad_pipeline_binarize.  Outputs, cap and workspace (b200vad_pipeline_workspace_bytes /
+ * b200vad_pipeline_sincnet_workspace_bytes at (B, N)) as those entries; B <= 65535. */
+B200VAD_API int b200vad_pipeline_rows(const void* packed_model, const void* packed_sincnet, int num_layers, const void* const* rows,
+                          int wav_i16, const int32_t* lens, int B, int64_t N, float thr, int kernel,
+                          const b200vad_binarize_params* params, float* prob, uint8_t* dec, int32_t* counts, int64_t* seg_off,
+                          int32_t* seg, int64_t cap, void* workspace, size_t ws_bytes, void* stream);
 
 /* ---- host-buffer session:the same path with HOST waveforms and HOST results -- what a caller holding
  * lhotse/DataLoader batches in host memory uses (src/engines/vad_engine.py:204-211 fed by

@@ -68,6 +68,7 @@ PROTOTYPES = {
     "b200vad_sincnet_forward_f32": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
     "b200vad_median_window": (c_int, [c_double, c_double]),
     "b200vad_threshold_median": (c_int, [c_void_p, c_int, c_int64, c_float, c_int, c_void_p, c_int, c_void_p, c_float, c_void_p]),
+    "b200vad_threshold_median_streams": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_float, c_int, c_void_p, c_void_p]),
     "b200vad_segments": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
     "b200vad_binarize": (c_int, [c_void_p, c_void_p, c_int, c_int64, _P_BIN, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
     "b200vad_pipeline_binarize": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int64, c_int64, _P_BIN,
@@ -84,6 +85,7 @@ PROTOTYPES = {
                                         c_void_p, c_void_p, c_void_p]),
     "b200vad_synth_corpus": (c_int, [c_void_p, c_int64, c_int, c_int64, C.c_uint64, c_void_p]),
     "b200vad_stitch_center": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int64, c_void_p]),
+    "b200vad_stitch_center_streams": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_void_p, c_void_p]),
     "b200vad_stream_create": (c_int, [c_int, c_void_p, c_int, c_int, c_int64, c_int, c_int, C.POINTER(c_void_p)]),
     "b200vad_stream_push": (c_int, [c_void_p, c_void_p, c_int, c_float, c_int, c_void_p, c_void_p, C.POINTER(c_float)]),
     "b200vad_stream_snapshot": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
@@ -98,6 +100,8 @@ PROTOTYPES = {
                                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
     "b200vad_pipeline_sincnet_i16": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int64, c_int64, c_float, c_int,
                                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
+    "b200vad_pipeline_rows": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int64, c_float, c_int, _P_BIN,
+                                      c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
     "b200vad_session_create_sincnet": (c_int, [c_int, c_void_p, c_void_p, c_int, c_int, c_int64, C.POINTER(c_void_p)]),
     "b200vad_stream_create_sincnet": (c_int, [c_int, c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_int, C.POINTER(c_void_p)]),
     "b200vad_session_submit_host_i16": (c_int, [c_void_p, c_int, c_void_p, c_int, c_float, c_int, c_void_p, c_void_p]),

@@ -8,10 +8,20 @@ run-length encoded (predict.py:472-490).
 
 Extension (hop < window): overlapping windows; probabilities are stitched by taking every frame from the window
 whose centre is nearest (``b200vad_stitch_center``), then threshold + median + segments run once over the stitched
-stream.  Windows are rows of an ``as_strided`` view of the waveform: nothing is copied.
+stream.
+
+Many recordings at once: ``LongFormVad(...)([wav, ...], durations)`` returns, for each recording, exactly what the call on
+that recording alone returns.  The windows of all recordings are rows of one pointer table (``vad_pipeline_rows``), read in
+place -- nothing is copied, a ragged last window included -- and packed into launches of ``max_rows`` rows, so a recording may
+straddle two launches.  Stitching (or, for hop == window, the per-recording slice of the concatenated windows), smoothing,
+segments and binarization then each run once over all recordings through stream offsets, and the host reads the segment
+triples once.  Each recording's stream is cut from its own windows (``recording_offsets([d], frames of its windows)``), as the
+single call does -- not by the consecutive slicing of one flat stream that ``get_segments(durations=...)`` keeps for parity
+with predict.py:447-458, which shifts every later recording once a tail window has been dropped.  The single-tensor call is
+the one-recording case of the same code.
 
 SincNet -> PyanNet (``sincnet_packed``), as predict_sincnet.get_new_cuts does it: the same 5 s windows, but the tail window
-is zero padded in AUDIO (the SincNet InstanceNorm sees the zeros; no lens), per-window median filter, concatenation, a slice
+is zero padded in AUDIO (samples past the recording read as 0; the SincNet InstanceNorm sees the zeros), per-window median filter, concatenation, a slice
 of ``ceil(get_num_frames(16000 d)) + 1`` frames per recording (predict_sincnet.py:330-337), run-length encoding that keeps
 single-frame runs and whole-second timestamps (predict_sincnet.py:348-370, 492-504).  Overlapped windows need a hop of whole
 SincNet frame steps (270 samples) so that every window's frames fall on one global grid.
@@ -24,12 +34,13 @@ decision stream covers -- so a region that crosses a window boundary stays one r
 
 from __future__ import annotations
 
-from typing import Optional
+from typing import List, Optional, Sequence, Union
 
+import numpy as np
 import torch
 
 from .binarize import mode_step
-from .host import (cut_into_windows, fbank_num_frames, get_num_frames, merge_intervals_with_buffer, recording_offsets,
+from .host import (fbank_num_frames, get_num_frames, merge_intervals_with_buffer, recording_offsets,
                    segments_to_intervals)
 
 SINC_STEP = 270       # samples between SincNet frames
@@ -51,74 +62,134 @@ class LongFormVad:
         self.thr, self.kernel, self.max_rows, self.fs = thr, kernel, max_rows, frame_shift
 
     # ---- window bookkeeping
+    def _window_arrays(self, num_samples: int):
+        """windows() as two int64 arrays (start_sample, valid_samples): hop == window is cut_into_windows (windows of at most
+        3 / 5 of a window dropped); otherwise windows every hop samples until one reaches the end, at least one."""
+        n = int(num_samples)
+        if self.hop == self.window:
+            s = np.arange(0, n, self.window, dtype=np.int64)
+            v = np.minimum(self.window, n - s)
+            keep = v > self.window * 3 // 5
+            return s[keep], v[keep]
+        s = np.arange(1 + max(0, -(-(n - self.window) // self.hop)), dtype=np.int64) * self.hop
+        return s, np.minimum(self.window, n - s)
+
     def windows(self, num_samples: int):
         """[(start_sample, valid_samples)] of the rows the recording is cut into."""
-        if self.hop == self.window:
-            return cut_into_windows(num_samples, self.window, min_keep=self.window * 3 // 5)
-        out, s = [], 0
-        while True:
-            n = min(self.window, num_samples - s)
-            out.append((s, n))
-            if s + self.window >= num_samples:
-                break
-            s += self.hop
-        return out
+        s, v = self._window_arrays(num_samples)
+        return list(zip(s.tolist(), v.tolist()))
 
-    def _rows(self, wav: torch.Tensor, wins):
-        """(rows, window) view of wav (row stride = hop) + per-row valid lengths; only the ragged tail is copied."""
-        N = wav.numel()
-        full = [w for w in wins if w[1] == self.window]
-        rows = torch.as_strided(wav, (len(full), self.window), (self.hop, 1)) if full else wav.new_empty((0, self.window))
-        lens = torch.full((len(wins),), self.window, dtype=torch.int32, device=wav.device)
-        if len(full) != len(wins):                      # last window is short: pad it into its own row
-            s, n = wins[-1]
-            tail = wav.new_zeros((1, self.window))
-            tail[0, :n] = wav[s:s + n]
-            lens[-1] = n
-            return rows, tail, lens
-        return rows, None, lens
+    @staticmethod
+    def _check(wav, what: str) -> None:
+        if not isinstance(wav, torch.Tensor) or wav.dim() != 1 or not wav.is_cuda or wav.dtype not in (torch.float32, torch.int16) \
+                or not wav.is_contiguous():
+            raise ValueError(f"{what} must be a contiguous 1-D float32 or int16 CUDA tensor")
 
     @torch.no_grad()
-    def __call__(self, wav: torch.Tensor, duration: Optional[float] = None):
-        """wav: (num_samples,) float32 CUDA tensor.  Returns dict(prob (W, Tw), stream_dec (L,) uint8, intervals)."""
-        if wav.dim() != 1 or not wav.is_cuda or wav.dtype != torch.float32 or not wav.is_contiguous():
-            raise ValueError("wav must be a contiguous 1-D float32 CUDA tensor")
-        N = wav.numel()
-        duration = N / 16000.0 if duration is None else duration
-        wins = self.windows(N)
-        rows, tail, lens = self._rows(wav, wins)
+    def __call__(self, wav: Union[torch.Tensor, Sequence[torch.Tensor]], duration=None, *, durations=None):
+        """wav: (num_samples,) float32 or int16 (16-bit PCM, read as int16 / 32768) CUDA tensor, duration in seconds (default
+        num_samples / 16000).  Returns dict(prob (W, Tw), stream_dec (L,) uint8, intervals, windows).
+
+        wav may also be a list of such recordings, all on one device and of one dtype, with ``durations`` None or a list of
+        seconds (also accepted in the second position); then the result is one such dict per recording, in input order, each
+        equal to the single call's on that recording.  Every recording is checked (ValueError naming its index) before any
+        device work."""
+        if isinstance(wav, torch.Tensor):
+            if durations is not None:
+                raise ValueError("durations= is for a list of recordings; pass duration= with a single tensor")
+            self._check(wav, "wav")
+            return self._run([wav], [duration])[0]
+        if duration is not None and durations is not None:
+            raise ValueError("pass the durations of a list of recordings once, as durations=")
+        durations = duration if durations is None else durations
+        wavs = list(wav)
+        durations = [None] * len(wavs) if durations is None else list(durations)
+        if len(durations) != len(wavs):
+            raise ValueError(f"{len(wavs)} recordings but {len(durations)} durations")
+        for i, w in enumerate(wavs):
+            self._check(w, f"wavs[{i}]")
+            if w.device != wavs[0].device or w.dtype != wavs[0].dtype:
+                raise ValueError(f"wavs[{i}] is {w.dtype} on {w.device}, wavs[0] is {wavs[0].dtype} on {wavs[0].device}: "
+                                 "one call takes recordings of one dtype on one device")
+        return self._run(wavs, durations)
+
+    def _window_outputs(self, wavs: List[torch.Tensor], rows: torch.Tensor, W: int, Tw: int):
+        """prob (W, Tw) f32 and per-window decisions dec (W, Tw) u8 of every window row, in launches of max_rows rows."""
+        per = min(self.max_rows, 65535)
+        probs, decs = [], []
+        for b0 in range(0, W, per):
+            p, d, _, _, _ = torch.ops.b200vad.vad_pipeline_rows(wavs, rows[b0:b0 + per], self.window, self.packed, self.sinc,
+                                                                self.L, self.thr, self.kernel)
+            probs.append(p); decs.append(d)
+        if not probs:
+            dev = wavs[0].device
+            return torch.empty((0, Tw), dtype=torch.float32, device=dev), torch.empty((0, Tw), dtype=torch.uint8, device=dev)
+        if len(probs) == 1:
+            return probs[0], decs[0]
+        return torch.cat(probs), torch.cat(decs)
+
+    def plan(self, num_samples: Sequence[int], durations: Sequence[float]):
+        """Host bookkeeping of a call on recordings of num_samples samples and durations seconds: (wins, rows, win_off,
+        frame_off, hop_frames) = each recording's windows(), the (W, 3) int64 host row table of (recording, start, valid) of all
+        windows in order, the (R + 1) offsets of each recording's windows among the rows and of its stream among the stream
+        frames, and the hop in frames at which the streams are cut from the windows (Tw for hop == window)."""
         sinc = self.sinc is not None
         Tw = get_num_frames(self.window) if sinc else fbank_num_frames(self.window)
-
-        def run(r, lens):
-            if sinc:            # the tail row is zero padded audio: no lens
-                return torch.ops.b200vad.vad_pipeline_sincnet(r, self.packed, self.sinc, self.L, self.thr, self.kernel)
-            return torch.ops.b200vad.vad_pipeline(r, lens, self.packed, self.L, self.thr, self.kernel)
-
-        probs, decs = [], []
-        for b0 in range(0, rows.shape[0], self.max_rows):
-            p, d, _, _ = run(rows[b0:b0 + self.max_rows], None)
-            probs.append(p); decs.append(d)
-        if tail is not None:
-            p, d, _, _ = run(tail, lens[-1:])
-            probs.append(p); decs.append(d)
-        prob = torch.cat(probs) if probs else wav.new_empty((0, Tw))
-        if self.binarize is not None:
-            return self._binarized(prob, N, duration, wins)
-        min_run = 1 if sinc else 2      # the SincNet RLE keeps single-frame runs (predict_sincnet.py:348-370)
+        arrays = [self._window_arrays(n) for n in num_samples]
+        wins = [list(zip(s.tolist(), v.tolist())) for s, v in arrays]
+        rows = torch.from_numpy(np.stack([np.repeat(np.arange(len(arrays), dtype=np.int64), [len(s) for s, _ in arrays]),
+                                          np.concatenate([s for s, _ in arrays]), np.concatenate([v for _, v in arrays])], axis=1))
         if self.hop == self.window:
-            # reference semantics: per-window median filter, concatenation, per-recording slice, RLE
-            dec = torch.cat(decs).reshape(-1) if decs else torch.empty(0, dtype=torch.uint8, device=wav.device)
-            offs = recording_offsets([duration], dec.numel(), self.fs, sincnet=sinc)
-            seg, _ = torch.ops.b200vad.segments(dec, torch.tensor(offs, dtype=torch.int64, device=wav.device), min_run)
-            stream = dec[: offs[1]]
+            # reference semantics: the recording's windows concatenated, cut to ceil(d / fs) + 1 frames (predict.py:447-458)
+            lens = [recording_offsets([d], len(w) * Tw, self.fs, sincnet=sinc)[1] for d, w in zip(durations, wins)]
+            hop_frames = Tw
         else:
-            L = get_num_frames(N) if sinc else fbank_num_frames(N)       # frames of the whole recording
-            sp = torch.ops.b200vad.stitch_center(prob, self.hop // (SINC_STEP if sinc else 160), L)
-            stream = torch.ops.b200vad.threshold_median(sp.view(1, -1), self.thr, self.kernel, False).view(-1)
-            seg, _ = torch.ops.b200vad.segments(stream.view(1, -1), None, min_run)
-        ivs = segments_to_intervals(seg.tolist(), 1, self.fs, sincnet_durations=[duration] if sinc else None)[0]
-        return {"prob": prob, "stream_dec": stream, "intervals": merge_intervals_with_buffer(ivs, duration, 0), "windows": wins}
+            lens = [get_num_frames(n) if sinc else fbank_num_frames(n) for n in num_samples]      # frames of the whole recording
+            hop_frames = self.hop // (SINC_STEP if sinc else 160)
+        win_off, frame_off = [0], [0]
+        for w, n in zip(wins, lens):
+            win_off.append(win_off[-1] + len(w))
+            frame_off.append(frame_off[-1] + n)
+        return wins, rows, win_off, frame_off, hop_frames
+
+    def _run(self, wavs: List[torch.Tensor], durations) -> List[dict]:
+        if not wavs:
+            return []
+        sinc = self.sinc is not None
+        dev = wavs[0].device
+        R = len(wavs)
+        Ns = [w.numel() for w in wavs]
+        durations = [n / 16000.0 if d is None else d for n, d in zip(Ns, durations)]
+        Tw = get_num_frames(self.window) if sinc else fbank_num_frames(self.window)
+        wins, rows, win_off, frame_off, hop_frames = self.plan(Ns, durations)
+        prob, dec = self._window_outputs(wavs, rows, win_off[-1], Tw)
+        # pinned and non-blocking: segments / binarize queue behind the pipeline instead of the host waiting for it here
+        offsets = torch.tensor(frame_off, dtype=torch.int64).pin_memory().to(dev, non_blocking=True)
+        if self.binarize is not None:
+            step, t0 = mode_step(sinc, self.fs)
+            f = self.binarize.frames(step)
+            sp = torch.ops.b200vad.stitch_center_streams(prob, win_off, frame_off, hop_frames)
+            if sp.numel() == 0:
+                stream, ivs = torch.empty(0, dtype=torch.uint8, device=dev), [[] for _ in range(R)]
+            else:
+                stream, seg, _ = torch.ops.b200vad.binarize(sp, offsets, f["onset"], f["offset"], f["pad_onset"], f["pad_offset"],
+                                                            f["min_off"], f["min_on"])
+                ivs = self.binarize.intervals(seg.tolist(), R, step, t0, durations)
+        else:
+            min_run = 1 if sinc else 2      # the SincNet RLE keeps single-frame runs (predict_sincnet.py:348-370)
+            if self.hop == self.window:     # per-window median filter, then the per-recording slice
+                stream = torch.ops.b200vad.stitch_center_streams(dec, win_off, frame_off, hop_frames)
+            else:                           # one median filter over each recording's stitched stream
+                sp = torch.ops.b200vad.stitch_center_streams(prob, win_off, frame_off, hop_frames)
+                stream = torch.ops.b200vad.threshold_median_streams(sp, frame_off, self.thr, self.kernel)
+            if stream.numel() == 0:
+                ivs = [[] for _ in range(R)]
+            else:
+                seg, _ = torch.ops.b200vad.segments(stream, offsets, min_run)
+                ivs = segments_to_intervals(seg.tolist(), R, self.fs, sincnet_durations=durations if sinc else None)
+            ivs = [merge_intervals_with_buffer(iv, d, 0) for iv, d in zip(ivs, durations)]
+        return [{"prob": prob[win_off[r]:win_off[r + 1]], "stream_dec": stream[frame_off[r]:frame_off[r + 1]], "intervals": ivs[r],
+                 "windows": wins[r]} for r in range(R)]
 
     def probability_stream(self, prob: torch.Tensor, num_samples: int, duration: float) -> torch.Tensor:
         """The recording's probability stream that binarization runs over: the stitched stream for hop < window, else the
@@ -129,12 +200,3 @@ class LongFormVad:
             return flat[: recording_offsets([duration], flat.numel(), self.fs, sincnet=sinc)[1]]
         L = get_num_frames(num_samples) if sinc else fbank_num_frames(num_samples)
         return torch.ops.b200vad.stitch_center(prob, self.hop // (SINC_STEP if sinc else 160), L)
-
-    def _binarized(self, prob, num_samples, duration, wins):
-        step, t0 = mode_step(self.sinc is not None, self.fs)
-        f = self.binarize.frames(step)
-        sp = self.probability_stream(prob, num_samples, duration)
-        dec, seg, _ = torch.ops.b200vad.binarize(sp.view(1, -1), None, f["onset"], f["offset"], f["pad_onset"], f["pad_offset"],
-                                                 f["min_off"], f["min_on"])
-        ivs = self.binarize.intervals(seg.tolist(), 1, step, t0, [duration])[0]
-        return {"prob": prob, "stream_dec": dec.view(-1), "intervals": ivs, "windows": wins}

@@ -12,6 +12,10 @@
                                                     -> prob, dec, seg, counts
   b200vad::regions_step(prob, state, onset, offset, pad_onset, pad_offset, min_off, min_on, flush?)
                                                     -> ev (S, nf + 1, 2) i64, counts (S,) i32; mutates state
+  b200vad::vad_pipeline_rows(wavs, rows (B, 3) host i64, window, packed, packed_sincnet?, L, thr, kernel, binarize?)
+                                                    -> prob, dec, seg (padded), counts, seg_off
+  b200vad::stitch_center_streams(prob, win_off, frame_off, hop_frames) -> (frame_off[-1],) f32 | u8
+  b200vad::threshold_median_streams(prob, offsets, thr, kernel)       -> (n,) u8
 
 Each op enqueues on ``torch.cuda.current_stream()`` and never synchronises, except
 ``segments`` / ``binarize`` and the exact-size ``vad_pipeline*`` ops, which read one int64 (the segment total) to size
@@ -20,8 +24,9 @@ their output.
 
 from __future__ import annotations
 
-from typing import Optional, Tuple
+from typing import List, Optional, Tuple
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -349,11 +354,8 @@ def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc=None, bin=
         if lens is not None:
             lens = _prep(lens.to(torch.int32), torch.int32, "lens")
             lens_ptr = lens.data_ptr()
+        ws = _pipeline_ws(B, N, T, sinc is not None, dev)
         if sinc is None:
-            need = L.b200vad_pipeline_workspace_bytes(B, N)
-            minimum = L.b200vad_pipeline_workspace_bytes(B, N) - L.b200vad_model_workspace_bytes(B, T) + \
-                L.b200vad_model_workspace_bytes(1, T)
-            ws = _ws(min(need, max(_MAX_WS_BYTES, minimum)), dev)
             if bin is not None:
                 _lib.check(L.b200vad_pipeline_binarize(packed.data_ptr(), None, num_layers, wav.data_ptr(), int(wav.dtype == torch.int16),
                                                        lens_ptr, B, N, wav.stride(0), bin, prob.data_ptr(), dec.data_ptr(),
@@ -368,9 +370,6 @@ def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc=None, bin=
         else:
             if lens is not None:
                 raise _lib.B200VadError("the SincNet path takes no lens: pad rows with zero audio, as the reference does")
-            need = L.b200vad_pipeline_sincnet_workspace_bytes(B, N)
-            minimum = 256 * B * T + L.b200vad_pipeline_sincnet_workspace_bytes(1, N)    # + the whole batch's layer-0 planes
-            ws = _ws(min(need, max(_MAX_WS_BYTES, minimum)), dev)
             if bin is not None:
                 _lib.check(L.b200vad_pipeline_binarize(packed.data_ptr(), sinc.data_ptr(), num_layers, wav.data_ptr(),
                                                        int(wav.dtype == torch.int16), None, B, N, wav.stride(0), bin, prob.data_ptr(),
@@ -386,6 +385,97 @@ def _pipeline_launch(wav, lens, packed, num_layers, thr, kernel, sinc=None, bin=
 
 
 _MAX_PIPELINE_ROWS = 65535        # grid limit of the per-row kernels behind one C call
+
+
+def _pipeline_ws(B: int, N: int, T: int, sincnet: bool, dev) -> torch.Tensor:
+    """Workspace of one pipeline launch of B rows of N samples (T frames), capped at _MAX_WS_BYTES unless the launch needs more."""
+    L = _lib.lib()
+    if not sincnet:
+        need = L.b200vad_pipeline_workspace_bytes(B, N)
+        minimum = need - L.b200vad_model_workspace_bytes(B, T) + L.b200vad_model_workspace_bytes(1, T)
+    else:
+        need = L.b200vad_pipeline_sincnet_workspace_bytes(B, N)
+        minimum = 256 * B * T + L.b200vad_pipeline_sincnet_workspace_bytes(1, N)    # + the whole batch's layer-0 planes
+    return _ws(min(need, max(_MAX_WS_BYTES, minimum)), dev)
+
+
+def _upload(values, dtype, dev) -> torch.Tensor:
+    """Host list or array -> device tensor through pinned memory: enqueued on the current stream, no synchronisation."""
+    return torch.as_tensor(np.asarray(values)).to(dtype).pin_memory().to(dev, non_blocking=True)
+
+
+# ------------------------------------------------------------------ windows of many recordings: rows through a pointer table
+@torch.library.custom_op("b200vad::vad_pipeline_rows", mutates_args=(), device_types="cuda")
+def vad_pipeline_rows(wavs: List[torch.Tensor], rows: torch.Tensor, window: int, packed: torch.Tensor,
+                      packed_sincnet: Optional[torch.Tensor], num_layers: int, thr: float, kernel: int,
+                      binarize: Optional[List[float]] = None
+                      ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """The whole path on B rows of ``window`` samples cut from several recordings (b200vad_pipeline_rows): ``rows`` is a (B, 3)
+    int64 host tensor of (recording, start, valid), and row b reads wavs[recording][start : start + valid] only, in place.
+    wavs: contiguous 1-D CUDA tensors on one device, all float32 or all int16 PCM.  fbank (packed_sincnet None): features past
+    the valid frames are LOG_EPS, as lens means for vad_pipeline; SincNet: samples past the valid ones are zeros.
+    ``binarize``: [onset, offset, pad_onset, pad_offset, min_off, min_on] -> binarization instead of threshold / median.
+    Returns what vad_pipeline_padded does -- prob (B, T), dec (B, T), seg at its fixed capacity, counts (B,), seg_off (B + 1,)
+    -- without any host synchronisation; the recordings must stay alive until the work on the current stream is done."""
+    if not wavs:
+        raise _lib.B200VadError("wavs is empty")
+    dev, dtype = wavs[0].device, wavs[0].dtype
+    if dtype not in (torch.float32, torch.int16):
+        raise _lib.B200VadError(f"wavs must be torch.float32 or torch.int16 (16-bit PCM), got {dtype}")
+    for i, w in enumerate(wavs):
+        if not w.is_cuda or w.device != dev or w.dtype != dtype or w.dim() != 1 or not w.is_contiguous():
+            raise _lib.B200VadError(f"wavs[{i}] must be a contiguous 1-D {dtype} tensor on {dev}")
+    if rows.device.type != "cpu" or rows.dim() != 2 or rows.shape[1] != 3:
+        raise _lib.B200VadError("rows must be a (B, 3) host tensor of (recording, start, valid)")
+    B, N = rows.shape[0], int(window)
+    L = _lib.lib()
+    sinc = packed_sincnet is not None
+    T = L.b200vad_sincnet_num_frames(N) if sinc else L.b200vad_fbank_num_frames(N)
+    if sinc and T < 1:
+        raise _lib.B200VadError("window shorter than the SincNet receptive field (991 samples)")
+    if B > _MAX_PIPELINE_ROWS:
+        raise _lib.B200VadError(f"one pipeline launch handles at most {_MAX_PIPELINE_ROWS} rows")
+    tab = rows.to(torch.int64).numpy()
+    rec, start, valid = tab[:, 0], tab[:, 1], tab[:, 2]
+    numel = np.asarray([w.numel() for w in wavs], dtype=np.int64)
+    ok = (rec >= 0) & (rec < len(wavs)) & (start >= 0) & (valid >= 0) & (valid <= N)
+    ok[ok] &= start[ok] + valid[ok] <= numel[rec[ok]]
+    if not ok.all():
+        b = int(np.flatnonzero(~ok)[0])
+        raise _lib.B200VadError(f"row {b}: {tuple(tab[b].tolist())} is not inside a recording or longer than the window")
+    # one upload: B row pointers, then the B int32 valid lengths packed two to an int64 word
+    base = np.asarray([w.data_ptr() for w in wavs], dtype=np.int64)
+    table = np.zeros(B + (B + 1) // 2, dtype=np.int64)
+    table[:B] = base[rec] + wavs[0].element_size() * start
+    table[B:].view(np.int32)[:B] = valid
+    prob = torch.empty((B, T), dtype=torch.float32, device=dev)
+    dec = torch.empty((B, T), dtype=torch.uint8, device=dev)
+    counts = torch.zeros(B, dtype=torch.int32, device=dev)
+    seg_off = torch.zeros(B + 1, dtype=torch.int64, device=dev)
+    if B == 0 or T == 0:
+        return prob, dec, torch.empty((0, 3), dtype=torch.int32, device=dev), counts, seg_off
+    bin = _bin_params(*binarize) if binarize is not None else None
+    cap = B * ((T + 1) // 2 if bin is not None else _seg_per_row(T, sinc))
+    seg = torch.empty((cap, 3), dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _ensure(dev)
+        table_d = _upload(table, torch.int64, dev)
+        ws = _pipeline_ws(B, N, T, sinc, dev)
+        _lib.check(L.b200vad_pipeline_rows(packed.data_ptr(), packed_sincnet.data_ptr() if sinc else None, num_layers, table_d.data_ptr(),
+                                           int(dtype == torch.int16), table_d.data_ptr() + 8 * B, B, N, float(thr), int(kernel), bin,
+                                           prob.data_ptr(), dec.data_ptr(), counts.data_ptr(), seg_off.data_ptr(), seg.data_ptr(), cap,
+                                           ws.data_ptr(), ws.numel(), _stream_ptr(dev)), "b200vad_pipeline_rows")
+    return prob, dec, seg, counts, seg_off
+
+
+@vad_pipeline_rows.register_fake
+def _(wavs, rows, window, packed, packed_sincnet, num_layers, thr, kernel, binarize=None):
+    B, N = rows.shape[0], int(window)
+    T = (N + 80) // 160 if packed_sincnet is None else _sincnet_frames(N)
+    cap = B * ((T + 1) // 2 if binarize is not None else _seg_per_row(T, packed_sincnet is not None))
+    w = wavs[0]
+    return (w.new_empty((B, T), dtype=torch.float32), w.new_empty((B, T), dtype=torch.uint8), w.new_empty((cap, 3), dtype=torch.int32),
+            w.new_empty((B,), dtype=torch.int32), w.new_empty((B + 1,), dtype=torch.int64))
 
 
 @torch.library.custom_op("b200vad::vad_pipeline_padded", mutates_args=(), device_types="cuda")
@@ -601,3 +691,78 @@ def stitch_center(prob: torch.Tensor, hop_frames: int, total_frames: int) -> tor
 @stitch_center.register_fake
 def _(prob, hop_frames, total_frames):
     return prob.new_empty((total_frames,))
+
+
+def _check_offsets(off: List[int], end: int, what: str) -> None:
+    if len(off) < 1 or off[0] != 0 or off[-1] != end or any(b < a for a, b in zip(off, off[1:])):
+        raise _lib.B200VadError(f"{what} must rise from 0 to {end}")
+
+
+_MAX_STREAMS = 65535              # grid limit of the ragged kernels behind one C call
+
+
+@torch.library.custom_op("b200vad::stitch_center_streams", mutates_args=(), device_types="cuda")
+def stitch_center_streams(prob: torch.Tensor, win_off: List[int], frame_off: List[int], hop_frames: int) -> torch.Tensor:
+    """stitch_center for R recordings at once (b200vad_stitch_center_streams): prob (W, Tw) float32 probabilities or uint8
+    decisions; recording r has the windows prob[win_off[r] : win_off[r + 1]] and its stitched stream is
+    out[frame_off[r] : frame_off[r + 1]] (host lists of R + 1 offsets from 0).  Frames no window covers are 0.  With
+    hop_frames = Tw each stream is its windows concatenated and cut to its length.  More than 65 535 recordings are split
+    across launches."""
+    if not prob.is_cuda or prob.dtype not in (torch.float32, torch.uint8) or prob.dim() != 2:
+        raise _lib.B200VadError("prob must be a (W, Tw) float32 or uint8 CUDA tensor")
+    prob = prob.contiguous()
+    W, Tw = prob.shape
+    R = len(win_off) - 1
+    if len(frame_off) != R + 1:
+        raise _lib.B200VadError("win_off and frame_off must both hold R + 1 offsets")
+    _check_offsets(win_off, W, "win_off")
+    _check_offsets(frame_off, frame_off[-1] if frame_off else 0, "frame_off")
+    dev = prob.device
+    out = torch.empty(frame_off[-1], dtype=prob.dtype, device=dev)
+    if out.numel() == 0:
+        return out
+    with torch.cuda.device(dev):
+        off = _upload(win_off + frame_off, torch.int64, dev)
+        wo, fo = off[:R + 1], off[R + 1:]
+        for r0 in range(0, R, _MAX_STREAMS):
+            r1 = min(R, r0 + _MAX_STREAMS)
+            max_len = max(b - a for a, b in zip(frame_off[r0:r1], frame_off[r0 + 1:r1 + 1]))
+            _lib.check(_lib.lib().b200vad_stitch_center_streams(prob.data_ptr(), prob.element_size(), wo[r0:].data_ptr(), fo[r0:].data_ptr(),
+                                                                r1 - r0, Tw, int(hop_frames), max_len, out.data_ptr(),
+                                                                _stream_ptr(dev)), "b200vad_stitch_center_streams")
+    return out
+
+
+@stitch_center_streams.register_fake
+def _(prob, win_off, frame_off, hop_frames):
+    return prob.new_empty((frame_off[-1],))
+
+
+@torch.library.custom_op("b200vad::threshold_median_streams", mutates_args=(), device_types="cuda")
+def threshold_median_streams(prob: torch.Tensor, offsets: List[int], thr: float, kernel: int) -> torch.Tensor:
+    """threshold_median on R ragged streams of a flat (n,) float32 buffer (b200vad_threshold_median_streams): stream r is
+    prob[offsets[r] : offsets[r + 1]] (host list of R + 1 offsets from 0 to n), zero padded at its own edges.  Returns (n,)
+    uint8.  More than 65 535 streams are split across launches."""
+    prob = _prep(prob, torch.float32, "prob")
+    if prob.dim() != 1:
+        raise _lib.B200VadError("prob must be a flat (n,) buffer")
+    _check_offsets(offsets, prob.numel(), "offsets")
+    dev = prob.device
+    out = torch.empty(prob.numel(), dtype=torch.uint8, device=dev)
+    if out.numel() == 0:
+        return out
+    R = len(offsets) - 1
+    with torch.cuda.device(dev):
+        off = _upload(offsets, torch.int64, dev)
+        for r0 in range(0, R, _MAX_STREAMS):
+            r1 = min(R, r0 + _MAX_STREAMS)
+            max_len = max(b - a for a, b in zip(offsets[r0:r1], offsets[r0 + 1:r1 + 1]))
+            _lib.check(_lib.lib().b200vad_threshold_median_streams(prob.data_ptr(), off[r0:].data_ptr(), r1 - r0, max_len, float(thr),
+                                                                   int(kernel), out.data_ptr(), _stream_ptr(dev)),
+                       "b200vad_threshold_median_streams")
+    return out
+
+
+@threshold_median_streams.register_fake
+def _(prob, offsets, thr, kernel):
+    return prob.new_empty(prob.shape, dtype=torch.uint8)

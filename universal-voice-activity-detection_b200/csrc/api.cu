@@ -651,16 +651,18 @@ size_t b200vad_sincnet_workspace_bytes(int B, int64_t N) {
 // (hi, lo) planes (B, Ts, 64) with channels 60..63 zero: the unscaled split of split_planes_pad_kernel, so model_forward sees
 // the same bits either way, without the fp32 round trip through HBM and the split pass.  Every chunk writes its own rows of
 // the whole-batch output.
+// rows != nullptr (tcgen05 path only): row b starts at rows[b] and has lens[b] valid samples, the rest read as 0 (wav is unused).
 static int sincnet_forward(const void* packed, const void* wav, int wav_i16, int B, int64_t N, int64_t wav_stride, float* out,
-                           __half* o_hi, __half* o_lo, void* workspace, size_t ws_bytes, cudaStream_t st) {
+                           __half* o_hi, __half* o_lo, void* workspace, size_t ws_bytes, cudaStream_t st,
+                           const void* const* rows = nullptr, const int32_t* lens = nullptr) {
     const bool planes = o_hi != nullptr;
-    B200VAD_CHECK_ARG(packed && wav && (out || (o_hi && o_lo)) && workspace, "null pointer");
+    B200VAD_CHECK_ARG(packed && (wav || (rows && lens)) && (out || (o_hi && o_lo)) && workspace, "null pointer");
     B200VAD_CHECK_ARG(B >= 0 && N >= 0 && wav_stride >= 1, "bad shape");
     B200VAD_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "workspace must be 256-byte aligned");
     const SincDims d = sinc_dims(N);
     B200VAD_CHECK_ARG(d.P3 >= 1, "waveform shorter than the SincNet receptive field (991 samples)");
-    if ((planes || wav_i16) && g_impl != 2) {
-        set_error("sincnet: int16 input and plane output need the tcgen05 path (b200vad_set_impl(2))");
+    if ((planes || wav_i16 || rows) && g_impl != 2) {
+        set_error("sincnet: int16 input, row tables and plane output need the tcgen05 path (b200vad_set_impl(2))");
         return B200VAD_ESTATE;
     }
     if (B == 0) return B200VAD_OK;
@@ -699,9 +701,10 @@ static int sincnet_forward(const void* packed, const void* wav, int wav_i16, int
             const int sms = num_sms_cached();
             __half* wn_hi = reinterpret_cast<__half*>(wn_raw);
             __half* wn_lo = wn_hi + 4 * (int64_t)bc * Np;
-            const void* wrow = reinterpret_cast<const char*>(wav) + (wav_i16 ? sizeof(int16_t) : sizeof(float)) * b0 * wav_stride;
+            const void* wrow = rows ? nullptr : reinterpret_cast<const char*>(wav) + (wav_i16 ? sizeof(int16_t) : sizeof(float)) * b0 * wav_stride;
             if ((rc = wave_norm_planes_launch(wrow, wav_i16, bc, N, wav_stride, Np, reinterpret_cast<const float*>(pk + s.wn_w),
-                                              reinterpret_cast<const float*>(pk + s.wn_b), stats, wn_hi, wn_lo, st, 0))) return rc;
+                                              reinterpret_cast<const float*>(pk + s.wn_b), stats, wn_hi, wn_lo, st, 0,
+                                              rows ? rows + b0 : nullptr, rows ? lens + b0 : nullptr))) return rc;
             if (sinc_fused()) {
                 // (three fp16 products per k-step: the 2-product scheme of the LSTM projections costs 3e-3 on the normalised SincNet
             // output -- three convolutions and InstanceNorms amplify it -- for 4 % of the front-end time; the kernels keep the option)
@@ -826,6 +829,14 @@ int b200vad_threshold_median(const float* prob, int B, int64_t T, float thr, int
     return threshold_median_launch(prob, B, T, thr, kernel, out, elem_bytes, near_count, near_tol, (cudaStream_t)stream);
 }
 
+int b200vad_threshold_median_streams(const float* prob, const int64_t* offsets, int R, int64_t max_len, float thr, int kernel,
+                                     uint8_t* out, void* stream) {
+    B200VAD_CHECK_ARG(R >= 0 && R <= 65535 && max_len >= 0, "need 0 <= R <= 65535 and max_len >= 0");
+    if (R == 0 || max_len == 0) return B200VAD_OK;
+    B200VAD_CHECK_ARG(prob && offsets && out, "null pointer");
+    return threshold_median_launch(prob, R, max_len, thr, kernel, out, 1, nullptr, 0.f, (cudaStream_t)stream, offsets);
+}
+
 // B200VAD_EINVAL unless the thresholds are finite with offset <= onset and every count is >= 0
 static int check_binarize(const b200vad_binarize_params* p) {
     B200VAD_CHECK_ARG(p, "null binarize params");
@@ -901,7 +912,19 @@ int b200vad_stitch_center(const float* prob, int num_windows, int frames_per_win
     B200VAD_CHECK_ARG(num_windows >= 1 && frames_per_window >= 1 && hop_frames >= 1 && hop_frames <= frames_per_window && L >= 0,
                       "need 1 <= hop_frames <= frames_per_window");
     B200VAD_CHECK_ARG(prob && (out || L == 0), "null pointer");
-    return stitch_center_launch(prob, num_windows, frames_per_window, hop_frames, out, L, (cudaStream_t)stream);
+    return stitch_center_launch(prob, nullptr, nullptr, 1, num_windows, frames_per_window, hop_frames, out, L, 4, (cudaStream_t)stream);
+}
+
+int b200vad_stitch_center_streams(const void* prob, int elem_bytes, const int64_t* win_off, const int64_t* frame_off, int R,
+                                  int frames_per_window, int hop_frames, int64_t max_len, void* out, void* stream) {
+    B200VAD_CHECK_ARG(elem_bytes == 1 || elem_bytes == 4, "elem_bytes must be 1 or 4");
+    B200VAD_CHECK_ARG(R >= 0 && R <= 65535 && max_len >= 0, "need 0 <= R <= 65535 and max_len >= 0");
+    B200VAD_CHECK_ARG(frames_per_window >= 1 && hop_frames >= 1 && hop_frames <= frames_per_window,
+                      "need 1 <= hop_frames <= frames_per_window");
+    if (R == 0 || max_len == 0) return B200VAD_OK;
+    B200VAD_CHECK_ARG(win_off && frame_off && out, "null pointer");
+    return stitch_center_launch(prob, win_off, frame_off, R, 0, frames_per_window, hop_frames, out, max_len, elem_bytes,
+                                (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------- fused device pipeline
@@ -928,11 +951,12 @@ size_t b200vad_pipeline_sincnet_workspace_bytes(int B, int64_t N) {
     return pipeline_ws_bytes(B, N, true);
 }
 
+// rows != nullptr: row b is read from rows[b] (lens required) instead of wav + b * stride
 static int pipeline_run(const void* packed, const void* sinc, int L, const void* wav, int wav_i16, const int32_t* lens, int B,
                         int64_t N, int64_t stride, float thr, int kernel, const b200vad_binarize_params* bin, int row_base, float* prob,
                         uint8_t* dec, int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, void* ws, size_t ws_bytes,
-                        cudaStream_t st) {
-    B200VAD_CHECK_ARG(packed && wav && prob && dec && counts && seg_off && ws, "null pointer");
+                        cudaStream_t st, const void* const* rows = nullptr) {
+    B200VAD_CHECK_ARG(packed && (wav || (rows && lens)) && prob && dec && counts && seg_off && ws, "null pointer");
     B200VAD_CHECK_ARG((reinterpret_cast<uintptr_t>(ws) & 255) == 0, "workspace must be 256-byte aligned");
     const int64_t T = fe_frames(sinc != nullptr, N);
     const int D = fe_dim(sinc != nullptr);
@@ -956,12 +980,12 @@ static int pipeline_run(const void* packed, const void* sinc, int L, const void*
             set_error("pipeline: the SincNet front end runs on the tcgen05 path only (b200vad_set_impl(2))");
             return B200VAD_ESTATE;
         }
-        rc = sincnet_forward(sinc, wav, wav_i16, B, N, stride, nullptr, f_hi, f_lo, w, ws_bytes - used, st);
+        rc = sincnet_forward(sinc, wav, wav_i16, B, N, stride, nullptr, f_hi, f_lo, w, ws_bytes - used, st, rows, lens);
     } else {
         int dev = 0;
         B200VAD_CUDA(cudaGetDevice(&dev));
         rc = fbank_launch(wav, wav_i16, lens, B, N, stride, planes ? nullptr : feats, planes ? f_hi : nullptr, planes ? f_lo : nullptr, T,
-                          sums, dev, st);
+                          sums, dev, st, rows);
     }
     if (rc) return rc;
     rc = model_forward(packed, D, L, planes ? nullptr : feats, f_hi, f_lo, B, T, prob, w, ws_bytes - used, st);
@@ -1023,6 +1047,22 @@ int b200vad_pipeline_binarize(const void* packed_model, const void* packed_sincn
     }
     return pipeline_run(packed_model, packed_sincnet, num_layers, wav, wav_i16 != 0, lens, B, N, wav_stride, 0.f, 0, params, 0, prob,
                         dec, counts, seg_off, seg, cap, ws, ws_bytes, (cudaStream_t)stream);
+}
+
+int b200vad_pipeline_rows(const void* packed_model, const void* packed_sincnet, int num_layers, const void* const* rows, int wav_i16,
+                          const int32_t* lens, int B, int64_t N, float thr, int kernel, const b200vad_binarize_params* params,
+                          float* prob, uint8_t* dec, int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, void* ws,
+                          size_t ws_bytes, void* stream) {
+    if (params) {
+        int rc = check_binarize(params);
+        if (rc) return rc;
+    }
+    B200VAD_CHECK_ARG(num_layers > 0 && B >= 0 && B <= 65535 && N >= 1 && cap >= 0, "bad shape");
+    B200VAD_CHECK_ARG(!packed_sincnet || N >= 991, "waveform shorter than the SincNet receptive field (991 samples)");
+    if (B == 0) return B200VAD_OK;
+    B200VAD_CHECK_ARG(rows && lens, "null pointer");
+    return pipeline_run(packed_model, packed_sincnet, num_layers, nullptr, wav_i16 != 0, lens, B, N, 1, thr, kernel, params, 0, prob, dec,
+                        counts, seg_off, seg, cap, ws, ws_bytes, (cudaStream_t)stream, rows);
 }
 
 // ---------------------------------------------------------------- host-buffer session

@@ -141,14 +141,22 @@ template <typename WT> __device__ __forceinline__ bool vec_aligned(const WT* p) 
     return (reinterpret_cast<uintptr_t>(p) & (4 * sizeof(WT) - 1)) == 0;
 }
 
+// Row b starts at rows[b] when a pointer table is given (windows of several recordings in one launch), else at
+// wav + b * stride.  Either way it reads only samples [0, min(lens[b], N)).
+template <typename WT>
+__device__ __forceinline__ const WT* row_ptr(const WT* wav, const WT* const* rows, int64_t stride, int b) {
+    return rows ? rows[b] : wav + (int64_t)b * stride;
+}
+
 // ---------------------------------------------------------------- row sums (DC offset)
 // grid (chunks, B): fp32 lane partials over <= 32 elements, then double.
 template <typename WT>
-__global__ void __launch_bounds__(256) row_sum_kernel(const WT* __restrict__ wav, const int32_t* __restrict__ lens,
-                                                      int64_t N, int64_t stride, double* __restrict__ sums) {
+__global__ void __launch_bounds__(256) row_sum_kernel(const WT* __restrict__ wav, const WT* const* __restrict__ rows,
+                                                      const int32_t* __restrict__ lens, int64_t N, int64_t stride,
+                                                      double* __restrict__ sums) {
     const int b = blockIdx.y;
     const int64_t n = lens ? min((int64_t)lens[b], N) : N;
-    const WT* row = wav + (int64_t)b * stride;
+    const WT* row = row_ptr(wav, rows, stride, b);
     const int64_t chunk = 256 * 32;
     int64_t begin = (int64_t)blockIdx.x * chunk;
     if (begin >= n) return;
@@ -249,7 +257,7 @@ __device__ __forceinline__ float preemph(float x, float xprev, float mean) {
 // fp32 feature round trip and the split kernel.
 template <bool PLANES, typename WT>
 __global__ void __launch_bounds__(kFbankThreads, 5)
-fbank_kernel(const WT* __restrict__ wav, const int32_t* __restrict__ lens, int64_t N, int64_t stride,
+fbank_kernel(const WT* __restrict__ wav, const WT* const* __restrict__ rows, const int32_t* __restrict__ lens, int64_t N, int64_t stride,
              const double* __restrict__ sums, const FbankTables* __restrict__ tab,
              float* __restrict__ feats, __half* __restrict__ feats_hi, __half* __restrict__ feats_lo, int64_t T_out) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -279,7 +287,7 @@ fbank_kernel(const WT* __restrict__ wav, const int32_t* __restrict__ lens, int64
         return;
     }
     const int nframes = (int)min((int64_t)kTileFrames, T - f0);
-    const WT* row = wav + (int64_t)b * stride;
+    const WT* row = row_ptr(wav, rows, stride, b);
     const float mean = (float)(sums[b] / (double)n);
     const int g = tid >> 4;         // group = frame slot
     const int j = tid & 15;         // lane within the group
@@ -298,6 +306,7 @@ fbank_kernel(const WT* __restrict__ wav, const int32_t* __restrict__ lens, int64
     // ---- stage the pre-emphasised span
     const int64_t start = f0 * kFrameShift - kPadLeft;               // original index of span[0]
     const int span = (nframes - 1) * kFrameShift + kFrameLen;
+    // interior: every sample read, [start - 1, start + span), lies in [0, n); anything else takes the mirrored path
     const bool interior = (start >= 4) && (start + span <= n) && vec_aligned(row);
     if (interior) {
         // start is a multiple of 8 samples -> aligned 4-sample vector loads
@@ -407,26 +416,27 @@ fbank_kernel(const WT* __restrict__ wav, const int32_t* __restrict__ lens, int64
 
 // exactly one of feats (fp32) / (feats_hi, feats_lo) (fp16 planes) is written; wav is fp32 or (wav_i16) 16-bit PCM
 template <typename WT>
-static int fbank_launch_t(const WT* wav, const int32_t* lens, int B, int64_t N, int64_t stride, float* feats, __half* feats_hi,
-                          __half* feats_lo, int64_t T_out, double* row_sums, const FbankTables* tab, cudaStream_t stream) {
+static int fbank_launch_t(const WT* wav, const WT* const* rows, const int32_t* lens, int B, int64_t N, int64_t stride, float* feats,
+                          __half* feats_hi, __half* feats_lo, int64_t T_out, double* row_sums, const FbankTables* tab,
+                          cudaStream_t stream) {
     int rc;
     if ((rc = set_max_dynamic_smem(reinterpret_cast<const void*>(fbank_kernel<false, WT>), (int)sizeof(FbankSmem)))) return rc;
     if ((rc = set_max_dynamic_smem(reinterpret_cast<const void*>(fbank_kernel<true, WT>), (int)sizeof(FbankSmem)))) return rc;
     if ((rc = zero_f64_launch(row_sums, B, stream))) return rc;
     dim3 g1((unsigned)((N + 256 * 32 - 1) / (256 * 32)), B);
-    row_sum_kernel<WT><<<g1, 256, 0, stream>>>(wav, lens, N, stride, row_sums);
+    row_sum_kernel<WT><<<g1, 256, 0, stream>>>(wav, rows, lens, N, stride, row_sums);
     B200VAD_LAUNCH_CHECK();
     dim3 g2((unsigned)((T_out + kTileFrames - 1) / kTileFrames), B);
     prof_begin(3, stream);
-    if (feats_hi) fbank_kernel<true, WT><<<g2, kFbankThreads, sizeof(FbankSmem), stream>>>(wav, lens, N, stride, row_sums, tab, nullptr, feats_hi, feats_lo, T_out);
-    else fbank_kernel<false, WT><<<g2, kFbankThreads, sizeof(FbankSmem), stream>>>(wav, lens, N, stride, row_sums, tab, feats, nullptr, nullptr, T_out);
+    if (feats_hi) fbank_kernel<true, WT><<<g2, kFbankThreads, sizeof(FbankSmem), stream>>>(wav, rows, lens, N, stride, row_sums, tab, nullptr, feats_hi, feats_lo, T_out);
+    else fbank_kernel<false, WT><<<g2, kFbankThreads, sizeof(FbankSmem), stream>>>(wav, rows, lens, N, stride, row_sums, tab, feats, nullptr, nullptr, T_out);
     prof_end(3, stream);
     B200VAD_LAUNCH_CHECK();
     return B200VAD_OK;
 }
 
 int fbank_launch(const void* wav, int wav_i16, const int32_t* lens, int B, int64_t N, int64_t stride, float* feats, __half* feats_hi,
-                 __half* feats_lo, int64_t T_out, double* row_sums, int device, cudaStream_t stream) {
+                 __half* feats_lo, int64_t T_out, double* row_sums, int device, cudaStream_t stream, const void* const* rows) {
     const FbankTables* tab = fbank_tables(device);
     if (!tab) {
         set_error("fbank: b200vad_init(%d) has not been called", device);
@@ -434,8 +444,10 @@ int fbank_launch(const void* wav, int wav_i16, const int32_t* lens, int B, int64
     }
     if (B == 0 || T_out == 0) return B200VAD_OK;
     if (wav_i16)
-        return fbank_launch_t(static_cast<const int16_t*>(wav), lens, B, N, stride, feats, feats_hi, feats_lo, T_out, row_sums, tab, stream);
-    return fbank_launch_t(static_cast<const float*>(wav), lens, B, N, stride, feats, feats_hi, feats_lo, T_out, row_sums, tab, stream);
+        return fbank_launch_t(static_cast<const int16_t*>(wav), reinterpret_cast<const int16_t* const*>(rows), lens, B, N, stride, feats,
+                              feats_hi, feats_lo, T_out, row_sums, tab, stream);
+    return fbank_launch_t(static_cast<const float*>(wav), reinterpret_cast<const float* const*>(rows), lens, B, N, stride, feats, feats_hi,
+                          feats_lo, T_out, row_sums, tab, stream);
 }
 
 }  // namespace b200vad

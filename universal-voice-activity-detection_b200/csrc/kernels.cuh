@@ -24,8 +24,9 @@ int gemm_launch(const GemmArgs& a, int a_half, int terms, cudaStream_t stream);
 int split_weights(const float* w, int N, int K, int Kp, __half* hi, __half* lo, cudaStream_t stream, int gate_scale = 0);
 int fbank_tables_init(int device);
 int zero_f64_launch(double* p, int64_t n, cudaStream_t stream);
+// rows != nullptr: row b starts at rows[b] (B device pointers of the sample type) instead of wav + b * stride
 int fbank_launch(const void* wav, int wav_i16, const int32_t* lens, int B, int64_t N, int64_t stride, float* feats, __half* feats_hi,
-                 __half* feats_lo, int64_t T_out, double* row_sums, int device, cudaStream_t stream);
+                 __half* feats_lo, int64_t T_out, double* row_sums, int device, cudaStream_t stream, const void* const* rows = nullptr);
 int lstm_recurrent_launch(const float* xg, const __half* whh, float* y, int B, int T, cudaStream_t stream);
 int lstm_tc_set_tile(int nb);
 // Scale s of the (x1, x2) activation planes of the 2-MMA projection: x1 = fp16((1 - s) x), x2 = fp16(x - x1) (gemm_tc.cu)
@@ -77,8 +78,10 @@ int lstm_pair_last_timeout(int* out7);
 void lstm_pair_set_opt(int opt);
 int lstm_pair_read_debug(long long* host, int n);
 int add_bias(const float* a, const float* b, float* out, int n, cudaStream_t stream);
+// stream_off == nullptr: B rows of T frames; else B streams prob[stream_off[b], stream_off[b + 1]) of at most T frames each, written
+// at the same offsets of out
 int threshold_median_launch(const float* prob, int B, int64_t T, float thr, int kernel, void* out, int elem,
-                            int32_t* near_count, float near_tol, cudaStream_t stream);
+                            int32_t* near_count, float near_tol, cudaStream_t stream, const int64_t* stream_off = nullptr);
 // offsets == nullptr: R uniform rows of uniform_T frames
 int segments_launch(const uint8_t* dec, const int64_t* offsets, int64_t uniform_T, int R, int min_run, int row_base,
                     int32_t* counts, int64_t* seg_off, int32_t* seg, int64_t cap, cudaStream_t stream);
@@ -96,9 +99,11 @@ int norm_lrelu_launch(float* pooled, int B, int64_t P, int C, const double* stat
                       cudaStream_t s, __half* p_hi = nullptr, __half* p_lo = nullptr, int Cp = 0, int scaled_planes = 0);
 int pool_norm_lrelu_launch(const float* in, int B, int64_t L, int C, float* pooled, double* stats, const float* gamma,
                            const float* beta, cudaStream_t s, __half* p_hi = nullptr, __half* p_lo = nullptr, int Cp = 0, int scaled_planes = 0);
-// wav: (B, N) f32 rows, or int16 PCM rows (wav_i16 != 0; samples int16 / 32768), `stride` elements apart
+// wav: (B, N) f32 rows, or int16 PCM rows (wav_i16 != 0; samples int16 / 32768), `stride` elements apart.  rows != nullptr: row
+// b starts at rows[b] instead, and lens[b] (required with rows) are its valid samples; samples at index >= lens[b] read as 0
 int wave_norm_planes_launch(const void* wav, int wav_i16, int B, int64_t N, int64_t stride, int64_t Np, const float* gamma,
-                            const float* beta, double* stats, __half* hi, __half* lo, cudaStream_t s, int scaled_planes = 0);
+                            const float* beta, double* stats, __half* hi, __half* lo, cudaStream_t s, int scaled_planes = 0,
+                            const void* const* rows = nullptr, const int32_t* lens = nullptr);
 int pad_rows_launch(const float* w, int Cout, int K, int ld, float* out, cudaStream_t s);
 int repack_conv_pad_launch(const float* w, int Cout, int Cin, int k, int Cp, int ld, float* out, cudaStream_t s);
 
@@ -106,7 +111,10 @@ int stat_scores_launch(const uint8_t* dec, const uint8_t* lab, int64_t n, int64_
 int score_intervals_launch(const int32_t* gt_iv, int64_t n_gt, const int32_t* pred_iv, int64_t n_pred, const int64_t* word_off,
                            const int32_t* nframes, int R, int64_t total_words, uint32_t* masks, int64_t* fa, int64_t* md,
                            int max_words_per_rec_hint, cudaStream_t st);
-int stitch_center_launch(const float* prob, int W, int Tw, int hop, float* out, int64_t L, cudaStream_t st);
+// win_off == nullptr: one recording of W windows and L frames; else R recordings, windows [win_off[r], win_off[r + 1]) of prob
+// stitched into out[frame_off[r], frame_off[r + 1]), each at most L frames.  elem: 4 (f32) or 1 (u8)
+int stitch_center_launch(const void* prob, const int64_t* win_off, const int64_t* frame_off, int R, int W, int Tw, int hop, void* out,
+                         int64_t L, int elem, cudaStream_t st);
 int stream_append_launch(float* ring, const float* chunk, float* lin, int S, int Wn, int hop, int pos, cudaStream_t st);
 int stream_newest_launch(const float* prob, const uint8_t* dec, int S, int64_t T, int nf, float* prob_out, uint8_t* dec_out,
                          cudaStream_t st);

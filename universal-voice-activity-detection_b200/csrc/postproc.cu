@@ -14,15 +14,20 @@ constexpr int kMedTile = 2048;      // frames per CTA
 constexpr int kMedMaxHalo = 512;    // supports kernel sizes up to 1025
 
 // prob: [B][T] fp32.  out: [B][T] uint8 (elem=1) or int64 (elem=8).  NaN -> 1 (x < thr is false).
+// With stream_off (B + 1 offsets), row b is the stream prob[stream_off[b], stream_off[b + 1]) instead, zero padded at its own
+// edges, and T bounds the stream lengths (grid.x covers T); its decisions go to the same offsets of out.
 __global__ void __launch_bounds__(256)
-threshold_median_kernel(const float* __restrict__ prob, int B, int64_t T, float thr, int half, void* __restrict__ out, int elem,
-                        int32_t* __restrict__ near_count, float near_tol) {
+threshold_median_kernel(const float* __restrict__ prob, const int64_t* __restrict__ stream_off, int B, int64_t T, float thr, int half,
+                        void* __restrict__ out, int elem, int32_t* __restrict__ near_count, float near_tol) {
     __shared__ int pre[kMedTile + 2 * kMedMaxHalo + 1];
     __shared__ int warp_tot[8];
     const int b = blockIdx.y;
     const int64_t t0 = (int64_t)blockIdx.x * kMedTile;
+    const int64_t first = stream_off ? stream_off[b] : (int64_t)b * T;     // the row's first frame in prob and out
+    if (stream_off) T = stream_off[b + 1] - first;
+    if (t0 >= T) return;                            // the whole CTA: this stream is shorter than the longest one
     const int span = kMedTile + 2 * half;           // frames [t0 - half, t0 + tile + half)
-    const float* row = prob + (int64_t)b * T;
+    const float* row = prob + first;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     int near = 0;
     // exclusive prefix sum of decisions over the span, 256 frames per round
@@ -58,8 +63,8 @@ threshold_median_kernel(const float* __restrict__ prob, int B, int64_t T, float 
         if (t >= T) break;
         int sum = pre[i + 2 * half + 1] - pre[i];   // window [t-half, t+half]
         int v = sum >= need;
-        if (elem == 1) reinterpret_cast<uint8_t*>(out)[(int64_t)b * T + t] = (uint8_t)v;
-        else reinterpret_cast<int64_t*>(out)[(int64_t)b * T + t] = (int64_t)v;
+        if (elem == 1) reinterpret_cast<uint8_t*>(out)[first + t] = (uint8_t)v;
+        else reinterpret_cast<int64_t*>(out)[first + t] = (int64_t)v;
     }
     if (near_count) {
         near = (int)warp_sum((float)near);
@@ -68,7 +73,7 @@ threshold_median_kernel(const float* __restrict__ prob, int B, int64_t T, float 
 }
 
 int threshold_median_launch(const float* prob, int B, int64_t T, float thr, int kernel, void* out, int elem,
-                            int32_t* near_count, float near_tol, cudaStream_t stream) {
+                            int32_t* near_count, float near_tol, cudaStream_t stream, const int64_t* stream_off) {
     if (B == 0 || T == 0) return B200VAD_OK;
     if (kernel < 1 || (kernel & 1) == 0 || kernel / 2 > kMedMaxHalo) {
         set_error("threshold_median: kernel size must be odd and <= %d", 2 * kMedMaxHalo + 1);
@@ -76,7 +81,7 @@ int threshold_median_launch(const float* prob, int B, int64_t T, float thr, int 
     }
     int half = kernel / 2;
     dim3 grid((unsigned)((T + kMedTile - 1) / kMedTile), B);
-    threshold_median_kernel<<<grid, 256, 0, stream>>>(prob, B, T, thr, half, out, elem, near_count, near_tol);
+    threshold_median_kernel<<<grid, 256, 0, stream>>>(prob, stream_off, B, T, thr, half, out, elem, near_count, near_tol);
     B200VAD_LAUNCH_CHECK();
     return B200VAD_OK;
 }

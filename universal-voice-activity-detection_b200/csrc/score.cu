@@ -172,9 +172,20 @@ int score_intervals_launch(const int32_t* gt_iv, int64_t n_gt, const int32_t* pr
 // ---------------------------------------------------------------- long-form: centre-crop stitching
 // prob: (W, Tw) per-window values; window w starts at global frame w * hop.  out: (L) stitched stream.
 // Frame f belongs to window w = clamp((f - (Tw - hop) / 2) / hop, 0, W - 1) (shifted down while f falls outside it).
+// With win_off / frame_off (R + 1 each), grid.y = R recordings: recording r has the windows [win_off[r], win_off[r + 1]) of prob
+// and its stream is out[frame_off[r], frame_off[r + 1]); W and L are unused then.  Frames no window covers (or every frame of
+// a recording without windows) get `fill`.  With hop = Tw this is the concatenation of the windows cut to the stream's length.
 template <typename T>
 __global__ void __launch_bounds__(256)
-stitch_center_kernel(const T* __restrict__ prob, int W, int Tw, int hop, T* __restrict__ out, int64_t L, T fill) {
+stitch_center_kernel(const T* __restrict__ prob, const int64_t* __restrict__ win_off, const int64_t* __restrict__ frame_off, int W,
+                     int Tw, int hop, T* __restrict__ out, int64_t L, T fill) {
+    const int r = blockIdx.y;
+    if (win_off) {
+        prob += win_off[r] * Tw;
+        W = (int)(win_off[r + 1] - win_off[r]);
+        out += frame_off[r];
+        L = frame_off[r + 1] - frame_off[r];
+    }
     const int64_t f = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (f >= L) return;
     const int margin = (Tw - hop) / 2;
@@ -182,11 +193,18 @@ stitch_center_kernel(const T* __restrict__ prob, int W, int Tw, int hop, T* __re
     if (f < margin) w = 0;
     if (w > W - 1) w = W - 1;
     const int64_t k = f - w * hop;
-    out[f] = (k >= 0 && k < Tw) ? prob[w * Tw + k] : fill;
+    out[f] = (w >= 0 && k >= 0 && k < Tw) ? prob[w * Tw + k] : fill;
 }
-int stitch_center_launch(const float* prob, int W, int Tw, int hop, float* out, int64_t L, cudaStream_t st) {
-    if (L <= 0) return B200VAD_OK;
-    stitch_center_kernel<float><<<(unsigned)((L + 255) / 256), 256, 0, st>>>(prob, W, Tw, hop, out, L, 0.f);
+int stitch_center_launch(const void* prob, const int64_t* win_off, const int64_t* frame_off, int R, int W, int Tw, int hop, void* out,
+                         int64_t L, int elem, cudaStream_t st) {
+    if (L <= 0 || R <= 0) return B200VAD_OK;
+    const dim3 grid((unsigned)((L + 255) / 256), R);
+    if (elem == 1)
+        stitch_center_kernel<uint8_t><<<grid, 256, 0, st>>>(static_cast<const uint8_t*>(prob), win_off, frame_off, W, Tw, hop,
+                                                            static_cast<uint8_t*>(out), L, 0);
+    else
+        stitch_center_kernel<float><<<grid, 256, 0, st>>>(static_cast<const float*>(prob), win_off, frame_off, W, Tw, hop,
+                                                          static_cast<float*>(out), L, 0.f);
     B200VAD_LAUNCH_CHECK();
     return B200VAD_OK;
 }

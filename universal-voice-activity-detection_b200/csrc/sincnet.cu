@@ -71,17 +71,32 @@ int repack_conv_launch(const float* w, int Cout, int Cin, int k, float* out, cud
 __device__ __forceinline__ float sample_f32(float v) { return v; }
 __device__ __forceinline__ float sample_f32(int16_t v) { return (float)v * (1.f / 32768.f); }
 
+// Rows of N samples, at wav + b * stride or, with a pointer table, at rows[b] (windows of several recordings in one launch).
+// With a table, lens[b] are the row's valid samples and every sample at index >= lens[b] is read as 0 without touching
+// memory: that is the zero-padded tail window of the reference, which the InstanceNorm sees.  The statistics walk all N
+// samples in the same order either way, and adding 0 changes no partial sum, so the statistics and planes of a row read
+// through the table equal those of the same samples copied into a zero-padded row, bit for bit.
+template <typename S>
+__device__ __forceinline__ const S* wave_row(const S* wav, const S* const* rows, int64_t stride, int b) {
+    return rows ? rows[b] : wav + (int64_t)b * stride;
+}
+__device__ __forceinline__ int64_t wave_valid(const int32_t* lens, int64_t N, int b) {
+    return lens ? min((int64_t)lens[b], N) : N;
+}
+
 // stats[b] = (sum, sumsq) in double
 template <typename S>
-__global__ void __launch_bounds__(256) wave_stats_kernel(const S* __restrict__ wav, int64_t N, int64_t stride,
+__global__ void __launch_bounds__(256) wave_stats_kernel(const S* __restrict__ wav, const S* const* __restrict__ rows,
+                                                         const int32_t* __restrict__ lens, int64_t N, int64_t stride,
                                                          double* __restrict__ stats) {
     const int b = blockIdx.y;
-    const S* row = wav + (int64_t)b * stride;
+    const S* row = wave_row(wav, rows, stride, b);
+    const int64_t n = wave_valid(lens, N, b);
     const int64_t chunk = 256 * 32;
     int64_t begin = (int64_t)blockIdx.x * chunk, end = min(begin + chunk, N);
     float s = 0.f, q = 0.f;
     for (int64_t i = begin + threadIdx.x; i < end; i += 256) {
-        float v = sample_f32(__ldg(row + i));
+        float v = i < n ? sample_f32(__ldg(row + i)) : 0.f;
         s += v;
         q = fmaf(v, v, q);
     }
@@ -118,7 +133,7 @@ int wave_instnorm_launch(const float* wav, int B, int64_t N, int64_t stride, con
                          double* stats, float* out, cudaStream_t s) {
     { int rc = zero_f64_launch(stats, (int64_t)2 * B, s); if (rc) return rc; }
     dim3 g1((unsigned)((N + 8191) / 8192), B);
-    wave_stats_kernel<float><<<g1, 256, 0, s>>>(wav, N, stride, stats);
+    wave_stats_kernel<float><<<g1, 256, 0, s>>>(wav, nullptr, nullptr, N, stride, stats);
     B200VAD_LAUNCH_CHECK();
     dim3 g2((unsigned)((N + 4095) / 4096), B);
     wave_norm_kernel<<<g2, 256, 0, s>>>(wav, N, stride, stats, gamma, beta, out);
@@ -146,7 +161,8 @@ __device__ __forceinline__ void load8_f32(const int16_t* row, float (&v)[8]) {
     }
 }
 template <typename S>
-__global__ void __launch_bounds__(256) wave_norm_planes_kernel(const S* __restrict__ wav, int64_t N, int64_t stride, int64_t Np,
+__global__ void __launch_bounds__(256) wave_norm_planes_kernel(const S* __restrict__ wav, const S* const* __restrict__ rows,
+                                                               const int32_t* __restrict__ lens, int64_t N, int64_t stride, int64_t Np,
                                                                int B, const double* __restrict__ stats, const float* __restrict__ gamma,
                                                                const float* __restrict__ beta, __half* __restrict__ hi,
                                                                __half* __restrict__ lo, float s1) {
@@ -155,17 +171,19 @@ __global__ void __launch_bounds__(256) wave_norm_planes_kernel(const S* __restri
     double var = stats[2 * b + 1] / (double)N - mean * mean;
     float rstd = (float)(1.0 / sqrt(fmax(var, 0.0) + 1e-5));
     float m = (float)mean, g = gamma[0], be = beta[0];
-    const S* row = wav + (int64_t)b * stride;
+    const S* row = wave_row(wav, rows, stride, b);
+    const int64_t n = wave_valid(lens, N, b);
     // 8 consecutive samples per thread (Np and the copies' bases are multiples of 8 elements): copy e receives them at
     // element i - 2 e, i.e. at a 16 / 4 / 8 / 4-byte aligned address for e = 0 / 1 / 2 / 3
-    const bool vec_ok = ((stride * (int64_t)sizeof(S)) % 16 == 0) && ((reinterpret_cast<uintptr_t>(wav) & 15) == 0);
+    const bool vec_ok = rows ? (reinterpret_cast<uintptr_t>(row) & 15) == 0
+                             : ((stride * (int64_t)sizeof(S)) % 16 == 0) && ((reinterpret_cast<uintptr_t>(wav) & 15) == 0);
     for (int64_t i = ((int64_t)blockIdx.x * 256 + threadIdx.x) * 8; i < Np + 8; i += (int64_t)gridDim.x * 256 * 8) {
         float v[8];
-        if (vec_ok && i + 8 <= N) {
+        if (vec_ok && i + 8 <= n) {
             load8_f32(row + i, v);
         } else {
 #pragma unroll
-            for (int j = 0; j < 8; ++j) v[j] = (i + j < N) ? sample_f32(row[i + j]) : 0.f;
+            for (int j = 0; j < 8; ++j) v[j] = (i + j < n) ? sample_f32(row[i + j]) : 0.f;
         }
         __align__(16) __half h[8], l[8];
 #pragma unroll
@@ -203,22 +221,27 @@ __global__ void __launch_bounds__(256) wave_norm_planes_kernel(const S* __restri
     }
 }
 template <typename S>
-static int wave_norm_planes_run(const S* wav, int B, int64_t N, int64_t stride, int64_t Np, const float* gamma, const float* beta,
-                                double* stats, __half* hi, __half* lo, cudaStream_t s, int scaled_planes) {
+static int wave_norm_planes_run(const S* wav, const S* const* rows, const int32_t* lens, int B, int64_t N, int64_t stride, int64_t Np,
+                                const float* gamma, const float* beta, double* stats, __half* hi, __half* lo, cudaStream_t s,
+                                int scaled_planes) {
     { int rc = zero_f64_launch(stats, (int64_t)2 * B, s); if (rc) return rc; }
     dim3 g1((unsigned)((N + 8191) / 8192), B);
-    wave_stats_kernel<S><<<g1, 256, 0, s>>>(wav, N, stride, stats);
+    wave_stats_kernel<S><<<g1, 256, 0, s>>>(wav, rows, lens, N, stride, stats);
     B200VAD_LAUNCH_CHECK();
     dim3 g2((unsigned)((Np + 8 + 2047) / 2048), B);
-    wave_norm_planes_kernel<S><<<g2, 256, 0, s>>>(wav, N, stride, Np, B, stats, gamma, beta, hi, lo, scaled_planes ? 1.f - kPlaneScale : 1.f);
+    wave_norm_planes_kernel<S><<<g2, 256, 0, s>>>(wav, rows, lens, N, stride, Np, B, stats, gamma, beta, hi, lo,
+                                                  scaled_planes ? 1.f - kPlaneScale : 1.f);
     B200VAD_LAUNCH_CHECK();
     return B200VAD_OK;
 }
 int wave_norm_planes_launch(const void* wav, int wav_i16, int B, int64_t N, int64_t stride, int64_t Np, const float* gamma,
-                            const float* beta, double* stats, __half* hi, __half* lo, cudaStream_t s, int scaled_planes) {
+                            const float* beta, double* stats, __half* hi, __half* lo, cudaStream_t s, int scaled_planes,
+                            const void* const* rows, const int32_t* lens) {
     if (wav_i16)
-        return wave_norm_planes_run(reinterpret_cast<const int16_t*>(wav), B, N, stride, Np, gamma, beta, stats, hi, lo, s, scaled_planes);
-    return wave_norm_planes_run(reinterpret_cast<const float*>(wav), B, N, stride, Np, gamma, beta, stats, hi, lo, s, scaled_planes);
+        return wave_norm_planes_run(reinterpret_cast<const int16_t*>(wav), reinterpret_cast<const int16_t* const*>(rows), lens, B, N, stride,
+                                    Np, gamma, beta, stats, hi, lo, s, scaled_planes);
+    return wave_norm_planes_run(reinterpret_cast<const float*>(wav), reinterpret_cast<const float* const*>(rows), lens, B, N, stride, Np,
+                                gamma, beta, stats, hi, lo, s, scaled_planes);
 }
 
 // GEMM weights for the tcgen05 path, zero padded to 128 output rows: (Cout, K) -> (128, ld)
